@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """AV-VAD inference benchmark (BASELINE.json metric: AV-VAD frames/sec, device-timed).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2]): full audio-visual net (DeepVAD_AV, use_mcb=True as in
 scripts/train_AV_net.py:70) inference on a batch of 256 synthetic utterances per GPU: 81,920
@@ -26,6 +26,10 @@ one pass of the whole hot path over one batch: peak-normalise -> STFT/log-power/
 `--impl reference` times that CPU port alone (the reference's own CPU implementation of the path:
 the reference cannot be pip-installed -- it has no setup.py -- and its MCB branch does not run on
 torch >= 1.8, see DESIGN.md).
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0; `value`'s device path: logits, posteriors,
+decisions; the CPU port: posteriors, decisions) as DIR/<name>.npy in float32.  Inputs and weights are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -52,6 +56,21 @@ T_FRAMES = 317
 METRIC = "AV-VAD frames/sec (device-timed)"
 # tensor-core work per frame of the 19 implicit-GEMM convolutions (layer1-4; conv1 runs as a direct conv)
 CONV_MAC_PER_FRAME = 216_633_600 - 1156 * 64 * 49
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """name -> tensor as out_dir/<name>.npy in float32.  Past DUMP_LIMIT_BYTES in all, every array keeps the same fixed,
+    seeded sample of rows (utterances) along its first axis."""
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: t.detach().float().cpu().numpy() for k, t in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        n = next(iter(host.values())).shape[0]
+        rows = np.sort(np.random.default_rng(0).choice(n, max(1, n * DUMP_LIMIT_BYTES // total), replace=False))
+        host = {k: a[rows] for k, a in host.items()}
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 def synth_batch(B: int, seed: int):
@@ -223,7 +242,7 @@ def train_block(args, rank, world, dev):
     for _ in range(3):
         loss = tr.step((a, v), tgt, ln)
     barrier()
-    steps = max(3, min(args.steps, 10))
+    steps = args.steps
     l0 = E.launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
@@ -405,9 +424,11 @@ def run_reference(args, rank, world):
     t0 = time.perf_counter()
     frames = 0
     for _ in range(args.steps):
-        _, _, lens = cpu_av_step(model, waves, vids, mean, std, synth.VIDEO_MEAN, synth.VIDEO_STD)
+        post, dec, lens = cpu_av_step(model, waves, vids, mean, std, synth.VIDEO_MEAN, synth.VIDEO_STD)
         frames += int(sum(lens))
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"posteriors": post, "decisions": dec})
     val = frames / dt
     sample = f"{B_s} utterances x {T_FRAMES} frames per step (bounded sample of the batch-256 workload)"
     line = {
@@ -482,13 +503,16 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        step_device()
+        out = step_device()
     e1.record()
     barrier()
     E.profile_enable(False)
     ms = e0.elapsed_time(e1)
     launches = E.launch_count() - l0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("logits", "posteriors", "decisions"), out)))
+    del out
     if os.environ.get("AVVAD_LAYER_DUMP") and rank == 0:  # needs AVVAD_PROFILE_PER_LAUNCH=1 for per-layer rows
         # per-layer table of the implicit-GEMM convolutions (grouped by algorithmic FLOPs per launch)
         lms, lfl = E.profile_dump(0)
@@ -718,7 +742,11 @@ def main():
     ap.add_argument("--no-config4", action="store_true", help="skip the 10,000-utterance sharded evaluation (config 4)")
     ap.add_argument("--train-batch", type=int, default=256, help="GLOBAL utterances per training step")
     ap.add_argument("--ncu", action="store_true", help="profiling mode: warm-up + one pass, prints nothing")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -8,7 +8,7 @@ import torch
 from oracle import models as om
 from avvad import engine as E
 from avvad import synth
-from util import golden, err_stats
+from util import err_stats, ref_models
 
 pytestmark = pytest.mark.gpu
 POST_TOL = 1e-2
@@ -16,7 +16,7 @@ POST_TOL = 1e-2
 
 @pytest.fixture(scope="module")
 def gref():
-    return golden("ref_models.npz")
+    return ref_models()
 
 
 def _sd(kind, seed, **kw):

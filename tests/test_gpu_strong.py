@@ -18,7 +18,7 @@ from oracle.reference_port import cpu_av_inputs
 from avvad import engine as E
 from avvad import synth
 from avvad.pipeline import AVVADPipeline
-from util import golden, err_stats, check_logits, sigmoid as _sig, POST_TOL
+from util import golden, ref_models, err_stats, check_logits, sigmoid as _sig, POST_TOL
 
 pytestmark = pytest.mark.gpu
 
@@ -30,7 +30,7 @@ def gs():
 
 @pytest.fixture(scope="module")
 def gref():
-    return golden("ref_models.npz")
+    return ref_models()
 
 
 def _with_bias(module, head, gs, key):

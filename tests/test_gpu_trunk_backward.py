@@ -16,7 +16,7 @@ import torch
 from oracle import models as om
 from avvad import engine as E
 from avvad import synth
-from util import golden, err_stats, grad_digest_of
+from util import golden, ref_models, err_stats, grad_digest_of
 
 pytestmark = pytest.mark.gpu
 CONV_TOL = 3e-2       # conv / BatchNorm gradients, relative Frobenius error (bf16 operands, fp32 accumulation)
@@ -122,7 +122,7 @@ def test_video_net_training_step_matches_reference_module_digest():
     BatchNorm running statistics are compared directly; the gradients -- which for ANY bf16 forward sit 18-36 % from the
     fp32 ones (oracle.models.bf16_ste) -- by the cosine of the reference's stored strided samples and by their norms."""
     from packages.models.Video_Net import DeepVAD_video
-    gs, gref = golden("ref_strong.npz"), golden("ref_models.npz")
+    gs, gref = golden("ref_strong.npz"), ref_models()
     v, lens = torch.tensor(gref["av_video"]), gref["av_len"].tolist()
     y = torch.tensor(gs["train_target"])
     m = synth.fill_module_(DeepVAD_video(2, 1024, 1), seed=47, family="strong").cuda().train()
@@ -245,7 +245,7 @@ def test_video_net_optimiser_steps_with_torch_adam_reduce_the_loss():
     assert not torch.equal(w0, m.features[0].weight.detach())      # conv1 really is being trained
 
 
-def test_weight_gradient_chunking_is_invisible():
+def test_weight_gradient_chunking_is_invisible(tmp_path):
     """The weight-gradient GEMMs run over chunks of <= 2^19 pixels and accumulate; with AVVAD_WGRAD_PIXELS=2048 the
     44-frame test input is split into up to 7 chunks per layer (and the last one is ragged).  Both settings must give the
     same gradients (fp32 accumulation order differs only across the split-K partials)."""
@@ -268,7 +268,7 @@ def test_weight_gradient_chunking_is_invisible():
     ) % (os.path.join(root, "audio-visual-vad_b200"), root)
     outs = []
     for px in ("524288", "2048"):
-        path = f"/tmp/avvad_wgrad_{px}.pt"
+        path = str(tmp_path / f"wgrad_{px}.pt")
         subprocess.run([sys.executable, "-c", code, path], check=True, env=dict(os.environ, AVVAD_WGRAD_PIXELS=px))
         outs.append(torch.load(path))
     for i, (a, b) in enumerate(zip(*outs)):

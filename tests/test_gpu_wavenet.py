@@ -53,7 +53,7 @@ def test_fused_stack_many_time_tiles_vs_oracle(k, dil, N, B):
     assert out.shape == ref.shape and st["rel_fro"] < 2e-2 and st["max"] < 3e-2 * max(1.0, st["ref_absmax"]), st
 
 
-def test_fused_and_per_layer_paths_agree():
+def test_fused_and_per_layer_paths_agree(tmp_path):
     """AVVAD_WAVENET_FUSED=0 selects the per-layer path (im2col copy + one GEMM per layer); both must give the
     reference's answer (run in a subprocess because the switch is read once per process)."""
     import os
@@ -72,7 +72,7 @@ def test_fused_and_per_layer_paths_agree():
          os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
     outs = []
     for flag in ("1", "0"):
-        path = f"/tmp/avvad_wn_{flag}.npy"
+        path = str(tmp_path / f"wn_{flag}.npy")
         env = dict(os.environ, AVVAD_WAVENET_FUSED=flag)
         subprocess.run([sys.executable, "-c", code, path], check=True, env=env)
         outs.append(np.load(path))

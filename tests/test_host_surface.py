@@ -65,18 +65,43 @@ def test_collate_matches_reference_golden():
     assert np.array_equal(pv.numpy(), g["collate_v"]) and np.array_equal(pt.numpy(), g["collate_t"])
 
 
-def test_path_builders_on_the_reference_subset():
-    root = "/root/reference/data/subset/processed/"
-    if not os.path.isdir(root):
-        pytest.skip("reference data not present (GPU box)")
+def test_path_builders_on_the_reference_subset(tmp_path):
+    """The test/34M part of the reference's data/subset/processed tree (SURVEY appendix A): sa1's label file verbatim
+    (tests/golden/h5), the other label files from the golden labels, upsampled ROI videos at the shipped shapes, and
+    files of the same directories that the builders must not pick up."""
+    import shutil
+    from avvad import h5min, synth
+    from oracle import video as ov
     from packages.dataset.ntcd_timit import proc_noisy_clean_pair_dict, proc_video_audio_pair_dict
     from packages.data_handling import WavWholeSequenceSpectrogramLabeledFrames
+    g = np.load(os.path.join(G, "golden_frontend_34M.npz"))
+    clean = tmp_path / "ntcd_timit" / "Clean" / "test" / "34M"
+    video = tmp_path / "ntcd_timit" / "matlab_raw" / "test" / "34M"
+    for d in (clean, video):
+        d.mkdir(parents=True)
+    shutil.copyfile(os.path.join(G, "h5", "ntcd_timit_statistics.h5"), video.parent.parent / "ntcd_timit_statistics.h5")
+    frames = {}
+    for k, (utt, F) in enumerate((("sa1", 152), ("sa2", 136), ("si494", 134))):
+        T = g[utt + "_vad"].shape[1]
+        if utt == "sa1":
+            shutil.copyfile(os.path.join(G, "h5", "sa1_vad_labels.h5"), clean / "sa1_vad_labels.h5")
+        else:
+            h5min.write_h5(str(clean / f"{utt}_vad_labels.h5"),
+                           {"Y": (g[utt + "_vad"].astype(np.float32), dict(maxshape=(1, None), creation_shape=(1, 0)))})
+        src = synth.synth_video_u8(F, k).astype(np.float32)
+        frames[utt] = np.ascontiguousarray(np.moveaxis(src[ov.upsample_index(F, T)], 0, -1))    # (67,67,T)
+        h5min.write_h5(str(video / f"{utt}_upsampled.h5"),
+                       {"X": (frames[utt], dict(maxshape=(67, 67, None), creation_shape=(67, 67, 0)))})
+        (clean / f"{utt}_ibm_labels.h5").touch()
+        (video / f"{utt}.mat").touch()
+    root = str(tmp_path) + "/"
     pairs = proc_noisy_clean_pair_dict(root, "test", "subset", "vad_labels", upsampled=False)
     assert list(pairs.items())[0] == ("ntcd_timit/Noisy/Babble/-5/test/34M/sa1.wav", "ntcd_timit/Clean/test/34M/sa1_vad_labels.h5")
     v, a = proc_video_audio_pair_dict(root, "test", "vad_labels", upsampled=True)
     assert len(v) == 3 and v[0].endswith("sa1_upsampled.h5") and a[0].endswith("sa1_vad_labels.h5")
     x, y, n = WavWholeSequenceSpectrogramLabeledFrames(root, "test", labels="vad_labels", upsampled=True)[0]
     assert tuple(x.shape) == (67, 67, 317) and tuple(y.shape) == (1, 317) and n == 317
+    assert np.array_equal(x.numpy(), frames["sa1"]) and np.array_equal(y.numpy(), g["sa1_vad"])
 
 
 def test_metrics_helpers():

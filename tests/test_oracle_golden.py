@@ -10,6 +10,7 @@ from oracle import frontend as ofe
 from oracle import models as om
 from oracle import video as ov
 from avvad import synth
+from util import ref_models
 
 G = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -26,7 +27,7 @@ def gup():
 
 @pytest.fixture(scope="module")
 def gref():
-    return np.load(os.path.join(G, "ref_models.npz"))
+    return ref_models()
 
 
 # ---- front end ---------------------------------------------------------------------------------

@@ -11,7 +11,7 @@ import torch
 
 from oracle import models as om
 from avvad import synth
-from util import golden, err_stats, grad_digest_of
+from util import golden, ref_models, err_stats, grad_digest_of
 
 
 @pytest.fixture(scope="module")
@@ -21,7 +21,7 @@ def gs():
 
 @pytest.fixture(scope="module")
 def gref():
-    return golden("ref_models.npz")
+    return ref_models()
 
 
 def _sd(kind, seed, family="strong", **kw):

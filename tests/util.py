@@ -11,6 +11,14 @@ def golden(name):
     return np.load(os.path.join(GOLDEN, name))
 
 
+def ref_models():
+    """tests/golden/ref_models.npz as a dict.  The AV cases ran on the video-only input, so av_video (== video_x) is
+    stored once."""
+    g = dict(golden("ref_models.npz"))
+    g["av_video"] = g["video_x"]
+    return g
+
+
 def err_stats(a, b):
     a = np.asarray(a, dtype=np.float64)
     b = np.asarray(b, dtype=np.float64)

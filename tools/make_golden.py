@@ -147,7 +147,7 @@ def ref_models():
     m = synth.fill_module_(DeepVAD_AV(2, 1024, 1, use_mcb=False, eps=1e-8), seed=13).eval()
     xa2 = torch.randn(2, 6, 513, generator=g)
     with torch.no_grad():
-        d["av_audio"], d["av_video"], d["av_len"] = xa2.numpy(), xv.numpy(), np.asarray(lv)
+        d["av_audio"], d["av_len"] = xa2.numpy(), np.asarray(lv)   # video input: video_x (tests/util.py::ref_models)
         d["av_out"] = m(xa2, xv, lv).numpy()
     # y_dim = 513 (IBM variant, train_AV_net.py:65-66)
     m = synth.fill_module_(DeepVAD_AV(2, 1024, 513, use_mcb=False, eps=1e-8), seed=14).eval()
@@ -252,7 +252,7 @@ def ref_strong():
     d["cbp_x"], d["cbp_y"], d["cbp_go"] = x.detach().numpy(), y.detach().numpy(), go.numpy()
     d["cbp_out"], d["cbp_gx"], d["cbp_gy"] = out.detach().numpy(), x.grad.numpy(), y.grad.numpy()
 
-    a6, v6, l6 = torch.tensor(base["av_audio"]), torch.tensor(base["av_video"]), base["av_len"].tolist()
+    a6, v6, l6 = torch.tensor(base["av_audio"]), torch.tensor(base["video_x"]), base["av_len"].tolist()
 
     def strong_forward(m, head, key, *inputs, lengths):
         """Forward with the strong family, head bias placed by synth.decision_bias (stored as <key>_bias)."""
