@@ -610,6 +610,25 @@ def lstm_train_forward(lstm: "Lstm", x_bf16: torch.Tensor, lengths):
     return logits, (tape, lens, x_bf16)
 
 
+def lstm_tape_views(lstm: "Lstm", tape, B: int, T: int):
+    """Views into a training tape (inspection hook for the state tests): one (gates, c, h) triple per layer with
+    gates bf16 (B, T, 4H) gate-interleaved (element 4u+g, g = i, f, g, o), c f32 (B, T, H) and h bf16 (B, T, H).
+    `tape` is the byte tensor or the pack lstm_train_forward returns."""
+    if isinstance(tape, tuple):
+        tape = tape[0]
+    H, Lyr = lstm.hidden, lstm.layers
+    off = (C.c_int64 * (3 * Lyr))()
+    L.check(L.lib().avvad_lstm_tape_layout(Lyr, H, B, T, off, 3 * Lyr))
+    assert tape.dtype == torch.uint8 and tape.numel() >= L.lib().avvad_lstm_tape_bytes(Lyr, H, B, T)
+
+    def view(o, numel, dtype, shape):
+        nbytes = numel * torch.empty((), dtype=dtype).element_size()
+        return tape[o:o + nbytes].view(dtype).view(shape)
+    n = B * T * H
+    return [(view(off[3 * l], 4 * n, torch.bfloat16, (B, T, 4 * H)), view(off[3 * l + 1], n, torch.float32, (B, T, H)),
+             view(off[3 * l + 2], n, torch.bfloat16, (B, T, H))) for l in range(Lyr)]
+
+
 def lstm_train_backward(lstm: "Lstm", tape_pack, dlogits: torch.Tensor, want_dx=False):
     """BPTT.  Returns dict(weight_ih=[...], weight_hh=[...], bias=[...], head_w, head_b, dx)."""
     tape, lens, x_bf16 = tape_pack

@@ -87,6 +87,7 @@ PROTOTYPES = {
     "avvad_lzf_compress": (C.c_int64, [VP, C.c_int64, VP, C.c_int64, C.c_int, VP]),
     "avvad_lzf_decompress": (C.c_int64, [VP, C.c_int64, VP, C.c_int64]),
     "avvad_lstm_tape_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int64, C.c_int64]),
+    "avvad_lstm_tape_layout": (C.c_int, [C.c_int, C.c_int, C.c_int64, C.c_int64, c_i64p, C.c_int]),
     "avvad_lstm_forward_train": (C.c_int, [VP, VP, VP, C.c_int64, C.c_int64, VP, C.c_size_t, VP, C.c_size_t, VP, VP]),
     "avvad_lstm_backward_workspace_bytes": (C.c_size_t, [VP, C.c_int64, C.c_int64]),
     "avvad_lstm_backward": (C.c_int, [VP, VP, VP, C.c_int64, C.c_int64, VP, VP, VP, C.c_size_t, VP, VP, VP, VP, VP, VP,

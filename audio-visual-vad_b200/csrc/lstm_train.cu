@@ -283,11 +283,37 @@ __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, 
 using namespace avvad;
 
 // ---- tape / workspace geometry (shared with lstm.cu through these helpers) --------------------------------------
+// Per layer l the tape holds, each region 256-byte aligned: gates bf16 [B][T][4H] (gate-interleaved, element 4u+g),
+// c f32 [B][T][H], hseq bf16 [B][T][H].  tape_offsets() is the one place that lays it out.
+namespace avvad {
+struct TapeOffsets {
+  size_t gates, c, hseq, per_layer;
+};
+static TapeOffsets tape_offsets(int l, int H, int64_t B, int64_t T) {
+  const size_t g = align_up((size_t)B * T * 4 * H * 2, 256), c = align_up((size_t)B * T * H * 4, 256),
+               h = align_up((size_t)B * T * H * 2, 256);
+  const size_t base = (size_t)l * (g + c + h);
+  return TapeOffsets{base, base + g, base + g + c, g + c + h};
+}
+}  // namespace avvad
+
 extern "C" size_t avvad_lstm_tape_bytes(int layers, int hidden, int64_t B, int64_t T) {
   if (layers <= 0 || hidden <= 0 || B <= 0 || T <= 0) return 0;
-  const size_t per = align_up((size_t)B * T * 4 * hidden * 2, 256) + align_up((size_t)B * T * hidden * 4, 256) +
-                     align_up((size_t)B * T * hidden * 2, 256);
-  return per * layers + 256;
+  return tape_offsets(0, hidden, B, T).per_layer * layers + 256;
+}
+
+// Byte offsets of the tape's tensors (inspection hook used by the state tests): offsets[3l + {0, 1, 2}] = gates, c and
+// hseq of layer l.
+extern "C" int avvad_lstm_tape_layout(int layers, int hidden, int64_t B, int64_t T, int64_t* offsets, int count) {
+  AVVAD_CHECK_ARG(layers >= 1 && layers <= 8 && hidden > 0 && B > 0 && T > 0, "bad sizes");
+  AVVAD_CHECK_ARG(offsets && count == 3 * layers, "offsets must hold 3 entries per layer");
+  for (int l = 0; l < layers; ++l) {
+    const TapeOffsets o = tape_offsets(l, hidden, B, T);
+    offsets[3 * l + 0] = (int64_t)o.gates;
+    offsets[3 * l + 1] = (int64_t)o.c;
+    offsets[3 * l + 2] = (int64_t)o.hseq;
+  }
+  return AVVAD_OK;
 }
 
 extern "C" int avvad_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr,
@@ -392,13 +418,12 @@ struct TapeView {
   __nv_bfloat16* hseq;
 };
 TapeView tape_layer(void* tape, int l, int H, int64_t B, int64_t T) {
-  const size_t g = align_up((size_t)B * T * 4 * H * 2, 256), c = align_up((size_t)B * T * H * 4, 256),
-               h = align_up((size_t)B * T * H * 2, 256);
-  uint8_t* p = (uint8_t*)tape + (size_t)l * (g + c + h);
+  const TapeOffsets o = tape_offsets(l, H, B, T);
+  uint8_t* p = (uint8_t*)tape;
   TapeView v;
-  v.gates = (__nv_bfloat16*)p;
-  v.c = (float*)(p + g);
-  v.hseq = (__nv_bfloat16*)(p + g + c);
+  v.gates = (__nv_bfloat16*)(p + o.gates);
+  v.c = (float*)(p + o.c);
+  v.hseq = (__nv_bfloat16*)(p + o.hseq);
   return v;
 }
 

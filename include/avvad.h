@@ -357,6 +357,13 @@ int avvad_lstm_forward(avvad_lstm* h, const void* x_bf16, const int32_t* lengths
  * replaces: autograd of packages/models/AV_Net.py:127-140 and torch.optim.Adam (scripts/train_AV_net.py:238,305-307).
  * ---------------------------------------------------------------------------------------- */
 size_t avvad_lstm_tape_bytes(int layers, int hidden, int64_t B, int64_t T);
+/* Byte offsets of the tape's tensors (inspection hook used by the state tests, host only): offsets[3l + 0, 1, 2] =
+ * layer l's
+ *   gates : bf16 [B][T][4H] post-activation gates, gate-interleaved (element 4u+g, g = i, f, g, o);
+ *   c     : f32  [B][T][H] cell state c_t;
+ *   hseq  : bf16 [B][T][H] output h_t in PyTorch unit order, exactly 0 for t >= len_b.
+ * count must be 3 * layers. */
+int avvad_lstm_tape_layout(int layers, int hidden, int64_t B, int64_t T, int64_t* offsets, int count);
 int avvad_lstm_forward_train(avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T,
                              void* workspace, size_t workspace_bytes, void* tape, size_t tape_bytes, float* logits,
                              void* stream);

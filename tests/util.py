@@ -31,6 +31,21 @@ def bf16_round(t: torch.Tensor) -> torch.Tensor:
     return t.to(torch.bfloat16).to(torch.float32)
 
 
+def lstm_test_weights(layers, input_size, hidden, seed):
+    """PyTorch-layout LSTM weights [(w_ih, w_hh, b_ih, b_hh)] for the state tests: U(+-2/sqrt(H)) in layer 0, as the
+    "strong" family uses, and U(+-4/sqrt(H)) above, where the input is an h sequence of std ~0.15 instead of ~0.5.  Both
+    keep the pre-activation std of every layer within [0.3, 3] for inputs N(0, 0.5^2), so the gates are neither flat nor
+    saturated (tests/test_lstm_step_oracle.py asserts it)."""
+    g = torch.Generator().manual_seed(seed)
+    ws = []
+    for l in range(layers):
+        k = (2.0 if l == 0 else 4.0) / hidden ** 0.5
+        il = input_size if l == 0 else hidden
+        shapes = ((4 * hidden, il), (4 * hidden, hidden), (4 * hidden,), (4 * hidden,))
+        ws.append(tuple((torch.rand(s, generator=g) * 2 - 1) * k for s in shapes))
+    return ws
+
+
 def grad_digest_of(g) -> tuple:
     """(Frobenius norm, strided sample of <= 2048 elements) -- the digest tools/make_golden.py::grad_digest stores for
     the reference modules' gradients."""
