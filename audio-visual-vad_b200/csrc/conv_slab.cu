@@ -5,7 +5,6 @@
 #include <mutex>
 
 #include "conv_slab.cuh"
-#include "conv_slab2.cuh"
 #include "conv_block.cuh"
 
 namespace avvad {
@@ -17,31 +16,13 @@ int encode_act_map(CUtensorMap* m, const void* ptr, int Cin, int W, int H, int64
                    const uint32_t estr[4]);
 int encode_weight_map(CUtensorMap* m, const void* ptr, uint64_t K, uint64_t N, uint32_t bn);
 
-static int slab_mode() {
-  static int v = [] {
-    const char* e = getenv("AVVAD_SLAB");
-    return e ? atoi(e) : 1;
-  }();
-  return v;
-}
-static int slab_bo() {
-  static int v = [] {
-    const char* e = getenv("AVVAD_SLAB_BO");
-    return e ? atoi(e) : 0;
-  }();
-  return v;
-}
-
+// 64 -> 64 channels (layer1): the 72 KB of weights stay resident in shared memory
 bool slab_supported(int H, int W, int Cin, int Cout, int R, int S, int stride, int pad) {
-  if (!tma_available() || slab_mode() == 0) return false;
-  if (!(R == 3 && S == 3 && stride == 1 && pad == 1 && H == W && Cin % 64 == 0 && Cout % 64 == 0)) return false;
-  if (slab_mode() == 1) return Cin == 64 && Cout == 64;  // layer1-type: weights fit in shared memory
-  return true;
+  return tma_available() && R == 3 && S == 3 && stride == 1 && pad == 1 && H == W && Cin == 64 && Cout == 64;
 }
 
 struct SlabPlan {
-  int F, hb, mb, bn, b_stages;
-  bool resident;
+  int F, hb, mb, bn;
   size_t smem;
   double eff;
 };
@@ -52,7 +33,6 @@ static bool plan(int H, int Cin, int Cout, SlabPlan* out) {
   SlabPlan best{};
   best.eff = -1;
   const int bn = 64;
-  const bool resident = (Cout == 64) && ((size_t)9 * cpb * bn * 128 <= 80 * 1024);
   for (int hb = 1; hb <= OH; ++hb) {
     const int Hs = hb + 2;
     if (Hs > 256 || Wp > 256) continue;
@@ -65,8 +45,7 @@ static bool plan(int H, int Cin, int Cout, SlabPlan* out) {
       const int slab_rows = mb * 128 + 2 * Wp + 2;
       if (slab_rows < rows) continue;
       const size_t slab_bytes = ((size_t)slab_rows * 128 + 1023) / 1024 * 1024;
-      const int b_stages = resident ? 0 : 6;
-      const size_t wbytes = resident ? (size_t)9 * cpb * bn * 128 : (size_t)b_stages * bn * 128;
+      const size_t wbytes = (size_t)9 * cpb * bn * 128;
       const size_t smem = 2 * slab_bytes + wbytes + 256 + 1024 + (size_t)Cout * 4;
       if (smem > 225 * 1024) continue;
       const int nb = (OH + hb - 1) / hb;
@@ -74,8 +53,7 @@ static bool plan(int H, int Cin, int Cout, SlabPlan* out) {
       const double eff = (double)OH * OW / ((double)nb * mb * 128.0 / F);
       // prefer higher efficiency, then more accumulator blocks per weight load
       if (eff > best.eff + 1e-9 || (eff > best.eff - 1e-9 && mb > best.mb)) {
-        best.F = F; best.hb = hb; best.mb = mb; best.bn = bn; best.b_stages = b_stages; best.resident = resident;
-        best.smem = smem; best.eff = eff;
+        best.F = F; best.hb = hb; best.mb = mb; best.bn = bn; best.smem = smem; best.eff = eff;
       }
     }
   }
@@ -84,18 +62,7 @@ static bool plan(int H, int Cin, int Cout, SlabPlan* out) {
   return true;
 }
 
-// AVVAD_SLAB_CG2=1: layer1 on CTA pairs (conv_slab.cuh).  Off by default: measured 29.12 ms of convolutions per step with
-// pairs against 29.04 ms without on the same box -- layer1 is bound by its 30 GB of activation traffic per step (64 %
-// of the HBM peak at the same time as 58 % tensor-pipe activity), not by the operand reads of its N = 64 MMAs.
-static int slab_pair() {
-  static int v = [] {
-    const char* e = getenv("AVVAD_SLAB_CG2");
-    return (e && atoi(e) == 1) ? 1 : 0;
-  }();
-  return v;
-}
-
-template <int BN, bool RES, int MBC = 0, int CG = 1>
+template <int MBC = 0>
 static int launch_k(const SlabMaps& maps, const SlabGeom& g, const EpiParams& ep, size_t smem, double flops,
                     cudaStream_t st) {
   static std::mutex mu;
@@ -106,7 +73,7 @@ static int launch_k(const SlabMaps& maps, const SlabGeom& g, const EpiParams& ep
     AVVAD_CHECK_ARG(dev >= 0 && dev < kMaxDevices, "device index out of range");
     std::lock_guard<std::mutex> lk(mu);
     if (smem > attr_set[dev]) {
-      AVVAD_CUDA(cudaFuncSetAttribute(tc_slab_kernel<BN, RES, MBC, CG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      AVVAD_CUDA(cudaFuncSetAttribute(tc_slab_kernel<64, MBC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       attr_set[dev] = smem;
     }
   }
@@ -116,99 +83,16 @@ static int launch_k(const SlabMaps& maps, const SlabGeom& g, const EpiParams& ep
     return n > 0 ? n : 148;
   }();
   void* tok = nullptr;
-  if (CG == 2) {
-    const int64_t pairs = num_sms / 2, want = (g.total_tiles + 1) / 2;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2u * (unsigned)(want < pairs ? want : pairs));
-    cfg.blockDim = dim3(kSlabThreads);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute la[1];
-    la[0].id = cudaLaunchAttributeClusterDimension;
-    la[0].val.clusterDim.x = 2; la[0].val.clusterDim.y = 1; la[0].val.clusterDim.z = 1;
-    cfg.attrs = la;
-    cfg.numAttrs = 1;
-    prof_begin(st, &tok);
-    cudaError_t le = cudaLaunchKernelEx(&cfg, tc_slab_kernel<BN, RES, MBC, CG>, maps, g, ep);
-    if (le != cudaSuccess) {
-      set_error(std::string("slab pair launch failed: ") + cudaGetErrorString(le));
-      return AVVAD_ERR_CUDA;
-    }
-    AVVAD_LAUNCHED();
-    prof_end(st, tok, 0, flops);
-    return AVVAD_OK;
-  }
   const unsigned grid = (unsigned)(g.total_tiles < num_sms ? g.total_tiles : num_sms);
   prof_begin(st, &tok);
-  tc_slab_kernel<BN, RES, MBC, CG><<<grid, kSlabThreads, smem, st>>>(maps, g, ep);
+  tc_slab_kernel<64, MBC><<<grid, kSlabThreads, smem, st>>>(maps, g, ep);
   AVVAD_LAUNCHED();
   prof_end(st, tok, 0, flops);
   return AVVAD_OK;
-}
-
-// Packed two-frame variant (conv_slab2.cuh) for the 64 -> 64 channel layers: opt-in with AVVAD_SLAB2=1.  It issues
-// one sixth fewer MMAs but has to stream the weights; measured on B200 (layer1, 81,152 frames): 9.6 ms against 9.1 ms
-// for the resident-weight kernel on the same box -- layer1 moves 2.2 GB per launch and sits at ~65 % of the HBM
-// peak as well as ~58 % tensor-pipe activity, so fewer MMAs alone do not shorten it.
-static int slab2_mode() {
-  static int v = [] {
-    const char* e = getenv("AVVAD_SLAB2");
-    return e ? atoi(e) : 0;
-  }();
-  return v;
-}
-
-static int launch_slab2(const __nv_bfloat16* in, const __nv_bfloat16* w, const EpiParams& ep, int64_t n, int H,
-                        cudaStream_t st) {
-  Slab2Geom g{};
-  g.n_frames = n;
-  g.OH = H; g.OW = H; g.Wp = H + 1;
-  g.per_frame = (H + 1) * (H + 1);
-  g.total_tiles = (n + kSlab2Frames - 1) / kSlab2Frames;
-  g.box_bytes = (uint32_t)kSlab2Frames * g.per_frame * 128u;
-  const uint32_t rows = kSlab2Blocks * 128 + 2 * g.Wp + 2;
-  g.slab_bytes = (rows * 128u + 1023u) & ~1023u;
-  SlabMaps maps;
-  const uint32_t box[4] = {64, (uint32_t)g.Wp, (uint32_t)(H + 1), (uint32_t)kSlab2Frames};
-  const uint32_t estr[4] = {1, 1, 1, 1};
-  int rc = encode_act_map(&maps.a, in, 64, H, H, n, box, estr);
-  if (rc) return rc;
-  rc = encode_weight_map(&maps.b, w, (uint64_t)9 * 64, 64, 64);
-  if (rc) return rc;
-  const size_t smem = 1024 + 2 * (size_t)g.slab_bytes + kSlab2WStages * kSlab2WTile + 8 * 24 + 16 + 64 * 4;
-  static PerDeviceOnce once;
-  AVVAD_CUDA(once.run([] {
-    return cudaFuncSetAttribute(tc_slab2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-  }));
-  static int num_sms = [] {
-    int dev = 0, v = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev);
-    return v > 0 ? v : 148;
-  }();
-  const unsigned grid = (unsigned)(g.total_tiles < num_sms ? g.total_tiles : num_sms);
-  const double flops = 2.0 * (double)n * H * H * 64 * 9.0 * 64;
-  void* tok = nullptr;
-  prof_begin(st, &tok);
-  tc_slab2_kernel<<<grid, kSlabThreads, smem, st>>>(maps, g, ep);
-  AVVAD_LAUNCHED();
-  prof_end(st, tok, 0, flops);
-  return AVVAD_OK;
-}
-
-// two frames must fit five 128-row blocks and the slabs must fit shared memory: true for the 17x17 maps of layer1
-static bool slab2_fits(int H, int Cin, int Cout) {
-  if (slab2_mode() == 0 || Cin != 64 || Cout != 64) return false;
-  const int Wp = H + 1, per_frame = (H + 1) * (H + 1);
-  const int last = per_frame + (H - 1) * Wp + (H - 1);  // last valid GEMM row of the second frame
-  const size_t slab = ((size_t)(kSlab2Blocks * 128 + 2 * Wp + 2) * 128 + 1023) / 1024 * 1024;
-  return last < kSlab2Blocks * 128 && last >= (kSlab2Blocks - 1) * 128 &&
-         (size_t)kSlab2Frames * per_frame * 128 <= slab &&
-         1024 + 2 * slab + kSlab2WStages * kSlab2WTile + 512 <= 227 * 1024;
 }
 
 int launch_slab_conv(const __nv_bfloat16* in, const __nv_bfloat16* w, const EpiParams& ep, int64_t n, int H, int Cin,
                      int Cout, cudaStream_t st) {
-  if (slab2_fits(H, Cin, Cout)) return launch_slab2(in, w, ep, n, H, st);
   SlabPlan p;
   if (!plan(H, Cin, Cout, &p)) {
     set_error("slab conv: no feasible plan");
@@ -224,22 +108,16 @@ int launch_slab_conv(const __nv_bfloat16* in, const __nv_bfloat16* w, const EpiP
   g.total_tiles = ((n + p.F - 1) / p.F) * g.nb * g.n_tiles;
   g.slab_rows = p.mb * 128 + 2 * g.Wp + 2;
   g.slab_tx = (uint32_t)p.F * g.Hs * g.Wp * 128u;
-  g.use_base_offset = slab_bo();
-  g.b_stages = p.b_stages;
   SlabMaps maps;
   const uint32_t box[4] = {64, (uint32_t)g.Wp, (uint32_t)g.Hs, (uint32_t)p.F};
   const uint32_t estr[4] = {1, 1, 1, 1};
   int rc = encode_act_map(&maps.a, in, Cin, H, H, n, box, estr);
   if (rc) return rc;
-  const bool pair = p.resident && slab_pair() && g.n_tiles == 1;
-  rc = encode_weight_map(&maps.b, w, (uint64_t)9 * Cin, (uint64_t)Cout, (uint32_t)(pair ? p.bn / 2 : p.bn));
+  rc = encode_weight_map(&maps.b, w, (uint64_t)9 * Cin, (uint64_t)Cout, (uint32_t)p.bn);
   if (rc) return rc;
   const double flops = 2.0 * (double)n * H * H * Cout * 9.0 * Cin;
-  if (pair && p.mb == 3) return launch_k<64, true, 3, 2>(maps, g, ep, p.smem, flops, st);
-  if (pair) return launch_k<64, true, 0, 2>(maps, g, ep, p.smem, flops, st);
-  if (p.resident && p.mb == 3) return launch_k<64, true, 3>(maps, g, ep, p.smem, flops, st);
-  if (p.resident) return launch_k<64, true>(maps, g, ep, p.smem, flops, st);
-  return launch_k<64, false>(maps, g, ep, p.smem, flops, st);
+  if (p.mb == 3) return launch_k<3>(maps, g, ep, p.smem, flops, st);
+  return launch_k(maps, g, ep, p.smem, flops, st);
 }
 
 // ---- fused BasicBlock of layer1 (conv_block.cuh); AVVAD_BLOCK17=0 keeps the two slab convolutions

@@ -4,10 +4,9 @@
 // (r,s) simply starts (r*(OW+2)+s) rows further down.  GEMM rows are positions of the padded grid, so a few rows
 // per image row (the two border columns) and per band (the two border rows) are computed and dropped -- in exchange
 // the A operand crosses L2 once instead of nine times and one weight K-block feeds `mb` accumulator blocks.
-// Weights are either fully resident in shared memory (layer1: 9 x [64][64] bf16 = 72 KB, loaded once per CTA) or
-// streamed through a ring (wider layers).
+// The weights stay resident in shared memory (64 -> 64 channels: 9 x [64][64] bf16 = 72 KB, loaded once per CTA).
 //
-//   warp 0  : TMA producer (slabs; weight ring or the one-off resident weight load)
+//   warp 0  : TMA producer (the one-off weight load, then the slabs)
 //   warp 1  : TMEM alloc + tcgen05.mma issue (mb accumulator blocks x 9 taps x cpb channel blocks x 4 K16 steps)
 //   warps 2-9: two epilogue groups (TMEM -> bias / residual / ReLU -> NHWC bf16), accumulators double-buffered
 #pragma once
@@ -24,8 +23,6 @@ struct SlabGeom {
   int OH, OW, Wp, Hs, hb, F, nb, mb, cpb, n_tiles, N;
   int slab_rows;        // rows allocated per slab buffer (>= mb*128 + 2*Wp + 2)
   uint32_t slab_tx;     // bytes one slab TMA box delivers
-  int use_base_offset;  // descriptor base_offset = (start >> 7) & 7 for row-shifted starts
-  int b_stages;         // weight ring depth (streamed mode)
 };
 
 struct SlabMaps {
@@ -33,44 +30,27 @@ struct SlabMaps {
   CUtensorMap b;
 };
 
-__device__ __forceinline__ uint64_t make_sw128_desc_bo(uint32_t saddr, int use_bo) {
-  uint64_t d = make_sw128_desc(saddr);
-  if (use_bo) d |= (uint64_t)((saddr >> 7) & 7u) << 49;
-  return d;
-}
-
-// dynamic smem: [slab 0][slab 1][weights: resident KB tiles or ring][barriers]
+// dynamic smem: [slab 0][slab 1][weights: KB resident tiles][barriers, TMEM slot, bias]
 // MBC > 0: the number of accumulator blocks per tile is a compile-time constant (3 for the 17x17 maps of layer1), so the
 // 9 x MBC x 4 MMAs of a channel block are straight-line code with immediate descriptor offsets -- the issuing thread
 // was spending ~45 % of its slots on short-scoreboard stalls (constant-bank reloads, loop arithmetic) between
 // 48-cycle MMAs.  MBC = 0 keeps the generic loops.
-// CG = 2 (resident weights only): a CTA PAIR works on two consecutive tiles at once as M = 256 MMAs (tcgen05
-// cta_group::2).  Each CTA stages the slab of ITS tile and keeps HALF of the weights (BN/2 output channels of every
-// tap); both tensor cores read both halves, so a K16 step reads 5 KB of operands per SM instead of 6 KB: 40 cycles
-// instead of 48 for 32 cycles of math at N = 64.
-template <int BN, bool RESIDENT_B, int MBC = 0, int CG = 1>
+template <int BN, int MBC = 0>
 __global__ void __launch_bounds__(kSlabThreads)
 tc_slab_kernel(const __grid_constant__ SlabMaps maps, const SlabGeom g, const EpiParams ep) {
-  static_assert(CG == 1 || RESIDENT_B, "pair mode needs resident weights");
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;
   uint8_t* smem = smem_raw + (base - raw);
   const uint32_t slab_bytes = ((uint32_t)g.slab_rows * 128u + 1023u) & ~1023u;
-  const uint32_t b_tile = (BN / CG) * 128u;  // per CTA
-  const uint32_t rank = (CG == 2) ? pair_rank() : 0u;
-  // pair mode: cluster c works on tiles 2c + rank, 2c + rank + 2 * clusters, ...; a tile index past the end is harmless
-  // (TMA zero-fills frames >= n_frames, the epilogue stores nothing for them)
-  const int64_t tile0 = (CG == 2) ? (int64_t)(blockIdx.x >> 1) * 2 + rank : (int64_t)blockIdx.x;
-  const int64_t tile_step = (int64_t)gridDim.x;  // pair mode: 2 tiles per cluster and round
-  const int64_t tile_end = (CG == 2) ? ((g.total_tiles + 1) / 2) * 2 : g.total_tiles;
+  const uint32_t b_tile = BN * 128u;
   const int KB = 9 * g.cpb;
-  const int nB = RESIDENT_B ? KB : g.b_stages;
   const uint32_t w_base = base + 2 * slab_bytes;
-  const uint32_t bar0 = w_base + (uint32_t)nB * b_tile;
-  // barriers: slab_full[2] | slab_empty[2] | tfull[2] | tempty[2] | b_full[nB'] | b_empty[nB']  (nB' <= 8 when streamed)
+  const uint32_t bar0 = w_base + (uint32_t)KB * b_tile;
+  // barriers: slab_full[2] | slab_empty[2] | tfull[2] | tempty[2] | b_full, in 192 reserved bytes; then the TMEM slot
+  // and, 16-byte aligned, the bias
   auto BAR = [&](int i) { return bar0 + 8u * (uint32_t)i; };
-  const int kBarBFull = 8, kBarBEmpty = 16;  // streamed ring: up to 8 stages; resident: b_full = BAR(8)
+  const int kBarBFull = 8;
   volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem + (bar0 - base) + 8 * 24);
 
   const int warp = threadIdx.x >> 5;
@@ -84,63 +64,36 @@ tc_slab_kernel(const __grid_constant__ SlabMaps maps, const SlabGeom g, const Ep
       mbar_init(BAR(0 + i), 1);              // slab full (expect_tx)
       mbar_init(BAR(2 + i), 1);              // slab empty (tcgen05.commit)
       mbar_init(BAR(4 + i), 1);              // tmem full
-      mbar_init(BAR(6 + i), CG * kSlabEpiWarps);  // tmem empty (pair mode: both CTAs' warps, on the leader)
+      mbar_init(BAR(6 + i), kSlabEpiWarps);  // tmem empty
     }
-    for (int i = 0; i < 8; ++i) {
-      mbar_init(BAR(kBarBFull + i), 1);
-      mbar_init(BAR(kBarBEmpty + i), 1);
-    }
+    mbar_init(BAR(kBarBFull), 1);
     fence_barrier_init();
     tma_prefetch_desc(&maps.a);
     tma_prefetch_desc(&maps.b);
   }
   if (warp == 1) {
-    if (CG == 2) {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                       smem_u32(const_cast<uint32_t*>(tmem_slot))),
-                   "r"(tmem_cols)
-                   : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    } else {
-      tmem_alloc(smem_u32(const_cast<uint32_t*>(tmem_slot)), tmem_cols);
-      tmem_relinquish();
-    }
+    tmem_alloc(smem_u32(const_cast<uint32_t*>(tmem_slot)), tmem_cols);
+    tmem_relinquish();
   }
   {  // folded-BN bias -> shared memory (zero when absent); the region sits behind the barriers
     float* bs = reinterpret_cast<float*>(smem + (bar0 - base) + 8 * 24 + 16);
     for (int i = threadIdx.x; i < g.N; i += kSlabThreads) bs[i] = ep.bias ? ep.bias[i] : 0.f;
   }
-  if (CG == 2 && warp == 0) {
-    // pair mode: this CTA's half of the weights is loaded (and waited for) before the pair synchronises, so the leader's
-    // MMAs may read both halves
-    if (elect_one_sync()) {
-      mbar_arrive_expect_tx(BAR(kBarBFull), (uint32_t)KB * b_tile);
-      for (int kb = 0; kb < KB; ++kb)
-        tma_load_2d(w_base + kb * b_tile, &maps.b, kb * BK, (int)rank * (BN / CG), BAR(kBarBFull));
-    }
-    __syncwarp();
-    mbar_wait(BAR(kBarBFull), 0);
-  }
   tc_fence_before();
   __syncthreads();
-  if (CG == 2) pair_sync();
   tc_fence_after();
   const uint32_t tmem_acc = *tmem_slot;
-  const uint32_t bar0_leader = (CG == 2) ? pair_mapa(bar0, 0) : bar0;
 
   if (warp == 0) {
     // ================= TMA producer (warp-converged; one elected lane issues) =================
-    if (RESIDENT_B && CG == 1) {
-      // all weight K blocks, once (n_tiles == 1 in this mode)
-      if (elect_one_sync()) {
-        mbar_arrive_expect_tx(BAR(kBarBFull), (uint32_t)KB * b_tile);
-        for (int kb = 0; kb < KB; ++kb) tma_load_2d(w_base + kb * b_tile, &maps.b, kb * BK, 0, BAR(kBarBFull));
-      }
-      __syncwarp();
+    // all weight K blocks, once (n_tiles == 1)
+    if (elect_one_sync()) {
+      mbar_arrive_expect_tx(BAR(kBarBFull), (uint32_t)KB * b_tile);
+      for (int kb = 0; kb < KB; ++kb) tma_load_2d(w_base + kb * b_tile, &maps.b, kb * BK, 0, BAR(kBarBFull));
     }
-    uint32_t si = 0, bi = 0;  // slab / weight-ring counters
-    for (int64_t tile = tile0; tile < tile_end; tile += tile_step) {
-      const int n_base = (int)(tile % g.n_tiles) * BN;
+    __syncwarp();
+    uint32_t si = 0;  // slab counter
+    for (int64_t tile = blockIdx.x; tile < g.total_tiles; tile += gridDim.x) {
       const int64_t mt = tile / g.n_tiles;
       const int band = (int)(mt % g.nb);
       const int n0 = (int)((mt / g.nb) * g.F);
@@ -149,38 +102,19 @@ tc_slab_kernel(const __grid_constant__ SlabMaps maps, const SlabGeom g, const Ep
         const int sb = si & 1;
         mbar_wait(BAR(2 + sb), ((si >> 1) & 1u) ^ 1u);
         if (elect_one_sync()) {
-          if (CG == 2) {
-            if (rank == 0) mbar_arrive_expect_tx(BAR(0 + sb), 2 * g.slab_tx);  // both CTAs' slabs
-            tma_load_4d_2sm(base + sb * slab_bytes, &maps.a, cb * BK, -1, hstart - 1, n0, bar0_leader + 8u * (uint32_t)sb);
-          } else {
-            mbar_arrive_expect_tx(BAR(0 + sb), g.slab_tx);
-            tma_load_4d(base + sb * slab_bytes, &maps.a, cb * BK, -1, hstart - 1, n0, BAR(0 + sb));
-          }
+          mbar_arrive_expect_tx(BAR(0 + sb), g.slab_tx);
+          tma_load_4d(base + sb * slab_bytes, &maps.a, cb * BK, -1, hstart - 1, n0, BAR(0 + sb));
         }
         __syncwarp();
-        if (!RESIDENT_B) {
-          for (int tap = 0; tap < 9; ++tap, ++bi) {
-            const int bs = bi % g.b_stages;
-            mbar_wait(BAR(kBarBEmpty + bs), ((bi / g.b_stages) & 1u) ^ 1u);
-            if (elect_one_sync()) {
-              mbar_arrive_expect_tx(BAR(kBarBFull + bs), b_tile);
-              tma_load_2d(w_base + bs * b_tile, &maps.b, (tap * g.cpb + cb) * BK, n_base, BAR(kBarBFull + bs));
-            }
-            __syncwarp();
-          }
-        }
       }
     }
   } else if (warp == 1) {
     // ================= MMA issuer (warp-converged; one elected lane issues MMAs and commits) =================
-    constexpr uint32_t idesc = (CG == 2) ? make_idesc_m256(BN) : make_idesc(BN);
-    uint32_t si = 0, bi = 0, tl = 0;
-    if (RESIDENT_B && CG == 1) {
-      mbar_wait(BAR(kBarBFull), 0);
-      tc_fence_after();
-    }
-    if (CG == 1 || rank == 0)  // pair mode: the leader issues for both CTAs
-    for (int64_t tile = tile0; tile < tile_end; tile += tile_step, ++tl) {
+    constexpr uint32_t idesc = make_idesc(BN);
+    uint32_t si = 0, tl = 0;
+    mbar_wait(BAR(kBarBFull), 0);
+    tc_fence_after();
+    for (int64_t tile = blockIdx.x; tile < g.total_tiles; tile += gridDim.x, ++tl) {
       const uint32_t acc = tl & 1u, aph = (tl >> 1) & 1u;
       mbar_wait(BAR(6 + acc), aph ^ 1u);
       tc_fence_after();
@@ -189,93 +123,47 @@ tc_slab_kernel(const __grid_constant__ SlabMaps maps, const SlabGeom g, const Ep
         mbar_wait(BAR(0 + sb), (si >> 1) & 1u);
         tc_fence_after();
         const uint32_t slab_lo = desc_lo(base + sb * slab_bytes);
-        if (RESIDENT_B) {
-          // every tap of this channel block in one elected region: 9 x mb x 4 MMAs issued back to back
-          if (elect_one_sync()) {
-            const int Wp = g.Wp, cpb = g.cpb;
-            const uint32_t d0 = tmem_acc + acc * acc_cols;
-            if (MBC > 0) {
+        // every tap of this channel block in one elected region: 9 x mb x 4 MMAs issued back to back
+        if (elect_one_sync()) {
+          const int Wp = g.Wp, cpb = g.cpb;
+          const uint32_t d0 = tmem_acc + acc * acc_cols;
+          if (MBC > 0) {
 #pragma unroll
-              for (int tap = 0; tap < 9; ++tap) {
-                const uint32_t w_lo = desc_lo(w_base + (uint32_t)(tap * cpb + cb) * b_tile);
-                const int fr = tap / 3, fs = tap - fr * 3;
-                // descriptor low words count 16-byte units: one slab row = 8, one accumulator block (128 rows) = 1024
-                const uint32_t a0 = slab_lo + (uint32_t)(fr * Wp + fs) * 8u;
-                const uint32_t first = (cb | tap) != 0;
-#pragma unroll
-                for (int m = 0; m < MBC; ++m) {
-                  if (CG == 2) {
-                    umma2_f16_lo2(d0 + m * BN, a0 + m * 1024u, w_lo, idesc, first, kDescHi);
-                    umma2_f16_lo2(d0 + m * BN, a0 + m * 1024u + 2, w_lo + 2, idesc, 1, kDescHi);
-                    umma2_f16_lo2(d0 + m * BN, a0 + m * 1024u + 4, w_lo + 4, idesc, 1, kDescHi);
-                    umma2_f16_lo2(d0 + m * BN, a0 + m * 1024u + 6, w_lo + 6, idesc, 1, kDescHi);
-                  } else {
-                    umma_f16_lo(d0 + m * BN, a0 + m * 1024u, w_lo, idesc, first);
-                    umma_f16_lo(d0 + m * BN, a0 + m * 1024u + 2, w_lo + 2, idesc, 1);
-                    umma_f16_lo(d0 + m * BN, a0 + m * 1024u + 4, w_lo + 4, idesc, 1);
-                    umma_f16_lo(d0 + m * BN, a0 + m * 1024u + 6, w_lo + 6, idesc, 1);
-                  }
-                }
-              }
-            } else {
-              const int mb = g.mb;
-#pragma unroll 1
-              for (int tap = 0; tap < 9; ++tap) {
-                const uint32_t w_lo = desc_lo(w_base + (uint32_t)(tap * cpb + cb) * b_tile);
-                const int fr = tap / 3, fs = tap - fr * 3;
-                uint32_t a_lo = slab_lo + (uint32_t)(fr * Wp + fs) * 8u;
-                uint32_t d_tmem = d0;
-                const uint32_t first = (cb | tap) != 0;
-                for (int m = 0; m < mb; ++m, a_lo += 1024u, d_tmem += BN) {
-                  if (CG == 2) {
-                    umma2_f16_lo2(d_tmem, a_lo, w_lo, idesc, first, kDescHi);
-                    umma2_f16_lo2(d_tmem, a_lo + 2, w_lo + 2, idesc, 1, kDescHi);
-                    umma2_f16_lo2(d_tmem, a_lo + 4, w_lo + 4, idesc, 1, kDescHi);
-                    umma2_f16_lo2(d_tmem, a_lo + 6, w_lo + 6, idesc, 1, kDescHi);
-                  } else {
-                    umma_f16_lo(d_tmem, a_lo, w_lo, idesc, first);
-                    umma_f16_lo(d_tmem, a_lo + 2, w_lo + 2, idesc, 1);
-                    umma_f16_lo(d_tmem, a_lo + 4, w_lo + 4, idesc, 1);
-                    umma_f16_lo(d_tmem, a_lo + 6, w_lo + 6, idesc, 1);
-                  }
-                }
-              }
-            }
-            if (CG == 2) {
-              umma2_commit_mc2(BAR(2 + sb));
-              if (cb == g.cpb - 1) umma2_commit_mc2(BAR(4 + acc));
-            } else {
-              umma_commit(BAR(2 + sb));
-              if (cb == g.cpb - 1) umma_commit(BAR(4 + acc));
-            }
-          }
-          __syncwarp();
-        } else {
-          for (int tap = 0; tap < 9; ++tap, ++bi) {
-            const int bs = bi % g.b_stages;
-            mbar_wait(BAR(kBarBFull + bs), (bi / g.b_stages) & 1u);
-            tc_fence_after();
-            if (elect_one_sync()) {
-              const uint32_t w_lo = desc_lo(w_base + bs * b_tile);
+            for (int tap = 0; tap < 9; ++tap) {
+              const uint32_t w_lo = desc_lo(w_base + (uint32_t)(tap * cpb + cb) * b_tile);
               const int fr = tap / 3, fs = tap - fr * 3;
-              uint32_t a_lo = slab_lo + (uint32_t)(fr * g.Wp + fs) * 8u;
-              uint32_t d_tmem = tmem_acc + acc * acc_cols;
+              // descriptor low words count 16-byte units: one slab row = 8, one accumulator block (128 rows) = 1024
+              const uint32_t a0 = slab_lo + (uint32_t)(fr * Wp + fs) * 8u;
               const uint32_t first = (cb | tap) != 0;
-              for (int m = 0; m < g.mb; ++m, a_lo += 1024u, d_tmem += BN) {
+#pragma unroll
+              for (int m = 0; m < MBC; ++m) {
+                umma_f16_lo(d0 + m * BN, a0 + m * 1024u, w_lo, idesc, first);
+                umma_f16_lo(d0 + m * BN, a0 + m * 1024u + 2, w_lo + 2, idesc, 1);
+                umma_f16_lo(d0 + m * BN, a0 + m * 1024u + 4, w_lo + 4, idesc, 1);
+                umma_f16_lo(d0 + m * BN, a0 + m * 1024u + 6, w_lo + 6, idesc, 1);
+              }
+            }
+          } else {
+            const int mb = g.mb;
+#pragma unroll 1
+            for (int tap = 0; tap < 9; ++tap) {
+              const uint32_t w_lo = desc_lo(w_base + (uint32_t)(tap * cpb + cb) * b_tile);
+              const int fr = tap / 3, fs = tap - fr * 3;
+              uint32_t a_lo = slab_lo + (uint32_t)(fr * Wp + fs) * 8u;
+              uint32_t d_tmem = d0;
+              const uint32_t first = (cb | tap) != 0;
+              for (int m = 0; m < mb; ++m, a_lo += 1024u, d_tmem += BN) {
                 umma_f16_lo(d_tmem, a_lo, w_lo, idesc, first);
                 umma_f16_lo(d_tmem, a_lo + 2, w_lo + 2, idesc, 1);
                 umma_f16_lo(d_tmem, a_lo + 4, w_lo + 4, idesc, 1);
                 umma_f16_lo(d_tmem, a_lo + 6, w_lo + 6, idesc, 1);
               }
-              umma_commit(BAR(kBarBEmpty + bs));
-              if (tap == 8) {
-                umma_commit(BAR(2 + sb));
-                if (cb == g.cpb - 1) umma_commit(BAR(4 + acc));
-              }
             }
-            __syncwarp();
           }
+          umma_commit(BAR(2 + sb));
+          if (cb == g.cpb - 1) umma_commit(BAR(4 + acc));
         }
+        __syncwarp();
       }
     }
   } else {
@@ -317,7 +205,7 @@ tc_slab_kernel(const __grid_constant__ SlabMaps maps, const SlabGeom g, const Ep
     const __nv_bfloat16* resp = ep.residual;
     __nv_bfloat16* outp = reinterpret_cast<__nv_bfloat16*>(ep.C);
     const bool relu = ep.relu != 0;
-    for (int64_t tile = tile0; tile < tile_end; tile += tile_step, ++tl) {
+    for (int64_t tile = blockIdx.x; tile < g.total_tiles; tile += gridDim.x, ++tl) {
       const int n_base = (int)(tile % g.n_tiles) * BN;
       const int64_t mt = tile / g.n_tiles;
       const int band = (int)(mt % g.nb);
@@ -388,20 +276,15 @@ tc_slab_kernel(const __grid_constant__ SlabMaps maps, const SlabGeom g, const Ep
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if (CG == 2) pair_arrive(bar0_leader + 8u * (uint32_t)(6 + acc));
-        else mbar_arrive(BAR(6 + acc));
-      }
+      if (lane == 0) mbar_arrive(BAR(6 + acc));
     }
   }
 
   tc_fence_before();
   __syncthreads();
-  if (CG == 2) pair_sync();
   if (warp == 1) {
     __syncwarp();
-    if (CG == 2) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_acc), "r"(tmem_cols) : "memory");
-    else tmem_dealloc(tmem_acc, tmem_cols);
+    tmem_dealloc(tmem_acc, tmem_cols);
   }
 }
 

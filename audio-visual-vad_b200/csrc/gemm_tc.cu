@@ -188,14 +188,6 @@ extern "C" int avvad_profile_clear(void) {
   return AVVAD_OK;
 }
 
-static int bn_override() {
-  static int v = [] {
-    const char* e = getenv("AVVAD_BN");
-    return e ? atoi(e) : 0;
-  }();
-  return v;
-}
-
 extern "C" int avvad_gemm_bf16(const void* A, int64_t lda, const void* W, int64_t ldw, const float* bias, void* Cp,
                                int64_t ldc, int c_is_bf16, int relu, int64_t M, int64_t N, int64_t K, void* stream) {
   AVVAD_CHECK_ARG(A && W && Cp, "null pointer");
@@ -206,7 +198,7 @@ extern "C" int avvad_gemm_bf16(const void* A, int64_t lda, const void* W, int64_
   ep.ldc = ldc;
   ep.relu = relu;
   return tc::gemm_dispatch((const __nv_bfloat16*)A, lda, (const __nv_bfloat16*)W, ldw, M, (int)N, (int)K, ep,
-                           c_is_bf16 ? tc::EPI_BF16 : tc::EPI_F32, bn_override(), (cudaStream_t)stream);
+                           c_is_bf16 ? tc::EPI_BF16 : tc::EPI_F32, 0, (cudaStream_t)stream);
 }
 
 extern "C" int avvad_conv2d_nhwc_bf16(const void* in, const void* w, const float* bias, const void* residual,
@@ -235,7 +227,7 @@ extern "C" int avvad_conv2d_nhwc_bf16(const void* in, const void* w, const float
     return tc::launch_slab_conv((const __nv_bfloat16*)in, (const __nv_bfloat16*)w, ep, n, H, Cin, Cout,
                                 (cudaStream_t)stream);
   return tc::launch_tma_conv((const __nv_bfloat16*)in, (const __nv_bfloat16*)w, ep, n, H, W, Cin, Cout, R, S, stride,
-                             pad, bn_override(), (cudaStream_t)stream);
+                             pad, 0, (cudaStream_t)stream);
 }
 
 extern "C" int avvad_conv2d_nhwc_bf16_dual(const void* in, const void* in2, const void* w, const float* bias, void* out,
@@ -258,7 +250,7 @@ extern "C" int avvad_conv2d_nhwc_bf16_dual(const void* in, const void* in2, cons
   so.in2 = (const __nv_bfloat16*)in2;
   so.H2 = H2; so.W2 = W2; so.Cin2 = Cin2; so.stride2 = stride2;
   return tc::launch_tma_conv((const __nv_bfloat16*)in, (const __nv_bfloat16*)w, ep, n, H, W, Cin, Cout, R, S, stride,
-                             pad, bn_override(), (cudaStream_t)stream, 0, 0.0, &so);
+                             pad, 0, (cudaStream_t)stream, 0, 0.0, &so);
 }
 
 extern "C" int avvad_pack_rows_bf16(const float* src, int64_t ld_src, void* dst, int64_t ld_dst, int64_t col_off,

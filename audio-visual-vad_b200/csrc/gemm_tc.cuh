@@ -26,7 +26,6 @@ struct EpiParams {
   __nv_bfloat16* hseq;    // [B][T][H] layer output (zero for t >= len_b)
   const int32_t* lengths;
   int t, T, H4;
-  int debug;  // experiments only (AVVAD_EPI_DEBUG): bit 0 = skip the output stores of the fast epilogue
 };
 
 // ---- PTX wrappers ---------------------------------------------------------------------------------

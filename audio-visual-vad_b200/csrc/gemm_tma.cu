@@ -123,19 +123,11 @@ static bool pair_enabled() {
   }();
   return v != 0;
 }
-// AVVAD_CG2_128 = 0: N = 128 tiles stay on single CTAs; 1 / 2 (default): pairs with one / two blocks per CTA
-static int pair128_mode() {
-  static int v = [] {
-    const char* e = getenv("AVVAD_CG2_128");
-    return e ? atoi(e) : 2;
-  }();
-  return v;
-}
 // kb = K blocks of the launch: short K loops (layer2's first convolution, K = 576) measured slower on pairs of
 // two-block CTAs (307 us against 266 us per 20,288-frame pass), so N = 128 pairs need at least 16 K blocks
 static bool use_pair(int bn, int ksplit, int epi_mode, int kb) {
   if (!pair_enabled() || ksplit > 1 || epi_mode == EPI_LSTM) return false;
-  return bn == 256 || (bn == 128 && pair128_mode() != 0 && kb >= 16);
+  return bn == 256 || (bn == 128 && kb >= 16);
 }
 
 template <int BN, int KE = 64, int MB = 1, int CG = 1>
@@ -162,12 +154,6 @@ static int launch_bn(const TmaMaps& maps, TmaGeom g, const EpiParams& ep, int ep
     return n > 0 ? n : 148;
   }();
   if (g.total_tiles <= 0) return AVVAD_OK;
-  static int epi_debug = [] {
-    const char* e = getenv("AVVAD_EPI_DEBUG");
-    return e ? atoi(e) : 0;
-  }();
-  EpiParams epd = ep;
-  epd.debug = epi_debug;
   void* tok = nullptr;
   if (CG == 2) {
     int64_t pairs = num_sms / 2;
@@ -183,7 +169,7 @@ static int launch_bn(const TmaMaps& maps, TmaGeom g, const EpiParams& ep, int ep
     cfg.attrs = la;
     cfg.numAttrs = 1;
     prof_begin(st, &tok);
-    cudaError_t le = cudaLaunchKernelEx(&cfg, tc_tma_kernel<BN, KE, MB, CG>, maps, g, epd, epi_mode);
+    cudaError_t le = cudaLaunchKernelEx(&cfg, tc_tma_kernel<BN, KE, MB, CG>, maps, g, ep, epi_mode);
     if (le != cudaSuccess) {
       set_error(std::string("pair launch failed: ") + cudaGetErrorString(le));
       return AVVAD_ERR_CUDA;
@@ -196,7 +182,7 @@ static int launch_bn(const TmaMaps& maps, TmaGeom g, const EpiParams& ep, int ep
   if (g.grid_cap > 0 && g.grid_cap < resident) resident = g.grid_cap;
   const unsigned grid = (unsigned)(g.total_tiles < resident ? g.total_tiles : resident);
   prof_begin(st, &tok);
-  tc_tma_kernel<BN, KE, MB, CG><<<grid, kTmaThreads, C::kSmemBytes, st>>>(maps, g, epd, epi_mode);
+  tc_tma_kernel<BN, KE, MB, CG><<<grid, kTmaThreads, C::kSmemBytes, st>>>(maps, g, ep, epi_mode);
   AVVAD_LAUNCHED();
   prof_end(st, tok, cat, flops);
   return AVVAD_OK;
@@ -206,19 +192,11 @@ static int dispatch(int bn, const TmaMaps& maps, const TmaGeom& g, const EpiPara
                     double flops, cudaStream_t st) {
   switch (bn) {
     case 64: return launch_bn<64>(maps, g, ep, epi_mode, cat, flops, st);
-    case 128: {
-      // two accumulator blocks per weight box unless AVVAD_MB=1 (see TmaCfg)
-      static int mb2 = [] {
-        const char* e = getenv("AVVAD_MB");
-        return (e && atoi(e) == 1) ? 0 : 1;
-      }();
-      if (g.pair) {
-        if (pair128_mode() == 1) return launch_bn<128, 64, 1, 2>(maps, g, ep, epi_mode, cat, flops, st);
-        return launch_bn<128, 64, 2, 2>(maps, g, ep, epi_mode, cat, flops, st);
-      }
-      if (mb2 && epi_mode != EPI_LSTM) return launch_bn<128, 64, 2>(maps, g, ep, epi_mode, cat, flops, st);
+    case 128:
+      // two accumulator blocks per weight box (see TmaCfg); the per-step LSTM epilogue keeps one
+      if (g.pair) return launch_bn<128, 64, 2, 2>(maps, g, ep, epi_mode, cat, flops, st);
+      if (epi_mode != EPI_LSTM) return launch_bn<128, 64, 2>(maps, g, ep, epi_mode, cat, flops, st);
       return launch_bn<128>(maps, g, ep, epi_mode, cat, flops, st);
-    }
     case 256:
       if (g.pair) return launch_bn<256, 64, 1, 2>(maps, g, ep, epi_mode, cat, flops, st);
       return launch_bn<256>(maps, g, ep, epi_mode, cat, flops, st);

@@ -324,13 +324,9 @@ tc_tma_kernel(const __grid_constant__ TmaMaps maps, const __grid_constant__ TmaG
             tma_load_2d_2sm(sa + MB * C::kABytes, &maps.b, kb * KE, n_base, full);
           } else {
           const uint32_t full = bar0 + 8 * s;
-          // debug knobs (AVVAD_EPI_DEBUG, see DESIGN.md section 3): 4 = no A loads, 8 = no B loads (operands stay
-          // whatever shared memory held), 2 = no MMAs, 1 = no stores -- to time the pipeline stages in isolation
-          const bool no_a = (ep.debug & 4) != 0, no_b = (ep.debug & 8) != 0;
-          mbar_arrive_expect_tx(full, (no_a ? 0u : bytes - g.bytesB) + (no_b ? 0u : g.bytesB));
+          mbar_arrive_expect_tx(full, bytes);
 #pragma unroll
           for (int mb = 0; mb < MB; ++mb) {
-            if (no_a) continue;
             if (g.mode == 0) {
               if (g.tm_bp)
                 tma_load_4d(sa + mb * C::kABytes, &maps.a[0], kb * KE, (int)(t[mb].n0 % g.tm_bp),
@@ -342,7 +338,7 @@ tc_tma_kernel(const __grid_constant__ TmaMaps maps, const __grid_constant__ TmaG
                           t[mb].hstart * g.stride + fr - g.pad, (int)t[mb].n0, full);
             }
           }
-          if (!no_b) tma_load_2d(sa + MB * C::kABytes, &maps.b, kb * KE, n_base, full);
+          tma_load_2d(sa + MB * C::kABytes, &maps.b, kb * KE, n_base, full);
           }
         }
         __syncwarp();
@@ -404,7 +400,6 @@ tc_tma_kernel(const __grid_constant__ TmaMaps maps, const __grid_constant__ TmaG
           const uint32_t b_lo = a0 + ((MB * C::kABytes) >> 4);
 #pragma unroll
           for (int mb = 0; mb < MB; ++mb) {
-            if (ep.debug & 2) continue;  // debug: feed + epilogue only
             const uint32_t a_lo = a0 + ((mb * C::kABytes) >> 4);
             const uint32_t d = d_tmem + mb * BN;
             if (CG == 2) {
@@ -551,7 +546,6 @@ tc_tma_kernel(const __grid_constant__ TmaMaps maps, const __grid_constant__ TmaG
                   for (int e = 0; e < 8; ++e)
                     o.v[e] = ep.relu ? pack_relu_bf16x2(f32[16 * c + 2 * e], f32[16 * c + 2 * e + 1])
                                      : pack_bf16x2(f32[16 * c + 2 * e], f32[16 * c + 2 * e + 1]);
-                  if ((ep.debug & 1) && o.v[0] != 0x12345678u) continue;
                   if (wide) {
                     st_global_256(cp + 16 * c, o);
                   } else {

@@ -377,15 +377,6 @@ extern "C" int avvad_resnet18_set_conv(avvad_resnet18* h, int layer, const float
   return AVVAD_OK;
 }
 
-// 0 disables the K-concatenated downsample branch (separate 1x1 launch + residual add, the pre-fusion path)
-static bool fuse_ds() {
-  static int v = [] {
-    const char* e = getenv("AVVAD_FUSE_DS");
-    return (e && atoi(e) == 0) ? 0 : 1;
-  }();
-  return v != 0 && tc::tma_available();
-}
-
 static const int kDsBlocks[3][2] = {{6, 7}, {11, 12}, {16, 17}};  // (conv_b, downsample) layer indices of stages 2-4
 
 static int build_fused(avvad_resnet18* h, cudaStream_t st) {
@@ -505,13 +496,12 @@ static const double kStageMac[4] = {42614784.0, 42467328.0, 52428800.0, 75497472
 
 // Runs the trunk on one chunk; stops after layer `upto` (20 = run everything).  Returns the buffer index holding the
 // last produced activation in *last.  Stage s = torchvision layer(s+1): two BasicBlocks, the first of stages 1-3 with
-// a stride-2 conv_a and a 1x1 downsample branch (K-concatenated into conv_b unless AVVAD_FUSE_DS=0).
+// a stride-2 conv_a and a 1x1 downsample branch, K-concatenated into conv_b (the layer-by-layer hook, upto == the
+// downsample layer, runs it as a separate 1x1 convolution added as the residual).
 static int run_trunk_chunk(avvad_resnet18* h, const StemInput& in, int64_t n, __nv_bfloat16* const buf[4], int upto,
                            int* last, cudaStream_t st) {
-  if (fuse_ds()) {
-    int frc = build_fused(h, st);
-    if (frc) return frc;
-  }
+  int frc = build_fused(h, st);
+  if (frc) return frc;
   // Note: running layer1/layer2 depth-first over L2-sized slices of the chunk was measured SLOWER (each persistent
   // launch pays a prologue and a tail; 512-frame slices cost +15 % on the convolutions), larger chunks are faster:
   // chunk 2048 -> 20288 frames = 36.3 -> 33.3 ms of convolutions per 81,152 frames.
@@ -559,7 +549,7 @@ static int run_trunk_chunk(avvad_resnet18* h, const StemInput& in, int64_t n, __
         if (rc) return rc;
         if (upto == la) { *last = o[0]; return AVVAD_OK; }
         const __nv_bfloat16* res = xin;
-        if (ds && fuse_ds() && upto != lds) {
+        if (ds && upto != lds) {
           // conv_b with the downsample branch appended along K: no 1x1 launch, no residual round trip
           const ConvSpec& sb = kSpecs[lb];
           const ConvSpec& sd = kSpecs[lds];

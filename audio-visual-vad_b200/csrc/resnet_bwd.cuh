@@ -549,12 +549,8 @@ static int conv_wgrad(const BwdCtx& c, int layer, const __nv_bfloat16* x, const 
   int64_t fc = c.chunk_pixels / pix_per_frame;
   if (fc < 1) fc = 1;
   // 64-column tiles (the split-K configuration the LSTM BPTT exercises) unless the GEMM is wide and tall enough for
-  // 256-column tiles (AVVAD_WGRAD_BN=64 forces the narrow tiles)
-  static const int bn_wide = [] {
-    const char* e = getenv("AVVAD_WGRAD_BN");
-    return e ? atoi(e) : 256;
-  }();
-  const int bn = (bn_wide == 256 && N % 256 == 0 && M >= 128) ? 256 : 64;
+  // 256-column tiles
+  const int bn = (N % 256 == 0 && M >= 128) ? 256 : 64;
   const int tiles = (int)(ceil_div(M, 128) * ceil_div(N, bn));
   bool first = true;
   for (int64_t f0 = 0; f0 < c.n; f0 += fc) {

@@ -34,9 +34,7 @@ def test_trunk_pairs_and_fused_block_bit_identical(tmp_path, n_frames, full):
     assert torch.equal(fast, plain)
     if full:
         block_only = _run("trunk_ab.py", [n_frames], {"AVVAD_CG2": "0"}, str(tmp_path / "blk.pt"))
-        slab_pairs = _run("trunk_ab.py", [n_frames], {"AVVAD_BLOCK17": "0", "AVVAD_SLAB_CG2": "1"}, str(tmp_path / "slabp.pt"))
         assert torch.equal(block_only, plain)
-        assert torch.equal(slab_pairs, plain)
 
 
 @pytest.mark.parametrize("B,T,full", [(256, 80, True), (200, 48, False), (300, 40, False), (64, 80, False)])
