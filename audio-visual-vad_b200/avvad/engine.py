@@ -60,8 +60,12 @@ def upsampled_length(n_src: int, num=FPS_NUM, den=FPS_DEN) -> int:
 
 
 def frontend_logpower(wave: torch.Tensor, n_samples, n_frames, t_max: int, mean: Optional[torch.Tensor],
-                      std: Optional[torch.Tensor], eps=1e-8, normalise=True, out: Optional[torch.Tensor] = None):
-    """(B,N) fp32 waveforms -> (B,t_max,513) standardised log-power features (SURVEY A1-A4)."""
+                      std: Optional[torch.Tensor], eps=1e-8, normalise=True, out: Optional[torch.Tensor] = None,
+                      peaks: Optional[torch.Tensor] = None):
+    """(B,N) fp32 waveforms -> (B,t_max,513) standardised log-power features (SURVEY A1-A4).
+
+    ``peaks`` (f32 (B,)): with ``normalise``, divide by these per-utterance peaks instead of max|x| over the samples
+    given -- a stream sees only part of the utterance."""
     L.require_cuda(wave)
     assert wave.dim() == 2 and wave.dtype == torch.float32
     wave = wave.contiguous()
@@ -70,11 +74,19 @@ def frontend_logpower(wave: torch.Tensor, n_samples, n_frames, t_max: int, mean:
     ns, nf = _i32(n_samples, dev), _i32(n_frames, dev)
     if out is None:
         out = torch.empty(B, t_max, 513, dtype=torch.float32, device=dev)
-    peak = torch.empty(B, dtype=torch.float32, device=dev)
+    mode = 0
+    if normalise:
+        mode = 2 if peaks is not None else 1
+    if peaks is not None:
+        peak = _f32(peaks.reshape(-1), dev)
+        if peak.numel() != B:
+            raise ValueError("frontend_logpower: one peak per utterance required")
+    else:
+        peak = torch.empty(B, dtype=torch.float32, device=dev)
     m = _f32(mean.reshape(-1), dev) if mean is not None else None
     s = _f32(std.reshape(-1), dev) if std is not None else None
     L.check(L.lib().avvad_frontend_logpower(L.ptr(wave), wave.stride(0), L.ptr(ns), L.ptr(nf), B, t_max,
-                                            1 if normalise else 0, L.ptr(m), L.ptr(s), eps, L.ptr(out), L.ptr(peak),
+                                            mode, L.ptr(m), L.ptr(s), eps, L.ptr(out), L.ptr(peak),
                                             L.stream_ptr()))
     return out
 
@@ -485,10 +497,13 @@ class Mcb:
                                           L.ptr(out_bf16), ld, L.ptr(out_f32), L.stream_ptr()))
 
     def forward_grouped(self, audio: torch.Tensor, video: torch.Tensor, lengths, t_max: int,
-                        out_bf16: Optional[torch.Tensor] = None, out_f32: Optional[torch.Tensor] = None):
+                        out_bf16: Optional[torch.Tensor] = None, out_f32: Optional[torch.Tensor] = None,
+                        norms_in: Optional[torch.Tensor] = None, norms_out: Optional[torch.Tensor] = None):
         """audio (B,t_max,513), video (B,t_max,512): every utterance normalised by its own L2 norm over its
         ``lengths[b]`` valid rows -- B stand-alone forward calls of the reference module in one launch
-        (scripts/evaluate_AV_net.py:186-236 calls the model once per utterance)."""
+        (scripts/evaluate_AV_net.py:186-236 calls the model once per utterance).  ``norms_in`` (f32 (B,)): use these
+        norms instead (a stream normalises every block of an utterance by one constant); ``norms_out`` (f32 (B,),
+        contiguous): receives the norms used."""
         L.require_cuda(audio, video)
         audio = audio.reshape(-1, 513).contiguous()
         video = video.reshape(-1, 512).contiguous()
@@ -502,8 +517,16 @@ class Mcb:
         nbytes = L.lib().avvad_mcb_grouped_workspace_bytes(B, t_max)
         ws = self.ws.get(nbytes, audio.device)
         ld = out_bf16.stride(-2) if out_bf16 is not None else 0
-        L.check(L.lib().avvad_mcb_forward_grouped(self.h, L.ptr(audio), L.ptr(video), B, t_max, L.ptr(lens), L.ptr(ws),
-                                                  ws.numel(), L.ptr(out_bf16), ld, L.ptr(out_f32), L.stream_ptr()))
+        nin = None
+        if norms_in is not None:
+            nin = _f32(norms_in.reshape(-1), audio.device)
+            if nin.numel() != B:
+                raise ValueError("forward_grouped: one norm per utterance required")
+        if norms_out is not None:
+            assert norms_out.dtype == torch.float32 and norms_out.is_contiguous() and norms_out.numel() == B
+        L.check(L.lib().avvad_mcb_forward_grouped_norms(self.h, L.ptr(audio), L.ptr(video), B, t_max, L.ptr(lens),
+                                                        L.ptr(nin), L.ptr(norms_out), L.ptr(ws), ws.numel(),
+                                                        L.ptr(out_bf16), ld, L.ptr(out_f32), L.stream_ptr()))
 
 
 def mcb_forward_train(mcb: "Mcb", audio, video, gamma, beta, running_mean, running_var, out_bf16, momentum=0.1):
@@ -562,21 +585,63 @@ class Lstm:
         """bf16 operand buffer (B,T,ld); columns >= input_size must stay zero."""
         return torch.zeros(B, T, self.ld, dtype=torch.bfloat16, device=device)
 
-    def forward(self, x_bf16: torch.Tensor, lengths, want_post=False, want_dec=False, want_last=False):
+    def forward(self, x_bf16: torch.Tensor, lengths, want_post=False, want_dec=False, want_last=False,
+                state: Optional["LstmState"] = None):
+        """With `state`, the recurrence continues from it and the call leaves each row's state after its
+        ``lengths[b]`` new steps there (rows with length 0 keep theirs)."""
         L.require_cuda(x_bf16)
         B, T, ld = x_bf16.shape
         assert ld == self.ld and x_bf16.is_contiguous() and x_bf16.dtype == torch.bfloat16
         dev = x_bf16.device
         lens = _i32(lengths, dev)
-        nbytes = L.lib().avvad_lstm_workspace_bytes(self.h, B, T)
+        if state is not None:
+            state.check(self, B, dev)
+            nbytes = L.lib().avvad_lstm_state_workspace_bytes(self.h, B, T)
+        else:
+            nbytes = L.lib().avvad_lstm_workspace_bytes(self.h, B, T)
         ws = self.ws.get(nbytes, dev)
         logits = torch.empty(B, T, self.y_dim, dtype=torch.float32, device=dev)
         post = torch.empty_like(logits) if want_post else None
         dec = torch.empty(B, T, self.y_dim, dtype=torch.int32, device=dev) if want_dec else None
         last = torch.empty(B, self.y_dim, dtype=torch.float32, device=dev) if want_last else None
-        L.check(L.lib().avvad_lstm_forward(self.h, L.ptr(x_bf16), L.ptr(lens), B, T, L.ptr(ws), ws.numel(),
-                                           L.ptr(logits), L.ptr(post), L.ptr(dec), L.ptr(last), L.stream_ptr()))
+        if state is not None:
+            L.check(L.lib().avvad_lstm_forward_state(self.h, L.ptr(x_bf16), L.ptr(lens), B, T, L.ptr(state.h),
+                                                     L.ptr(state.c), L.ptr(state.h), L.ptr(state.c), L.ptr(ws),
+                                                     ws.numel(), L.ptr(logits), L.ptr(post), L.ptr(dec), L.ptr(last),
+                                                     L.stream_ptr()))
+        else:
+            L.check(L.lib().avvad_lstm_forward(self.h, L.ptr(x_bf16), L.ptr(lens), B, T, L.ptr(ws), ws.numel(),
+                                               L.ptr(logits), L.ptr(post), L.ptr(dec), L.ptr(last), L.stream_ptr()))
         return logits, post, dec, last
+
+
+class LstmState:
+    """Recurrent state of an :class:`Lstm` over ``B`` rows, updated in place by ``Lstm.forward(..., state=)``:
+    ``h`` bf16 (layers, B, H) -- the h the recurrence feeds its MMA -- and ``c`` f32 (layers, B, H).  Zero when
+    created, as at the start of a sequence."""
+
+    def __init__(self, lstm: Lstm, B: int, device="cuda"):
+        self.h = torch.zeros(lstm.layers, B, lstm.hidden, dtype=torch.bfloat16, device=device)
+        self.c = torch.zeros(lstm.layers, B, lstm.hidden, dtype=torch.float32, device=device)
+
+    def reset(self, rows=None):
+        """Start new sequences in ``rows`` (an index, a list of indices or a bool mask; None = every row)."""
+        if rows is None:
+            self.h.zero_()
+            self.c.zero_()
+        else:
+            self.h[:, rows] = 0
+            self.c[:, rows] = 0
+
+    def check(self, lstm: Lstm, B: int, device):
+        shape = (lstm.layers, B, lstm.hidden)
+        if tuple(self.h.shape) != shape or tuple(self.c.shape) != shape:
+            raise ValueError(f"LstmState: expected h, c of shape {shape}, got {tuple(self.h.shape)}, "
+                             f"{tuple(self.c.shape)}")
+        if self.h.device != torch.device(device) or self.c.device != torch.device(device):
+            raise ValueError("LstmState: state and input on different devices")
+        assert self.h.dtype == torch.bfloat16 and self.c.dtype == torch.float32
+        assert self.h.is_contiguous() and self.c.is_contiguous()
 
 
 def _ptr_array(tensors):

@@ -80,6 +80,8 @@ PROTOTYPES = {
     "avvad_mcb_forward": (C.c_int, [VP, VP, VP, C.c_int64, VP, C.c_size_t, VP, C.c_int64, VP, VP]),
     "avvad_mcb_grouped_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int64]),
     "avvad_mcb_forward_grouped": (C.c_int, [VP, VP, VP, C.c_int64, C.c_int64, VP, VP, C.c_size_t, VP, C.c_int64, VP, VP]),
+    "avvad_mcb_forward_grouped_norms": (C.c_int, [VP, VP, VP, C.c_int64, C.c_int64, VP, VP, VP, VP, C.c_size_t, VP,
+                                                  C.c_int64, VP, VP]),
     "avvad_count_sketch_forward": (C.c_int, [VP, C.c_int64, C.c_int, C.c_int, VP, VP, VP, VP, VP]),
     "avvad_count_sketch_backward": (C.c_int, [VP, C.c_int64, C.c_int, C.c_int, VP, VP, VP, VP]),
     "avvad_mcb_raw_forward": (C.c_int, [VP] * 8 + [C.c_int64, VP, VP]),
@@ -111,6 +113,9 @@ PROTOTYPES = {
     "avvad_lstm_input_ld": (C.c_int64, [VP]),
     "avvad_lstm_workspace_bytes": (C.c_size_t, [VP, C.c_int64, C.c_int64]),
     "avvad_lstm_forward": (C.c_int, [VP, VP, VP, C.c_int64, C.c_int64, VP, C.c_size_t, VP, VP, VP, VP, VP]),
+    "avvad_lstm_state_workspace_bytes": (C.c_size_t, [VP, C.c_int64, C.c_int64]),
+    "avvad_lstm_forward_state": (C.c_int, [VP, VP, VP, C.c_int64, C.c_int64, VP, VP, VP, VP, VP, C.c_size_t, VP, VP,
+                                           VP, VP, VP]),
 }
 
 

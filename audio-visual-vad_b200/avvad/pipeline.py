@@ -69,7 +69,7 @@ class AVVADPipeline:
 
     def infer_device(self, wave: torch.Tensor, n_samples, video_u8: torch.Tensor, n_src, lengths=None,
                      t_max: Optional[int] = None, _video_ready=None, _wave_ready=None,
-                     per_utterance: Optional[bool] = None):
+                     per_utterance: Optional[bool] = None, mcb_norms_out: Optional[torch.Tensor] = None):
         """wave (B,N) f32 and video (B,F,67,67) u8/f32 already on the device.
         Returns (logits, posteriors, decisions), each (B,t_max,y_dim) on the device.
 
@@ -77,6 +77,8 @@ class AVVADPipeline:
         over its valid frames, so the batched call returns what B separate forward calls of the reference return --
         the semantics of scripts/evaluate_AV_net.py:186-236, which calls the model once per utterance.  Off: one norm
         over the whole padded (B,T,1024) tensor of the call (AV_Net.py:117 for a batched call, the training scripts).
+        ``mcb_norms_out`` (f32 (B,) on the device, with ``per_utterance`` and ``use_mcb``): receives the norms used --
+        the constants :class:`avvad.stream.AVVADStream` needs to stream these utterances.
 
         The video branch runs in pieces of ``self.piece`` utterances (frames of an utterance are independent for
         the trunk); ``_video_ready[k]`` / ``_wave_ready`` are optional CUDA events the current stream waits on
@@ -143,8 +145,10 @@ class AVVADPipeline:
                 front_end()  # the waveforms arrive behind the first video piece
         if self.use_mcb:
             if self.per_utterance if per_utterance is None else per_utterance:
-                self.mcb.forward_grouped(audio.view(M, 513), feat, lens, t_max, out_bf16=xv)
+                self.mcb.forward_grouped(audio.view(M, 513), feat, lens, t_max, out_bf16=xv, norms_out=mcb_norms_out)
             else:
+                if mcb_norms_out is not None:
+                    raise ValueError("mcb_norms_out needs per_utterance=True")
                 self.mcb.forward(audio.view(M, 513), feat, out_bf16=xv)
         logits, post, dec, _ = self.lstm.forward(x, lens, want_post=True, want_dec=True)
         return logits, post, dec

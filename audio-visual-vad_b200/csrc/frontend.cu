@@ -250,6 +250,7 @@ static int launch_frontend(int mode, const float* wave, int64_t wave_stride, con
   AVVAD_CHECK_ARG(wave && n_samples && n_frames && out, "null pointer");
   AVVAD_CHECK_ARG(B > 0 && t_max > 0 && wave_stride > 0, "B, t_max, wave_stride must be positive");
   AVVAD_CHECK_ARG((mean == nullptr) == (stdv == nullptr), "mean and std must both be given or both NULL");
+  AVVAD_CHECK_ARG(normalise >= 0 && normalise <= 2, "normalise must be 0, 1 or 2");
   AVVAD_CHECK_ARG(!normalise || peak_scratch, "peak_scratch required when normalise != 0");
   const float2* tw = fft_twiddles_device();
   if (!tw) {
@@ -260,7 +261,7 @@ static int launch_frontend(int mode, const float* wave, int64_t wave_stride, con
   // 256 new samples in + 513 (x2 for the raw STFT) floats out per frame (SURVEY 8d)
   void* ptok = nullptr;
   tc::prof_begin(st, &ptok);
-  if (normalise) {
+  if (normalise == 1) {  // 2: peak_scratch already holds the caller's peaks
     AVVAD_CUDA(cudaMemsetAsync(peak_scratch, 0, sizeof(float) * B, st));
     int chunks = (int)std::min<int64_t>(64, ceil_div(wave_stride, 256 * 16));
     absmax_kernel<<<dim3(chunks, B), 256, 0, st>>>(wave, wave_stride, n_samples, peak_scratch);

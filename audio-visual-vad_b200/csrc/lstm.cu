@@ -96,6 +96,41 @@ __global__ void gather_last_kernel(const __nv_bfloat16* __restrict__ hseq, const
   for (int i = threadIdx.x; i < H / 8; i += blockDim.x) dst[i] = src[i];
 }
 
+// Streaming state (avvad_lstm_forward_state): the persistent recurrences run the call's steps at positions 1..T of a
+// [B][T+1][H] sequence whose position 0 holds h_in, so their masks see len_b + 1
+__global__ void shift_lengths_kernel(const int32_t* __restrict__ lengths, int B, int32_t* __restrict__ out) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b < B) out[b] = lengths[b] + 1;
+}
+
+// Final state of one layer: h_out[b] = hseq[b][len_b - 1 + shift], c_out[b] = cseq[b][len_b - 1 + shift] (sequences of
+// Ts steps), or h_in[b] / c_in[b] (zero when null) when len_b = 0.  Every element is read and written by the same
+// thread, so h_out / c_out may alias h_in / c_in.
+__global__ void gather_state_kernel(const __nv_bfloat16* __restrict__ hseq, const float* __restrict__ cseq,
+                                    const int32_t* __restrict__ lengths, int Ts, int shift, int H,
+                                    const __nv_bfloat16* h_in, const float* c_in, __nv_bfloat16* h_out, float* c_out) {
+  const int b = blockIdx.x;
+  const int len = lengths[b];
+  const int64_t src = ((int64_t)b * Ts + len - 1 + shift) * H;
+  const int64_t dst = (int64_t)b * H;
+  if (h_out) {
+    for (int i = threadIdx.x; i < H / 8; i += blockDim.x) {
+      uint4 v = make_uint4(0u, 0u, 0u, 0u);
+      if (len > 0) v = reinterpret_cast<const uint4*>(hseq + src)[i];
+      else if (h_in) v = reinterpret_cast<const uint4*>(h_in + dst)[i];
+      reinterpret_cast<uint4*>(h_out + dst)[i] = v;
+    }
+  }
+  if (c_out) {
+    for (int i = threadIdx.x; i < H / 4; i += blockDim.x) {
+      float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (len > 0) v = reinterpret_cast<const float4*>(cseq + src)[i];
+      else if (c_in) v = reinterpret_cast<const float4*>(c_in + dst)[i];
+      reinterpret_cast<float4*>(c_out + dst)[i] = v;
+    }
+  }
+}
+
 }  // namespace avvad
 
 namespace avvad {
@@ -240,9 +275,13 @@ struct LstmWs {
   float* c;
   __nv_bfloat16* hlast;
   unsigned int* counters;
+  // streaming state only: c_t of every step of the layers in flight (f32 [B][T+1][H]) and the shifted lengths
+  float* cseq[2];
+  int32_t* len1;
   size_t total;
 };
-LstmWs carve(const avvad_lstm* h, int64_t B, int64_t T, void* base) {
+// `state`: the layout of avvad_lstm_forward_state, whose sequences have one more step (position 0 holds h_in)
+LstmWs carve(const avvad_lstm* h, int64_t B, int64_t T, void* base, bool state = false) {
   LstmWs w{};
   size_t off = 0;
   auto take = [&](size_t bytes) {
@@ -251,6 +290,11 @@ LstmWs carve(const avvad_lstm* h, int64_t B, int64_t T, void* base) {
     return p;
   };
   const int64_t H = h->H;
+  if (state) {
+    ++T;
+    for (int l = 0; l < (h->layers >= 2 ? 2 : 1); ++l) w.cseq[l] = (float*)take((size_t)B * T * H * sizeof(float));
+    w.len1 = (int32_t*)take((size_t)B * sizeof(int32_t));
+  }
   w.xproj = (float*)take((size_t)((B + 127) / 128 * 128) * T * 4 * H * sizeof(float));  // xT layout pads B to 128
   w.xproj1 = (h->layers >= 2) ? (float*)take((size_t)((B + 127) / 128 * 128) * T * 4 * H * sizeof(float)) : nullptr;
   w.c1 = (float*)take((size_t)B * H * sizeof(float));
@@ -269,6 +313,11 @@ LstmWs carve(const avvad_lstm* h, int64_t B, int64_t T, void* base) {
 extern "C" size_t avvad_lstm_workspace_bytes(const avvad_lstm* h, int64_t B, int64_t T) {
   if (!h || B <= 0 || T <= 0) return 0;
   return carve(h, B, T, nullptr).total;
+}
+
+extern "C" size_t avvad_lstm_state_workspace_bytes(const avvad_lstm* h, int64_t B, int64_t T) {
+  if (!h || B <= 0 || T <= 0) return 0;
+  return carve(h, B, T, nullptr, true).total;
 }
 
 // ---- persistent recurrence (one cooperative launch per layer and batch group) ---------------------------------
@@ -550,11 +599,23 @@ static int run_head(avvad_lstm* h, const __nv_bfloat16* hs, int64_t rows, float*
   return AVVAD_OK;
 }
 
+namespace {
+// Recurrent state of avvad_lstm_forward_state: h bf16 [L][B][H], c f32 [L][B][H]; null inputs mean zero
+struct LstmStateIO {
+  const __nv_bfloat16* h_in;
+  const float* c_in;
+  __nv_bfloat16* h_out;
+  float* c_out;
+};
+}  // namespace
+
 static int lstm_forward_impl(avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T,
                              void* workspace, size_t workspace_bytes, float* logits, float* post, int32_t* dec,
-                             float* last_logits, void* tape, void* stream) {
+                             float* last_logits, void* tape, void* stream, const LstmStateIO* sio = nullptr) {
   AVVAD_CHECK_ARG(h && x_bf16 && lengths && workspace && B > 0 && T > 0, "bad argument");
-  AVVAD_CHECK_ARG(logits || post || dec || last_logits, "no output requested");
+  const bool want_head = logits || post || dec || last_logits;
+  AVVAD_CHECK_ARG(want_head || (sio && (sio->h_out || sio->c_out)), "no output requested");
+  AVVAD_CHECK_ARG(!(sio && tape), "lstm: the training forward takes no initial state");
   for (int l = 0; l < h->layers; ++l)
     if (!h->set[l]) {
       set_error("lstm: layer " + std::to_string(l) + " not loaded");
@@ -564,20 +625,60 @@ static int lstm_forward_impl(avvad_lstm* h, const void* x_bf16, const int32_t* l
     set_error("lstm: head not loaded");
     return AVVAD_ERR_STATE;
   }
-  if (workspace_bytes < avvad_lstm_workspace_bytes(h, B, T)) {
+  if (workspace_bytes < (sio ? avvad_lstm_state_workspace_bytes(h, B, T) : avvad_lstm_workspace_bytes(h, B, T))) {
     set_error("lstm: workspace too small");
     return AVVAD_ERR_WORKSPACE;
   }
   cudaStream_t st = (cudaStream_t)stream;
   const int H = h->H;
   const int H4 = 4 * H;
-  LstmWs ws = carve(h, B, T, workspace);
+  LstmWs ws = carve(h, B, T, workspace, sio != nullptr);
   const int64_t rows = B * T;
 
   const __nv_bfloat16* layer_in = (const __nv_bfloat16*)x_bf16;
   int64_t ld_in = h->ld0;
+  int64_t in_stride = T;  // steps per batch row of layer_in
   __nv_bfloat16* layer_out = nullptr;
   const bool persistent = persistent_ok(h, T);
+
+  // ---- streaming state.  The persistent recurrences run this call's steps at positions s = 1 .. T of [B][T+1][H]
+  // sequences whose position 0 holds h_in, with c_in in c_state: exactly the hand-over between two chunks of one layer,
+  // so the kernels are the ones the stateless call runs.  They record c_t of every step (the training tape's c store),
+  // from which the final state is gathered at len_b - 1.  The per-step fallback seeds its h operand instead (s = 0).
+  const int s = (sio && persistent) ? 1 : 0;
+  const int64_t Ts = T + s;
+  const int64_t Bp = (B + 127) / 128 * 128;
+  const int32_t* lens_rec = lengths;  // lengths the recurrence masks with (positions, not steps)
+  if (s) {
+    shift_lengths_kernel<<<(unsigned)ceil_div(B, 256), 256, 0, st>>>(lengths, (int)B, ws.len1);
+    AVVAD_LAUNCHED();
+    lens_rec = ws.len1;
+  }
+  // layer l's initial state: h_in[l] -> position 0 of `hs` (rows `pitch` steps apart), c_in[l] -> c_state
+  auto seed = [&](int l, __nv_bfloat16* hs, int64_t pitch, float* c_state) -> int {
+    const size_t hrow = (size_t)H * 2, crow = (size_t)H * sizeof(float);
+    const int64_t off = (int64_t)l * B * H;
+    if (sio->h_in)
+      AVVAD_CUDA(cudaMemcpy2DAsync(hs, pitch * hrow, sio->h_in + off, hrow, hrow, B, cudaMemcpyDeviceToDevice, st));
+    else
+      AVVAD_CUDA(cudaMemset2DAsync(hs, pitch * hrow, 0, hrow, B, st));
+    if (sio->c_in)
+      AVVAD_CUDA(cudaMemcpyAsync(c_state, sio->c_in + off, B * crow, cudaMemcpyDeviceToDevice, st));
+    else
+      AVVAD_CUDA(cudaMemsetAsync(c_state, 0, B * crow, st));
+    return AVVAD_OK;
+  };
+  // layer l's final state from its output sequence and its record of c
+  auto emit = [&](int l, const __nv_bfloat16* hs, const float* cseq) -> int {
+    const int64_t off = (int64_t)l * B * H;
+    gather_state_kernel<<<(unsigned)B, 128, 0, st>>>(hs, cseq, lengths, (int)Ts, s, H,
+                                                     sio->h_in ? sio->h_in + off : nullptr,
+                                                     sio->c_in ? sio->c_in + off : nullptr,
+                                                     sio->h_out ? sio->h_out + off : nullptr,
+                                                     sio->c_out ? sio->c_out + off : nullptr);
+    AVVAD_LAUNCHED();
+    return AVVAD_OK;
+  };
 
   // ---- two layers, chunked: layer 1 follows layer 0 one chunk of time steps behind on a side stream.  Both recurrences
   // are latency chains on 64 SMs each, so they overlap almost perfectly; layer 1's input projection of a chunk (a GEMM
@@ -607,22 +708,30 @@ static int lstm_forward_impl(avvad_lstm* h, const void* x_bf16, const int32_t* l
     }
     __nv_bfloat16* out0 = ws.hseq[0];
     __nv_bfloat16* out1 = ws.hseq[1];
+    float* crec0 = ws.cseq[0];
+    float* crec1 = ws.cseq[1];
     TapeView tv0{}, tv1{};
     if (tape) {
       tv0 = tape_layer(tape, 0, H, B, T);
       tv1 = tape_layer(tape, 1, H, B, T);
       out0 = tv0.hseq;
       out1 = tv1.hseq;
+      crec0 = tv0.c;
+      crec1 = tv1.c;
     }
-    const int64_t Bp = (B + 127) / 128 * 128;
-    int rc = tc::launch_tma_gemm_xt(layer_in, ld_in, h->w_ih[0], ld_in, B, T, T, H4, (int)ld_in, h->bias[0], ws.xproj, st);
+    int rc;
+    if (sio) {  // on `st` before the first chunk's event: the side stream sees layer 1's seed too
+      if ((rc = seed(0, out0, Ts, ws.c)) || (rc = seed(1, out1, Ts, ws.c1))) return rc;
+    }
+    rc = tc::launch_tma_gemm_xt(layer_in, ld_in, h->w_ih[0], ld_in, B, T, T, H4, (int)ld_in, h->bias[0],
+                                ws.xproj + s * H4 * Bp, st);
     if (rc) return rc;
     const int free_sms = lstm_num_sms() - 2 * (4 * H / 128);  // SMs a layer-0 pair launch leaves to the projection GEMM
     for (int c = 0; c < n_chunks; ++c) {
-      const int t0 = (int)(T * c / n_chunks), t1 = (int)(T * (c + 1) / n_chunks);
+      const int t0 = s + (int)(T * c / n_chunks), t1 = s + (int)(T * (c + 1) / n_chunks);
       bool done = false;
-      rc = run_recurrence_persistent(h, 0, ws.xproj, out0, lengths, B, T, ws.counters, st, &done, tv0.gates, tv0.c, t0, t1,
-                                     ws.c);
+      rc = run_recurrence_persistent(h, 0, ws.xproj, out0, lens_rec, B, Ts, ws.counters, st, &done, tv0.gates, crec0,
+                                     t0, t1, ws.c);
       if (rc) return rc;
       if (!done) {
         set_error("lstm: persistent recurrence unavailable");
@@ -630,35 +739,42 @@ static int lstm_forward_impl(avvad_lstm* h, const void* x_bf16, const int32_t* l
       }
       AVVAD_CUDA(cudaEventRecord(h->ev_chunk[c], st));
       AVVAD_CUDA(cudaStreamWaitEvent(h->side, h->ev_chunk[c], 0));
-      rc = tc::launch_tma_gemm_xt(out0 + (int64_t)t0 * H, H, h->w_ih[1], H, B, t1 - t0, T, H4, H, h->bias[1],
+      rc = tc::launch_tma_gemm_xt(out0 + (int64_t)t0 * H, H, h->w_ih[1], H, B, t1 - t0, Ts, H4, H, h->bias[1],
                                   ws.xproj1 + (int64_t)t0 * H4 * Bp, h->side, free_sms > 16 ? free_sms : 0);
       if (rc) return rc;
-      rc = run_recurrence_persistent(h, 1, ws.xproj1, out1, lengths, B, T, ws.counters + kCounterBytes / 4, h->side, &done,
-                                     tv1.gates, tv1.c, t0, t1, ws.c1);
+      rc = run_recurrence_persistent(h, 1, ws.xproj1, out1, lens_rec, B, Ts, ws.counters + kCounterBytes / 4, h->side,
+                                     &done, tv1.gates, crec1, t0, t1, ws.c1);
       if (rc) return rc;
     }
     AVVAD_CUDA(cudaEventRecord(h->ev_done, h->side));
     AVVAD_CUDA(cudaStreamWaitEvent(st, h->ev_done, 0));
+    if (sio) {
+      if ((rc = emit(0, out0, crec0)) || (rc = emit(1, out1, crec1))) return rc;
+    }
     layer_out = out1;
   } else {
   for (int l = 0; l < h->layers; ++l) {
     layer_out = ws.hseq[l & 1];
+    float* crec = ws.cseq[l & 1];
     TapeView tv{};
     if (tape) {
       tv = tape_layer(tape, l, H, B, T);
       layer_out = tv.hseq;
+      crec = tv.c;
     }
+    int rc;
+    if (s && (rc = seed(l, layer_out, Ts, ws.c))) return rc;
     // (1) input projection for every (b,t): xproj = X * W_ih'^T + (b_ih + b_hh)'.  The persistent recurrences read it
     // time-major and unit-major (xT[t][u][b][4]: lane = batch row -> coalesced), the per-step fallback row-major.
-    int rc = persistent ? tc::launch_tma_gemm_xt(layer_in, ld_in, h->w_ih[l], ld_in, B, T, T, H4, (int)ld_in, h->bias[l],
-                                                 ws.xproj, st)
-                        : avvad_gemm_bf16(layer_in, ld_in, h->w_ih[l], ld_in, h->bias[l], ws.xproj, H4, 0, 0, rows, H4,
-                                          ld_in, st);
+    rc = persistent ? tc::launch_tma_gemm_xt(layer_in, ld_in, h->w_ih[l], ld_in, B, T, in_stride, H4, (int)ld_in,
+                                             h->bias[l], ws.xproj + s * H4 * Bp, st)
+                    : avvad_gemm_bf16(layer_in, ld_in, h->w_ih[l], ld_in, h->bias[l], ws.xproj, H4, 0, 0, rows, H4,
+                                      ld_in, st);
     if (rc) return rc;
     // (2) recurrence: one persistent cooperative kernel per layer, or (fallback) one GEMM launch per time step
     bool done = false;
-    rc = run_recurrence_persistent(h, l, ws.xproj, layer_out, lengths, B, T, ws.counters, st, &done, tv.gates, tv.c, 0,
-                                   (int)T, ws.c);
+    rc = run_recurrence_persistent(h, l, ws.xproj, layer_out, lens_rec, B, Ts, ws.counters, st, &done, tv.gates, crec,
+                                   s, (int)Ts, ws.c);
     if (rc) return rc;
     if (persistent && !done) {
       set_error("lstm: persistent recurrence unavailable after the xT input projection");
@@ -669,12 +785,18 @@ static int lstm_forward_impl(avvad_lstm* h, const void* x_bf16, const int32_t* l
       return AVVAD_ERR_STATE;
     }
     if (done) {
-      layer_in = layer_out;
+      if (sio && (rc = emit(l, layer_out, crec))) return rc;
+      layer_in = layer_out + (int64_t)s * H;
       ld_in = H;
+      in_stride = Ts;
       continue;
     }
-    AVVAD_CUDA(cudaMemsetAsync(ws.hbuf[0], 0, (size_t)B * H * 2, st));
-    AVVAD_CUDA(cudaMemsetAsync(ws.c, 0, (size_t)B * H * sizeof(float), st));
+    if (sio) {
+      if ((rc = seed(l, ws.hbuf[0], 1, ws.c))) return rc;
+    } else {
+      AVVAD_CUDA(cudaMemsetAsync(ws.hbuf[0], 0, (size_t)B * H * 2, st));
+      AVVAD_CUDA(cudaMemsetAsync(ws.c, 0, (size_t)B * H * sizeof(float), st));
+    }
     for (int t = 0; t < (int)T; ++t) {
       tc::EpiParams ep{};
       ep.xproj = ws.xproj;
@@ -687,10 +809,21 @@ static int lstm_forward_impl(avvad_lstm* h, const void* x_bf16, const int32_t* l
       ep.H4 = H4;
       rc = tc::gemm_dispatch(ws.hbuf[t & 1], H, h->w_hh[l], H, B, H4, H, ep, tc::EPI_LSTM, 64, st);
       if (rc) return rc;
+      if (sio)  // the epilogue keeps updating c past the length: record c_t for the final-state gather
+        AVVAD_CUDA(cudaMemcpy2DAsync(crec + (int64_t)t * H, (size_t)T * H * sizeof(float), ws.c, (size_t)H * sizeof(float),
+                                     (size_t)H * sizeof(float), B, cudaMemcpyDeviceToDevice, st));
     }
+    if (sio && (rc = emit(l, layer_out, crec))) return rc;
     layer_in = layer_out;
     ld_in = H;
   }
+  }
+  if (!want_head) return AVVAD_OK;
+  if (s) {  // the head reads [B][T][H] rows: drop position 0 into the sequence buffer the last layer did not use
+    __nv_bfloat16* compact = layer_out == ws.hseq[0] ? ws.hseq[1] : ws.hseq[0];
+    AVVAD_CUDA(cudaMemcpy2DAsync(compact, (size_t)T * H * 2, layer_out + H, (size_t)Ts * H * 2, (size_t)T * H * 2, B,
+                                 cudaMemcpyDeviceToDevice, st));
+    layer_out = compact;
   }
   if (logits || post || dec) {
     float* lg = logits;
@@ -712,6 +845,15 @@ extern "C" int avvad_lstm_forward(avvad_lstm* h, const void* x_bf16, const int32
                                   float* last_logits, void* stream) {
   return lstm_forward_impl(h, x_bf16, lengths, B, T, workspace, workspace_bytes, logits, post, dec, last_logits, nullptr,
                            stream);
+}
+
+extern "C" int avvad_lstm_forward_state(avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T,
+                                        const void* h_in, const float* c_in, void* h_out, float* c_out,
+                                        void* workspace, size_t workspace_bytes, float* logits, float* post,
+                                        int32_t* dec, float* last_logits, void* stream) {
+  const LstmStateIO sio{(const __nv_bfloat16*)h_in, c_in, (__nv_bfloat16*)h_out, c_out};
+  return lstm_forward_impl(h, x_bf16, lengths, B, T, workspace, workspace_bytes, logits, post, dec, last_logits, nullptr,
+                           stream, &sio);
 }
 
 extern "C" size_t avvad_lstm_tape_bytes(int layers, int hidden, int64_t B, int64_t T);

@@ -751,10 +751,12 @@ extern "C" size_t avvad_mcb_grouped_workspace_bytes(int64_t n_groups, int64_t t_
   return avvad_mcb_workspace_bytes(n_groups * t_max) + align_up((size_t)n_groups * sizeof(float), 256);
 }
 
-extern "C" int avvad_mcb_forward_grouped(avvad_mcb* h, const float* audio, const float* video, int64_t n_groups,
-                                         int64_t t_max, const int32_t* lengths, void* workspace,
-                                         size_t workspace_bytes, void* out_bf16, int64_t ld_out, float* out_f32,
-                                         void* stream) {
+// norms_in (optional, f32 [n_groups]): use these norms instead of computing them -- a streaming caller normalises
+// every block of an utterance by one constant.  norms_out (optional): the norms the call used.
+extern "C" int avvad_mcb_forward_grouped_norms(avvad_mcb* h, const float* audio, const float* video, int64_t n_groups,
+                                               int64_t t_max, const int32_t* lengths, const float* norms_in,
+                                               float* norms_out, void* workspace, size_t workspace_bytes,
+                                               void* out_bf16, int64_t ld_out, float* out_f32, void* stream) {
   AVVAD_CHECK_ARG(h && audio && video && workspace && lengths && n_groups > 0 && t_max > 0, "bad argument");
   AVVAD_CHECK_ARG(out_bf16 || out_f32, "at least one output required");
   AVVAD_CHECK_ARG(!out_bf16 || ld_out >= kMcbOut, "ld_out must be >= 1024");
@@ -781,15 +783,29 @@ extern "C" int avvad_mcb_forward_grouped(avvad_mcb* h, const float* audio, const
   void* ptok = nullptr;
   tc::prof_begin(st, &ptok);
   if (int rc = launch_mcb_rows(audio, video, tb, rounds_of(h), tw, h->eps, y, rowsq, rows, lengths, (int)t_max, st)) return rc;
-  mcb_norm_grouped_kernel<<<(unsigned)n_groups, 256, 0, st>>>(rowsq, lengths, (int)t_max, norms);
-  AVVAD_LAUNCHED();
+  const float* nrm = norms_in;
+  if (!norms_in) {
+    mcb_norm_grouped_kernel<<<(unsigned)n_groups, 256, 0, st>>>(rowsq, lengths, (int)t_max, norms);
+    AVVAD_LAUNCHED();
+    nrm = norms;
+  }
+  if (norms_out && norms_out != nrm)
+    AVVAD_CUDA(cudaMemcpyAsync(norms_out, nrm, (size_t)n_groups * sizeof(float), cudaMemcpyDeviceToDevice, st));
   const int64_t total = rows * kMcbOut;
   mcb_apply_kernel<<<(unsigned)ceil_div(total / 8, 256), 256, 0, st>>>(
-      y, norms, lengths, (int)t_max, h->bn_mean, h->bn_invstd, h->bn_gamma, h->bn_beta, rows,
+      y, nrm, lengths, (int)t_max, h->bn_mean, h->bn_invstd, h->bn_gamma, h->bn_beta, rows,
       (__nv_bfloat16*)out_bf16, ld_out, out_f32);
   AVVAD_LAUNCHED();
   tc::prof_end(st, ptok, 5, (double)rows * (4100.0 + (out_f32 ? 4096.0 : 2048.0)));
   return AVVAD_OK;
+}
+
+extern "C" int avvad_mcb_forward_grouped(avvad_mcb* h, const float* audio, const float* video, int64_t n_groups,
+                                         int64_t t_max, const int32_t* lengths, void* workspace,
+                                         size_t workspace_bytes, void* out_bf16, int64_t ld_out, float* out_f32,
+                                         void* stream) {
+  return avvad_mcb_forward_grouped_norms(h, audio, video, n_groups, t_max, lengths, nullptr, nullptr, workspace,
+                                         workspace_bytes, out_bf16, ld_out, out_f32, stream);
 }
 
 

@@ -69,7 +69,9 @@ int64_t avvad_stft_num_frames(int64_t n_samples, double fs, double wlen_sec, dou
  * mean,std  : f32 [513] device or NULL (no standardisation)
  * out       : f32 [B][t_max][513] device.  Rows t >= n_frames[b] get the collate value
  *             (0-mean)/(std+eps) (or 0 when mean==NULL).
- * peak_scratch : f32 [B] device scratch (per-utterance max|x|), only used when normalise!=0
+ * normalise : 0 = none, 1 = divide by max|x| over the utterance's samples (AV_Net.py:117's peak normalisation),
+ *             2 = divide by the peaks the caller put in peak_scratch (a stream cannot see the whole utterance)
+ * peak_scratch : f32 [B] device scratch (per-utterance max|x|) with normalise == 1, the given peaks with 2
  * nfft must be 1024 and hop 256 (the reference's 64 ms / 25 % at 16 kHz). */
 int avvad_frontend_logpower(const float* wave, int64_t wave_stride, const int32_t* n_samples,
                             const int32_t* n_frames, int32_t B, int32_t t_max, int normalise,
@@ -283,6 +285,12 @@ size_t avvad_mcb_grouped_workspace_bytes(int64_t n_groups, int64_t t_max);
 int avvad_mcb_forward_grouped(avvad_mcb* h, const float* audio, const float* video, int64_t n_groups, int64_t t_max,
                               const int32_t* lengths, void* workspace, size_t workspace_bytes, void* out_bf16,
                               int64_t ld_out, float* out_f32, void* stream);
+/* As avvad_mcb_forward_grouped; norms_in (f32 [n_groups] device or NULL): divide by these norms instead of computing
+ * them (streaming: every block of an utterance uses one norm); norms_out (or NULL): receives the norms used. */
+int avvad_mcb_forward_grouped_norms(avvad_mcb* h, const float* audio, const float* video, int64_t n_groups,
+                                    int64_t t_max, const int32_t* lengths, const float* norms_in, float* norms_out,
+                                    void* workspace, size_t workspace_bytes, void* out_bf16, int64_t ld_out,
+                                    float* out_f32, void* stream);
 
 /* Training mode (module in train()): BatchNorm1d uses this call's batch statistics and the CURRENT gamma/beta, updates
  * running_mean/var in place (NULL = leave); the workspace then carries what avvad_mcb_backward_bn needs to turn the
@@ -351,6 +359,18 @@ size_t avvad_lstm_workspace_bytes(const avvad_lstm* h, int64_t B, int64_t T);
 int avvad_lstm_forward(avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T,
                        void* workspace, size_t workspace_bytes, float* logits, float* post,
                        int32_t* dec, float* last_logits, void* stream);
+/* Streaming: as avvad_lstm_forward, continuing from a recurrent state and returning the state after the call.
+ * h_in / h_out : bf16 [layers][B][H] (the h the recurrence feeds its MMA), c_in / c_out : f32 [layers][B][H].
+ * Row b carries lengths[b] new steps (0 <= lengths[b] <= T; 0 passes the state through).  h_in / c_in NULL = zero
+ * state; h_out / c_out may be NULL or alias h_in / c_in (the call reads its input state before it writes the output).
+ * h_out[l][b] / c_out[l][b] are layer l's h and c at step lengths[b] - 1.  Running a sequence in blocks with the state
+ * carried gives the logits of one call on the whole sequence, bit for bit, on every recurrence path.
+ * workspace: avvad_lstm_state_workspace_bytes(h, B, T).  The logit outputs may all be NULL when h_out or c_out is set. */
+size_t avvad_lstm_state_workspace_bytes(const avvad_lstm* h, int64_t B, int64_t T);
+int avvad_lstm_forward_state(avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T,
+                             const void* h_in, const float* c_in, void* h_out, float* c_out,
+                             void* workspace, size_t workspace_bytes, float* logits, float* post,
+                             int32_t* dec, float* last_logits, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Training step of the LSTM + head (SURVEY §8a O1): forward that keeps activations, BPTT, fused Adam
