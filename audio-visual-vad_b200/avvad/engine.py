@@ -649,16 +649,44 @@ def _ptr_array(tensors):
     return arr
 
 
-def lstm_train_forward(lstm: "Lstm", x_bf16: torch.Tensor, lengths):
-    """Forward that keeps the activations BPTT needs.  Returns (logits (B,T,1), tape)."""
+def _state_pair(lstm: "Lstm", state, B: int, dev):
+    """(h bf16, c f32), both (layers, B, H) contiguous, from an LstmState or an (h, c) pair (h of any float dtype is
+    rounded to bf16, the h the recurrence feeds its MMA; None = a zero state)."""
+    if isinstance(state, LstmState):
+        state.check(lstm, B, dev)
+        return state.h, state.c
+    shape = (lstm.layers, B, lstm.hidden)
+
+    def take(t, dtype):
+        if t is None:
+            return None
+        if tuple(t.shape) != shape:
+            raise ValueError(f"state: expected h, c of shape {shape}, got {tuple(t.shape)}")
+        if t.device != torch.device(dev):
+            raise ValueError("state and input on different devices")
+        return t.detach().to(dtype).contiguous()
+    return take(state[0], torch.bfloat16), take(state[1], torch.float32)
+
+
+def lstm_train_forward(lstm: "Lstm", x_bf16: torch.Tensor, lengths, state=None):
+    """Forward that keeps the activations BPTT needs.  Returns (logits (B,T,y_dim), tape).
+
+    With `state` (an LstmState or an (h, c) pair of shape (layers, B, H)) the recurrence continues from it, the tape
+    holds T + 1 positions per row (position 0 = the state; its pack carries a fourth entry that marks it stateful) and
+    the call returns (logits, tape, (h_out, c_out)): h_out bf16 and c_out f32 (layers, B, H) at each row's last step
+    (the input state for rows of length 0)."""
     L.require_cuda(x_bf16)
     B, T, ld = x_bf16.shape
     assert ld == lstm.ld and x_bf16.is_contiguous()
     dev = x_bf16.device
     lens = _i32(lengths, dev)
-    nbytes = L.lib().avvad_lstm_workspace_bytes(lstm.h, B, T)
+    if state is not None:
+        h_in, c_in = _state_pair(lstm, state, B, dev)
+        nbytes = L.lib().avvad_lstm_train_state_workspace_bytes(lstm.h, B, T)
+    else:
+        nbytes = L.lib().avvad_lstm_workspace_bytes(lstm.h, B, T)
     ws = lstm.ws.get(nbytes, dev)
-    tb = L.lib().avvad_lstm_tape_bytes(lstm.layers, lstm.hidden, B, T)
+    tb = L.lib().avvad_lstm_tape_bytes(lstm.layers, lstm.hidden, B, T + (state is not None))
     # The tape lives with the engine and is reused step after step: its address is baked into the cached CUDA graph of
     # the backward recurrence (csrc/lstm_train.cu), so a stable buffer means graph replays instead of re-captures.  A
     # second forward before the first one's backward (gradient accumulation over micro-batches) gets its own tape.
@@ -670,9 +698,17 @@ def lstm_train_forward(lstm: "Lstm", x_bf16: torch.Tensor, lengths):
     if tape is getattr(lstm, "_tape", None):
         lstm._tape_busy = True
     logits = torch.empty(B, T, lstm.y_dim, dtype=torch.float32, device=dev)
-    L.check(L.lib().avvad_lstm_forward_train(lstm.h, L.ptr(x_bf16), L.ptr(lens), B, T, L.ptr(ws), ws.numel(),
-                                             L.ptr(tape), tape.numel(), L.ptr(logits), L.stream_ptr()))
-    return logits, (tape, lens, x_bf16)
+    if state is None:
+        L.check(L.lib().avvad_lstm_forward_train(lstm.h, L.ptr(x_bf16), L.ptr(lens), B, T, L.ptr(ws), ws.numel(),
+                                                 L.ptr(tape), tape.numel(), L.ptr(logits), L.stream_ptr()))
+        return logits, (tape, lens, x_bf16)
+    shape = (lstm.layers, B, lstm.hidden)
+    h_out = torch.empty(shape, dtype=torch.bfloat16, device=dev)
+    c_out = torch.empty(shape, dtype=torch.float32, device=dev)
+    L.check(L.lib().avvad_lstm_forward_train_state(lstm.h, L.ptr(x_bf16), L.ptr(lens), B, T, L.ptr(h_in), L.ptr(c_in),
+                                                   L.ptr(h_out), L.ptr(c_out), L.ptr(ws), ws.numel(), L.ptr(tape),
+                                                   tape.numel(), L.ptr(logits), L.stream_ptr()))
+    return logits, (tape, lens, x_bf16, "state"), (h_out, c_out)
 
 
 def lstm_tape_views(lstm: "Lstm", tape, B: int, T: int):
@@ -694,14 +730,25 @@ def lstm_tape_views(lstm: "Lstm", tape, B: int, T: int):
              view(off[3 * l + 2], n, torch.bfloat16, (B, T, H))) for l in range(Lyr)]
 
 
-def lstm_train_backward(lstm: "Lstm", tape_pack, dlogits: torch.Tensor, want_dx=False):
-    """BPTT.  Returns dict(weight_ih=[...], weight_hh=[...], bias=[...], head_w, head_b, dx)."""
-    tape, lens, x_bf16 = tape_pack
+def lstm_train_backward(lstm: "Lstm", tape_pack, dlogits: torch.Tensor, want_dx=False, d_state=None,
+                        want_state_grad=False):
+    """BPTT.  Returns dict(weight_ih=[...], weight_hh=[...], bias=[...], head_w, head_b, dx).
+
+    For a stateful tape (lstm_train_forward with `state`): `d_state` = (dh_out, dc_out), the gradients w.r.t. the
+    returned (h_out, c_out) (either may be None = zero), and with `want_state_grad` the dict also holds dh_in and
+    dc_in, f32 (layers, B, H), the gradients w.r.t. the input state."""
+    tape, lens, x_bf16 = tape_pack[:3]
+    stateful = len(tape_pack) > 3
+    if not stateful and (d_state is not None or want_state_grad):
+        raise ValueError("state gradients need a tape from lstm_train_forward(..., state=)")
     B, T, _ = x_bf16.shape
     dev = x_bf16.device
     H, Lyr = lstm.hidden, lstm.layers
     dl = dlogits.detach().to(torch.float32).contiguous()
-    nbytes = L.lib().avvad_lstm_backward_workspace_bytes(lstm.h, B, T)
+    if stateful:
+        nbytes = L.lib().avvad_lstm_backward_state_workspace_bytes(lstm.h, B, T)
+    else:
+        nbytes = L.lib().avvad_lstm_backward_workspace_bytes(lstm.h, B, T)
     if not hasattr(lstm, "bws"):
         lstm.bws = _Workspace()
     ws = lstm.bws.get(nbytes, dev)
@@ -711,12 +758,31 @@ def lstm_train_backward(lstm: "Lstm", tape_pack, dlogits: torch.Tensor, want_dx=
     dhw = torch.empty(lstm.y_dim, H, dtype=torch.float32, device=dev)
     dhb = torch.empty(lstm.y_dim, dtype=torch.float32, device=dev)
     dx = torch.empty(B, T, lstm.input_size, dtype=torch.float32, device=dev) if want_dx else None
-    L.check(L.lib().avvad_lstm_backward(lstm.h, L.ptr(x_bf16), L.ptr(lens), B, T, L.ptr(tape), L.ptr(dl), L.ptr(ws),
-                                        ws.numel(), _ptr_array(dwi), _ptr_array(dwh), _ptr_array(dbs), L.ptr(dhw),
-                                        L.ptr(dhb), L.ptr(dx), L.stream_ptr()))
+    out = {}
+    if stateful:
+        shape = (Lyr, B, H)
+
+        def grad_in(g):
+            if g is None:
+                return None
+            assert tuple(g.shape) == shape, f"state gradient: expected shape {shape}, got {tuple(g.shape)}"
+            return g.detach().to(device=dev, dtype=torch.float32).contiguous()
+        dh_out, dc_out = (grad_in(g) for g in (d_state if d_state is not None else (None, None)))
+        dh_in = torch.empty(shape, dtype=torch.float32, device=dev) if want_state_grad else None
+        dc_in = torch.empty(shape, dtype=torch.float32, device=dev) if want_state_grad else None
+        L.check(L.lib().avvad_lstm_backward_state(lstm.h, L.ptr(x_bf16), L.ptr(lens), B, T, L.ptr(tape), L.ptr(dl),
+                                                  L.ptr(dh_out), L.ptr(dc_out), L.ptr(dh_in), L.ptr(dc_in), L.ptr(ws),
+                                                  ws.numel(), _ptr_array(dwi), _ptr_array(dwh), _ptr_array(dbs),
+                                                  L.ptr(dhw), L.ptr(dhb), L.ptr(dx), L.stream_ptr()))
+        if want_state_grad:
+            out = {"dh_in": dh_in, "dc_in": dc_in}
+    else:
+        L.check(L.lib().avvad_lstm_backward(lstm.h, L.ptr(x_bf16), L.ptr(lens), B, T, L.ptr(tape), L.ptr(dl),
+                                            L.ptr(ws), ws.numel(), _ptr_array(dwi), _ptr_array(dwh), _ptr_array(dbs),
+                                            L.ptr(dhw), L.ptr(dhb), L.ptr(dx), L.stream_ptr()))
     if tape is getattr(lstm, "_tape", None):
         lstm._tape_busy = False
-    return {"weight_ih": dwi, "weight_hh": dwh, "bias": dbs, "head_w": dhw, "head_b": dhb, "dx": dx}
+    return {"weight_ih": dwi, "weight_hh": dwh, "bias": dbs, "head_w": dhw, "head_b": dhb, "dx": dx, **out}
 
 
 def adam_step(param: torch.Tensor, grad: torch.Tensor, exp_avg: torch.Tensor, exp_avg_sq: torch.Tensor, step: int,

@@ -94,6 +94,12 @@ PROTOTYPES = {
     "avvad_lstm_backward_workspace_bytes": (C.c_size_t, [VP, C.c_int64, C.c_int64]),
     "avvad_lstm_backward": (C.c_int, [VP, VP, VP, C.c_int64, C.c_int64, VP, VP, VP, C.c_size_t, VP, VP, VP, VP, VP, VP,
                                       VP]),
+    "avvad_lstm_train_state_workspace_bytes": (C.c_size_t, [VP, C.c_int64, C.c_int64]),
+    "avvad_lstm_forward_train_state": (C.c_int, [VP, VP, VP, C.c_int64, C.c_int64, VP, VP, VP, VP, VP, C.c_size_t, VP,
+                                                 C.c_size_t, VP, VP]),
+    "avvad_lstm_backward_state_workspace_bytes": (C.c_size_t, [VP, C.c_int64, C.c_int64]),
+    "avvad_lstm_backward_state": (C.c_int, [VP, VP, VP, C.c_int64, C.c_int64, VP, VP, VP, VP, VP, VP, VP, C.c_size_t,
+                                            VP, VP, VP, VP, VP, VP, VP]),
     "avvad_adam_step": (C.c_int, [VP, VP, VP, VP, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float, C.c_int64, VP]),
     "avvad_bce_loss": (C.c_int, [VP, VP, VP, C.c_int32, C.c_int32, C.c_int32, C.c_float, VP, VP, VP, VP]),
     "avvad_f1_metrics": (C.c_int, [VP, VP, VP, C.c_int32, C.c_int32, C.c_float, VP, VP, VP]),

@@ -135,6 +135,7 @@ __global__ void gather_state_kernel(const __nv_bfloat16* __restrict__ hseq, cons
 
 namespace avvad {
 struct BpttGraphCache;
+struct BpttState;
 BpttGraphCache* bptt_cache_create();
 void bptt_cache_destroy(BpttGraphCache* c);
 }  // namespace avvad
@@ -259,8 +260,16 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
                        const void* x_bf16, const int32_t* lengths,
                        int64_t B, int64_t T, void* tape, const float* dlogits, void* workspace, size_t workspace_bytes,
                        float* const* dW_ih, float* const* dW_hh, float* const* db, float* dW_head, float* db_head,
-                       float* dx, cudaStream_t st, BpttGraphCache* cache);
+                       float* dx, cudaStream_t st, BpttGraphCache* cache, const BpttState* bs);
 size_t lstm_backward_workspace(int layers, int input_size, int64_t ld0, int H, int y_dim, int64_t B, int64_t T);
+int lstm_backward_state_impl(int layers, int input_size, int64_t ld0, int H, int y_dim, __nv_bfloat16* const* w_ih,
+                             __nv_bfloat16* const* w_hh, const float* head_w32, const __nv_bfloat16* head_w16,
+                             const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T, void* tape,
+                             const float* dlogits, const float* dh_out, const float* dc_out, float* dh_in, float* dc_in,
+                             void* workspace, size_t workspace_bytes, float* const* dW_ih, float* const* dW_hh,
+                             float* const* db, float* dW_head, float* db_head, float* dx, cudaStream_t st,
+                             BpttGraphCache* cache);
+size_t lstm_backward_state_workspace(int layers, int input_size, int64_t ld0, int H, int y_dim, int64_t B, int64_t T);
 }  // namespace avvad
 
 namespace {
@@ -615,7 +624,6 @@ static int lstm_forward_impl(avvad_lstm* h, const void* x_bf16, const int32_t* l
   AVVAD_CHECK_ARG(h && x_bf16 && lengths && workspace && B > 0 && T > 0, "bad argument");
   const bool want_head = logits || post || dec || last_logits;
   AVVAD_CHECK_ARG(want_head || (sio && (sio->h_out || sio->c_out)), "no output requested");
-  AVVAD_CHECK_ARG(!(sio && tape), "lstm: the training forward takes no initial state");
   for (int l = 0; l < h->layers; ++l)
     if (!h->set[l]) {
       set_error("lstm: layer " + std::to_string(l) + " not loaded");
@@ -654,8 +662,10 @@ static int lstm_forward_impl(avvad_lstm* h, const void* x_bf16, const int32_t* l
     AVVAD_LAUNCHED();
     lens_rec = ws.len1;
   }
-  // layer l's initial state: h_in[l] -> position 0 of `hs` (rows `pitch` steps apart), c_in[l] -> c_state
-  auto seed = [&](int l, __nv_bfloat16* hs, int64_t pitch, float* c_state) -> int {
+  // layer l's initial state: h_in[l] -> position 0 of `hs` (rows `pitch` steps apart), c_in[l] -> c_state.  A training
+  // tape (`tv`) also gets c_in at position 0 of its c record and zero gates there: the stateful BPTT reads position 0
+  // as the given state and never differentiates it.
+  auto seed = [&](int l, __nv_bfloat16* hs, int64_t pitch, float* c_state, const TapeView* tv = nullptr) -> int {
     const size_t hrow = (size_t)H * 2, crow = (size_t)H * sizeof(float);
     const int64_t off = (int64_t)l * B * H;
     if (sio->h_in)
@@ -666,6 +676,13 @@ static int lstm_forward_impl(avvad_lstm* h, const void* x_bf16, const int32_t* l
       AVVAD_CUDA(cudaMemcpyAsync(c_state, sio->c_in + off, B * crow, cudaMemcpyDeviceToDevice, st));
     else
       AVVAD_CUDA(cudaMemsetAsync(c_state, 0, B * crow, st));
+    if (tv && tv->gates) {
+      AVVAD_CUDA(cudaMemset2DAsync(tv->gates, pitch * 4 * hrow, 0, 4 * hrow, B, st));
+      if (sio->c_in)
+        AVVAD_CUDA(cudaMemcpy2DAsync(tv->c, pitch * crow, sio->c_in + off, crow, crow, B, cudaMemcpyDeviceToDevice, st));
+      else
+        AVVAD_CUDA(cudaMemset2DAsync(tv->c, pitch * crow, 0, crow, B, st));
+    }
     return AVVAD_OK;
   };
   // layer l's final state from its output sequence and its record of c
@@ -712,8 +729,8 @@ static int lstm_forward_impl(avvad_lstm* h, const void* x_bf16, const int32_t* l
     float* crec1 = ws.cseq[1];
     TapeView tv0{}, tv1{};
     if (tape) {
-      tv0 = tape_layer(tape, 0, H, B, T);
-      tv1 = tape_layer(tape, 1, H, B, T);
+      tv0 = tape_layer(tape, 0, H, B, Ts);
+      tv1 = tape_layer(tape, 1, H, B, Ts);
       out0 = tv0.hseq;
       out1 = tv1.hseq;
       crec0 = tv0.c;
@@ -721,7 +738,7 @@ static int lstm_forward_impl(avvad_lstm* h, const void* x_bf16, const int32_t* l
     }
     int rc;
     if (sio) {  // on `st` before the first chunk's event: the side stream sees layer 1's seed too
-      if ((rc = seed(0, out0, Ts, ws.c)) || (rc = seed(1, out1, Ts, ws.c1))) return rc;
+      if ((rc = seed(0, out0, Ts, ws.c, &tv0)) || (rc = seed(1, out1, Ts, ws.c1, &tv1))) return rc;
     }
     rc = tc::launch_tma_gemm_xt(layer_in, ld_in, h->w_ih[0], ld_in, B, T, T, H4, (int)ld_in, h->bias[0],
                                 ws.xproj + s * H4 * Bp, st);
@@ -758,12 +775,12 @@ static int lstm_forward_impl(avvad_lstm* h, const void* x_bf16, const int32_t* l
     float* crec = ws.cseq[l & 1];
     TapeView tv{};
     if (tape) {
-      tv = tape_layer(tape, l, H, B, T);
+      tv = tape_layer(tape, l, H, B, Ts);
       layer_out = tv.hseq;
       crec = tv.c;
     }
     int rc;
-    if (s && (rc = seed(l, layer_out, Ts, ws.c))) return rc;
+    if (s && (rc = seed(l, layer_out, Ts, ws.c, &tv))) return rc;
     // (1) input projection for every (b,t): xproj = X * W_ih'^T + (b_ih + b_hh)'.  The persistent recurrences read it
     // time-major and unit-major (xT[t][u][b][4]: lane = batch row -> coalesced), the per-step fallback row-major.
     rc = persistent ? tc::launch_tma_gemm_xt(layer_in, ld_in, h->w_ih[l], ld_in, B, T, in_stride, H4, (int)ld_in,
@@ -889,5 +906,44 @@ extern "C" int avvad_lstm_backward(avvad_lstm* h, const void* x_bf16, const int3
   return lstm_backward_impl(h->layers, h->input_size, h->ld0, h->H, h->y_dim, h->w_ih, h->w_hh, h->head_w32,
                             h->head_w16, x_bf16,
                             lengths, B, T, tape, dlogits, workspace, workspace_bytes, dW_ih, dW_hh, db, dW_head, db_head,
-                            dx, (cudaStream_t)stream, h->bptt);
+                            dx, (cudaStream_t)stream, h->bptt, nullptr);
+}
+
+// ---- training with a carried state (truncated BPTT, nn.LSTM's hx).  The forward is avvad_lstm_forward_state's
+// recurrence with a tape of T + 1 positions per row: position 0 holds the initial state (h_in in hseq, c_in in c, zero
+// gates), positions 1..T the call's steps.
+extern "C" size_t avvad_lstm_train_state_workspace_bytes(const avvad_lstm* h, int64_t B, int64_t T) {
+  return avvad_lstm_state_workspace_bytes(h, B, T);
+}
+
+extern "C" int avvad_lstm_forward_train_state(avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B,
+                                              int64_t T, const void* h_in, const float* c_in, void* h_out, float* c_out,
+                                              void* workspace, size_t workspace_bytes, void* tape, size_t tape_bytes,
+                                              float* logits, void* stream) {
+  AVVAD_CHECK_ARG(h && tape && logits, "bad argument");
+  if (tape_bytes < avvad_lstm_tape_bytes(h->layers, h->H, B, T + 1)) {
+    set_error("lstm: tape too small (a stateful tape holds T + 1 positions)");
+    return AVVAD_ERR_WORKSPACE;
+  }
+  const LstmStateIO sio{(const __nv_bfloat16*)h_in, c_in, (__nv_bfloat16*)h_out, c_out};
+  return lstm_forward_impl(h, x_bf16, lengths, B, T, workspace, workspace_bytes, logits, nullptr, nullptr, nullptr, tape,
+                           stream, &sio);
+}
+
+extern "C" size_t avvad_lstm_backward_state_workspace_bytes(const avvad_lstm* h, int64_t B, int64_t T) {
+  if (!h || B <= 0 || T <= 0) return 0;
+  return lstm_backward_state_workspace(h->layers, h->input_size, h->ld0, h->H, h->y_dim, B, T);
+}
+
+extern "C" int avvad_lstm_backward_state(avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T,
+                                         void* tape, const float* dlogits, const float* dh_out, const float* dc_out,
+                                         float* dh_in, float* dc_in, void* workspace, size_t workspace_bytes,
+                                         float* const* dW_ih, float* const* dW_hh, float* const* db, float* dW_head,
+                                         float* db_head, float* dx, void* stream) {
+  AVVAD_CHECK_ARG(h && x_bf16 && lengths && tape && dlogits && workspace && dW_ih && dW_hh && db && dW_head && db_head,
+                  "null pointer");
+  return lstm_backward_state_impl(h->layers, h->input_size, h->ld0, h->H, h->y_dim, h->w_ih, h->w_hh, h->head_w32,
+                                  h->head_w16, x_bf16, lengths, B, T, tape, dlogits, dh_out, dc_out, dh_in, dc_in,
+                                  workspace, workspace_bytes, dW_ih, dW_hh, db, dW_head, db_head, dx,
+                                  (cudaStream_t)stream, h->bptt);
 }

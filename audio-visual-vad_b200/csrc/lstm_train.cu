@@ -11,6 +11,8 @@
 //                             dW_ih = dG^T * X, dW_hh = dG^T * H_prev          (GEMMs over K = B*T on transposed copies)
 //                             db = column sums of dG
 // Gradients are returned in PyTorch's layout (gate-major rows i,f,g,o), fp32.
+// With a carried state (avvad_lstm_backward_state) the same schedules run over a tape of T + 1 positions whose position 0
+// holds the initial state; see lstm_bwd_cell_state_kernel and lstm_backward_state_impl.
 #include <vector>
 
 #include "gemm_tma.cuh"
@@ -124,6 +126,153 @@ __global__ void lstm_bwd_cell_wf_kernel(const __nv_bfloat16* __restrict__ gates1
   *gout = o;
   if (aout) *aout = o;
 }
+// ---- stateful BPTT (avvad_lstm_backward_state).  The tape has T + 1 positions per row and lengths are shifted by one:
+// position 0 holds the initial state (h_in in hseq, c_in in c) and is frozen -- read, never differentiated.  The
+// stateless kernels above are left exactly as they were (their SASS is unchanged); these are their stateful twins.
+//   * position t >= 1 reads cp = c[t-1], so the first step's forget-gate term uses c_in
+//   * at the last valid position len_b (shifted) - 1 the incoming state gradients dh_out / dc_out [B][H] are added
+//   * at position 0 nothing is written to dG but zeros; the state gradients leave as dh_in = the recurrent term of
+//     step 1 (dG_1 * W_hh) and dc_in = dc after step 1.  A row of length 0 has its last valid position at 0, where
+//     the recurrent term is exactly zero: dh_in = dh_out and dc_in = dc_out.
+struct BwdStateArgs {
+  const float* dh_out;  // [B][H] of this layer (zero-filled when the caller passes none)
+  const float* dc_out;
+  float* dh_in;         // null: no state gradient requested
+  float* dc_in;
+};
+__device__ __forceinline__ uint2 lstm_cell_bwd(uint2 gp, float c, float cp, float dh, float* dc) {
+  const float gi = bf16lo(gp.x), gf = bf16hi(gp.x), gg = bf16lo(gp.y), go = bf16hi(gp.y);
+  const float tc = tanhf(c);
+  const float d_o = dh * tc * go * (1.f - go);
+  const float dcc = dh * go * (1.f - tc * tc) + *dc;
+  const float d_i = dcc * gg * gi * (1.f - gi);
+  const float d_g = dcc * gi * (1.f - gg * gg);
+  const float d_f = dcc * cp * gf * (1.f - gf);
+  *dc = dcc * gf;
+  uint2 o;
+  o.x = pack_bf16x2(d_i, d_f);
+  o.y = pack_bf16x2(d_g, d_o);
+  return o;
+}
+// position 0 of a stateful tape: dh_rec_sum = the recurrent term from step 1 (exactly zero for a row of length 0)
+__device__ __forceinline__ void lstm_state_grad_out(const BwdStateArgs& sa, int idx, bool last, float dh_rec_sum,
+                                                    float dc) {
+  if (sa.dh_in) sa.dh_in[idx] = (last ? sa.dh_out[idx] : 0.f) + dh_rec_sum;
+  if (sa.dc_in) sa.dc_in[idx] = dc + (last ? sa.dc_out[idx] : 0.f);
+}
+
+__global__ void lstm_bwd_cell_state_kernel(const __nv_bfloat16* __restrict__ gates, const float* __restrict__ cst,
+                                           const float* __restrict__ dY, const float* __restrict__ dl,
+                                           const float* __restrict__ w_head, const float* __restrict__ dh_rec,
+                                           float* __restrict__ dc, const int32_t* __restrict__ lengths, int B, int T,
+                                           int H, int t, int has_rec, __nv_bfloat16* __restrict__ dG, BwdStateArgs sa) {
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= B * H) return;
+  const int b = idx / H, u = idx - b * H;
+  const int64_t row = (int64_t)b * T + t;
+  uint2* out = reinterpret_cast<uint2*>(dG + row * 4 * H + 4 * u);
+  const int len = lengths[b];
+  if (t == 0) {  // frozen initial state
+    float rec = 0.f;
+    for (int sp = 0; sp < has_rec; ++sp) rec += dh_rec[(int64_t)sp * B * H + idx];
+    lstm_state_grad_out(sa, idx, len == 1, rec, dc[idx]);
+    *out = make_uint2(0u, 0u);
+    return;
+  }
+  if (t >= len) {
+    *out = make_uint2(0u, 0u);
+    dc[idx] = 0.f;
+    return;
+  }
+  const uint2 gp = *reinterpret_cast<const uint2*>(gates + row * 4 * H + 4 * u);
+  const float c = cst[row * H + u];
+  const float cp = cst[(row - 1) * H + u];
+  float dh = dY ? dY[row * H + u] : dl[row] * w_head[u];
+  for (int sp = 0; sp < has_rec; ++sp) dh += dh_rec[(int64_t)sp * B * H + idx];
+  float dcv = dc[idx];
+  if (t == len - 1) {
+    dh += sa.dh_out[idx];
+    dcv += sa.dc_out[idx];
+  }
+  *out = lstm_cell_bwd(gp, c, cp, dh, &dcv);
+  dc[idx] = dcv;
+}
+
+// Stateful twin of lstm_bwd_cell_wf_kernel (same schedule over T + 1 positions); sa0 / sa1: layer 0 / layer 1
+__global__ void lstm_bwd_cell_wf_state_kernel(const __nv_bfloat16* __restrict__ gates1, const float* __restrict__ cst1,
+                                              const __nv_bfloat16* __restrict__ gates0, const float* __restrict__ cst0,
+                                              const float* __restrict__ dY1, const float* __restrict__ dl,
+                                              const float* __restrict__ w_head, const float* __restrict__ Cpart,
+                                              int nsplit, float* __restrict__ dc2, const int32_t* __restrict__ lengths,
+                                              int B, int T, int H, int s, __nv_bfloat16* __restrict__ dG1,
+                                              __nv_bfloat16* __restrict__ dG0, __nv_bfloat16* __restrict__ Abuf,
+                                              BwdStateArgs sa1, BwdStateArgs sa0) {
+  const int layer = 1 - (int)blockIdx.y;
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= B * H) return;
+  const int b = idx / H, u = idx - b * H;
+  const int t = (layer == 1) ? (T - 1 - s) : (T - s);
+  const int64_t K2 = 8ll * H;
+  uint2* aout = Abuf ? reinterpret_cast<uint2*>(Abuf + (int64_t)(layer == 1 ? b : B + b) * K2 + (layer == 1 ? 0 : 4 * H) + 4 * u)
+                     : nullptr;
+  if (t < 0 || t > T - 1) {
+    if (aout) *aout = make_uint2(0u, 0u);
+    return;
+  }
+  const int64_t row = (int64_t)b * T + t;
+  __nv_bfloat16* dG = layer == 1 ? dG1 : dG0;
+  uint2* gout = reinterpret_cast<uint2*>(dG + row * 4 * H + 4 * u);
+  float* dc = dc2 + (int64_t)layer * B * H;
+  const int64_t cstride = 2ll * B * 2 * H;
+  const int len = lengths[b];
+  if (t == 0) {  // frozen initial state: the recurrent term of step 1 is dh_in
+    float rec = 0.f;
+    if (layer == 1) {
+      if (s > 0)
+        for (int sp = 0; sp < nsplit; ++sp) rec += Cpart[sp * cstride + (int64_t)b * 2 * H + u];
+    } else if (T > 1) {
+      for (int sp = 0; sp < nsplit; ++sp) rec += Cpart[sp * cstride + (int64_t)(B + b) * 2 * H + u];
+    }
+    lstm_state_grad_out(layer == 1 ? sa1 : sa0, idx, len == 1, rec, dc[idx]);
+    *gout = make_uint2(0u, 0u);
+    if (aout) *aout = make_uint2(0u, 0u);
+    return;
+  }
+  if (t >= len) {
+    *gout = make_uint2(0u, 0u);
+    if (aout) *aout = make_uint2(0u, 0u);
+    dc[idx] = 0.f;
+    return;
+  }
+  const __nv_bfloat16* gates = layer == 1 ? gates1 : gates0;
+  const float* cst = layer == 1 ? cst1 : cst0;
+  const uint2 gp = *reinterpret_cast<const uint2*>(gates + row * 4 * H + 4 * u);
+  const float c = cst[row * H + u];
+  const float cp = cst[(row - 1) * H + u];
+  float dh;
+  if (layer == 1) {
+    dh = dY1 ? dY1[row * H + u] : dl[row] * w_head[u];
+    if (s > 0)
+      for (int sp = 0; sp < nsplit; ++sp) dh += Cpart[sp * cstride + (int64_t)b * 2 * H + u];
+  } else {
+    dh = 0.f;
+    for (int sp = 0; sp < nsplit; ++sp) {
+      dh += Cpart[sp * cstride + (int64_t)b * 2 * H + H + u];
+      if (t < T - 1) dh += Cpart[sp * cstride + (int64_t)(B + b) * 2 * H + u];
+    }
+  }
+  float dcv = dc[idx];
+  if (t == len - 1) {
+    const BwdStateArgs& sa = layer == 1 ? sa1 : sa0;
+    dh += sa.dh_out[idx];
+    dcv += sa.dc_out[idx];
+  }
+  const uint2 o = lstm_cell_bwd(gp, c, cp, dh, &dcv);
+  dc[idx] = dcv;
+  *gout = o;
+  if (aout) *aout = o;
+}
+
 // Wcat [2H][8H] from the gate-interleaved packed weights W' [4H][ld] (see the layout above)
 __global__ void lstm_wf_pack_w_kernel(const __nv_bfloat16* __restrict__ whh1, const __nv_bfloat16* __restrict__ wih1,
                                       const __nv_bfloat16* __restrict__ whh0, int H, __nv_bfloat16* __restrict__ out) {
@@ -365,13 +514,27 @@ struct BpttGraphCache {
 BpttGraphCache* bptt_cache_create() { return new BpttGraphCache(); }
 void bptt_cache_destroy(BpttGraphCache* c) { delete c; }
 
+// Stateful backward (the tape and `lengths` of lstm_backward_impl are then those of T + 1 positions, position 0 =
+// state): the state gradients in f32 [L][B][H], all at stable workspace addresses so that the captured graphs replay.
+// dh_in / dc_in null: no state gradient requested, and the recurrent GEMM of step 1 is skipped.
+struct BpttState {
+  const float* dh_out;
+  const float* dc_out;
+  float* dh_in;
+  float* dc_in;
+  BwdStateArgs layer(int l, int64_t B, int H) const {
+    const int64_t o = (int64_t)l * B * H;
+    return BwdStateArgs{dh_out + o, dc_out + o, dh_in ? dh_in + o : nullptr, dc_in ? dc_in + o : nullptr};
+  }
+};
+
 // exposed to lstm.cu
 int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim, __nv_bfloat16* const* w_ih,
                        __nv_bfloat16* const* w_hh, const float* head_w32, const __nv_bfloat16* head_w16,
                        const void* x_bf16, const int32_t* lengths,
                        int64_t B, int64_t T, void* tape, const float* dlogits, void* workspace, size_t workspace_bytes,
                        float* const* dW_ih, float* const* dW_hh, float* const* db, float* dW_head, float* db_head,
-                       float* dx, cudaStream_t st, BpttGraphCache* cache);
+                       float* dx, cudaStream_t st, BpttGraphCache* cache, const BpttState* bs);
 // split-K factor of the per-step recurrent-gradient GEMMs (AVVAD_BPTT_SPLIT = 1..8, buffers are sized for 8)
 constexpr int kBpttSplitMax = 8;
 // Default: 8 for per-rank batches up to 64 rows (one m-tile: 256 CTAs instead of 128, backward 6.0 -> 5.4 ms at B = 32),
@@ -549,7 +712,7 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
                        const void* x_bf16, const int32_t* lengths,
                        int64_t B, int64_t T, void* tape, const float* dlogits, void* workspace, size_t workspace_bytes,
                        float* const* dW_ih, float* const* dW_hh, float* const* db, float* dW_head, float* db_head,
-                       float* dx, cudaStream_t st, BpttGraphCache* cache) {
+                       float* dx, cudaStream_t st, BpttGraphCache* cache, const BpttState* bs) {
   AVVAD_CHECK_ARG(y_dim >= 1, "bad y_dim");
   AVVAD_CHECK_ARG(workspace_bytes >= lstm_backward_workspace(layers, input_size, ld0, H, y_dim, B, T),
                   "workspace too small");
@@ -576,6 +739,21 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
   const float* dl_step = (y_dim == 1) ? dl_st : dlogits;
   const bool use_graph = cache && bptt_graph_enabled() && !tc::profiling_on() && !sync_debug();
   const int kBpttSplit = bptt_split(B);  // split-K factor of the per-step GEMMs of this call
+  // stateful: the last position visited (0 when state gradients leave through the frozen position 0, else 1)
+  const int t_min = (bs && !bs->dh_in) ? 1 : 0;
+  // stateful: position 0 of dG is never differentiated; zero it once so the weight-gradient GEMMs see zero rows even
+  // where the recurrence stops at position 1
+  auto zero_pos0 = [&](__nv_bfloat16* dGl) -> int {
+    if (bs) AVVAD_CUDA(cudaMemset2DAsync(dGl, (size_t)T * H4 * 2, 0, (size_t)H4 * 2, (size_t)B, st));
+    return AVVAD_OK;
+  };
+  // the state's kernel-parameter pointers join the graph keys (a stateless key is shorter, so the two never match)
+  auto state_key = [&](std::vector<uintptr_t> key) {
+    if (bs)
+      for (uintptr_t v : {(uintptr_t)bs->dh_out, (uintptr_t)bs->dc_out, (uintptr_t)bs->dh_in, (uintptr_t)bs->dc_in})
+        key.push_back(v);
+    return key;
+  };
 
   const float* dY_head = nullptr;  // y_dim > 1: gradient of the top layer's output through the head (GEMM)
   if (y_dim == 1) {
@@ -699,6 +877,8 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
                                                                                           Wcat);
     AVVAD_LAUNCHED();
     AVVAD_CUDA(cudaMemsetAsync(dc2, 0, (size_t)2 * B * H * 4, st));
+    if (int rcz = zero_pos0(dG)) return rcz;
+    if (int rcz = zero_pos0(dG0)) return rcz;
     if (wf_mode == 1) AVVAD_CUDA(cudaMemsetAsync(Abuf, 0, (size_t)128 * 8 * H * 2, st));  // rows 2B..127 stay zero
     const int64_t cstride = 2 * B * 2 * H;
     // mode 1: C [2B][2H] = A [2B][8H] * Wcat^T
@@ -734,11 +914,16 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
       }();
       cudaStream_t s2 = (use_graph && wf_mode == 2 && fork_pref) ? cache->cap_stream2 : nullptr;
       for (int s = 0; s <= (int)T; ++s) {
-        lstm_bwd_cell_wf_kernel<<<dim3((unsigned)ceil_div(B * H, 256), 2), 256, 0, s1>>>(
-            t1.gates, t1.c, t0.gates, t0.c, dY_head, dl_step, head_w32, Cpart, kBpttSplit, dc2, len_st, (int)B, (int)T, H,
-            s, dG, dG0, wf_mode == 1 ? Abuf : nullptr);
+        if (bs)  // layer 0 reaches position 1 in iteration T - 1 and the frozen position 0 in iteration T
+          lstm_bwd_cell_wf_state_kernel<<<dim3((unsigned)ceil_div(B * H, 256), 2), 256, 0, s1>>>(
+              t1.gates, t1.c, t0.gates, t0.c, dY_head, dl_step, head_w32, Cpart, kBpttSplit, dc2, len_st, (int)B, (int)T,
+              H, s, dG, dG0, wf_mode == 1 ? Abuf : nullptr, bs->layer(1, B, H), bs->layer(0, B, H));
+        else
+          lstm_bwd_cell_wf_kernel<<<dim3((unsigned)ceil_div(B * H, 256), 2), 256, 0, s1>>>(
+              t1.gates, t1.c, t0.gates, t0.c, dY_head, dl_step, head_w32, Cpart, kBpttSplit, dc2, len_st, (int)B, (int)T,
+              H, s, dG, dG0, wf_mode == 1 ? Abuf : nullptr);
         AVVAD_LAUNCHED();
-        if (s >= (int)T) break;
+        if (s >= (int)T - t_min) break;
         if (wf_mode == 1) {
           int rc = wf_gemm(s1);
           if (rc) return rc;
@@ -765,11 +950,12 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
       }
       return AVVAD_OK;
     };
-    const std::vector<uintptr_t> key = {(uintptr_t)t1.gates, (uintptr_t)t1.c, (uintptr_t)t0.gates, (uintptr_t)t0.c,
+    std::vector<uintptr_t> key = {(uintptr_t)t1.gates, (uintptr_t)t1.c, (uintptr_t)t0.gates, (uintptr_t)t0.c,
                                         (uintptr_t)dY_head, (uintptr_t)dl_step, (uintptr_t)head_w32, (uintptr_t)Cpart,
                                         (uintptr_t)dc2, (uintptr_t)len_st, (uintptr_t)dG, (uintptr_t)dG0,
                                         (uintptr_t)Abuf, (uintptr_t)Wcat, (uintptr_t)B, (uintptr_t)T, (uintptr_t)H,
                                         (uintptr_t)wf_mode};
+    key = state_key(key);
     auto warm = [&]() -> int {
       if (wf_mode == 1) return wf_gemm(st);
       int rc = gemm_l1(0, st);
@@ -811,15 +997,23 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
     AVVAD_LAUNCHED();
     AVVAD_CUDA(cudaMemsetAsync(dc, 0, (size_t)B * H * 4, st));
     AVVAD_CUDA(cudaMemsetAsync(dc0, 0, (size_t)B * H * 4, st));
-    // steps te-1 .. tb of one layer: (cell, recurrent split-K GEMM) pairs
-    auto steps_of = [&](const TapeView& tv, const float* dYl, float* dh, float* dcl, __nv_bfloat16* dGl,
+    if (int rcz = zero_pos0(dG)) return rcz;
+    if (int rcz = zero_pos0(dG0)) return rcz;
+    // steps te-1 .. tb of layer l: (cell, recurrent split-K GEMM) pairs
+    auto steps_of = [&](int l, const TapeView& tv, const float* dYl, float* dh, float* dcl, __nv_bfloat16* dGl,
                         const __nv_bfloat16* WTl, int tb, int te, cudaStream_t s2) -> int {
-      for (int t = te - 1; t >= tb; --t) {
+      for (int t = te - 1; t >= tb && t >= t_min; --t) {
         const int has_rec = (t < (int)T - 1) ? kBpttSplit : 0;
-        lstm_bwd_cell_kernel<<<(unsigned)ceil_div(B * H, 256), 256, 0, s2>>>(tv.gates, tv.c, dYl, dl_step, head_w32, dh, dcl,
-                                                                            len_st, (int)B, (int)T, H, t, has_rec, dGl);
+        if (bs)
+          lstm_bwd_cell_state_kernel<<<(unsigned)ceil_div(B * H, 256), 256, 0, s2>>>(
+              tv.gates, tv.c, dYl, dl_step, head_w32, dh, dcl, len_st, (int)B, (int)T, H, t, has_rec, dGl,
+              bs->layer(l, B, H));
+        else
+          lstm_bwd_cell_kernel<<<(unsigned)ceil_div(B * H, 256), 256, 0, s2>>>(tv.gates, tv.c, dYl, dl_step, head_w32, dh,
+                                                                              dcl, len_st, (int)B, (int)T, H, t, has_rec,
+                                                                              dGl);
         AVVAD_LAUNCHED();
-        if (t > 0) {
+        if (t > t_min) {
           tc::EpiParams ep{};
           ep.C = dh;
           ep.ldc = H;
@@ -848,12 +1042,14 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
     for (int c = n_chunks - 1; c >= 0; --c) {
       const int tb = (int)(T * c / n_chunks), te = (int)(T * (c + 1) / n_chunks);
       {  // layer 1, chunk c, on the caller's stream
-        const std::vector<uintptr_t> key = {(uintptr_t)tv1.gates, (uintptr_t)tv1.c, (uintptr_t)dY_head, (uintptr_t)dl_step,
-                                            (uintptr_t)head_w32, (uintptr_t)dh_rec, (uintptr_t)dc, (uintptr_t)len_st,
-                                            (uintptr_t)dG, (uintptr_t)WT, (uintptr_t)B, (uintptr_t)T, (uintptr_t)H,
-                                            (uintptr_t)tb, (uintptr_t)te, (uintptr_t)kBpttSplit};
+        const std::vector<uintptr_t> key = state_key({(uintptr_t)tv1.gates, (uintptr_t)tv1.c, (uintptr_t)dY_head,
+                                                      (uintptr_t)dl_step, (uintptr_t)head_w32, (uintptr_t)dh_rec,
+                                                      (uintptr_t)dc, (uintptr_t)len_st, (uintptr_t)dG, (uintptr_t)WT,
+                                                      (uintptr_t)B, (uintptr_t)T, (uintptr_t)H, (uintptr_t)tb,
+                                                      (uintptr_t)te, (uintptr_t)kBpttSplit});
         int rc = run_captured(use_graph ? cache : nullptr, 3 + c, key, no_warm,
-                              [&](cudaStream_t s2) { return steps_of(tv1, dY_head, dh_rec, dc, dG, WT, tb, te, s2); }, st);
+                              [&](cudaStream_t s2) { return steps_of(1, tv1, dY_head, dh_rec, dc, dG, WT, tb, te, s2); },
+                              st);
         if (rc) return rc;
       }
       AVVAD_CUDA(cudaEventRecord(cache->ev_chunk[c], st));
@@ -862,12 +1058,14 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
       int rc = tc::launch_tma_gemm_tm(dG + (int64_t)tb * H4, H4, WTi, H4, B, te - tb, T, H, H4, dY0 + (int64_t)tb * H, H, side);
       if (rc) return rc;
       {  // layer 0, chunk c, on the side stream
-        const std::vector<uintptr_t> key = {(uintptr_t)tv0.gates, (uintptr_t)tv0.c, (uintptr_t)dY0, (uintptr_t)dl_step,
-                                            (uintptr_t)head_w32, (uintptr_t)dh_rec0, (uintptr_t)dc0, (uintptr_t)len_st,
-                                            (uintptr_t)dG0, (uintptr_t)WT0, (uintptr_t)B, (uintptr_t)T, (uintptr_t)H,
-                                            (uintptr_t)tb, (uintptr_t)te, (uintptr_t)kBpttSplit};
+        const std::vector<uintptr_t> key = state_key({(uintptr_t)tv0.gates, (uintptr_t)tv0.c, (uintptr_t)dY0,
+                                                      (uintptr_t)dl_step, (uintptr_t)head_w32, (uintptr_t)dh_rec0,
+                                                      (uintptr_t)dc0, (uintptr_t)len_st, (uintptr_t)dG0, (uintptr_t)WT0,
+                                                      (uintptr_t)B, (uintptr_t)T, (uintptr_t)H, (uintptr_t)tb,
+                                                      (uintptr_t)te, (uintptr_t)kBpttSplit});
         rc = run_captured(use_graph ? cache : nullptr, 3 + kBpttMaxChunks + c, key, no_warm,
-                          [&](cudaStream_t s2) { return steps_of(tv0, dY0, dh_rec0, dc0, dG0, WT0, tb, te, s2); }, side);
+                          [&](cudaStream_t s2) { return steps_of(0, tv0, dY0, dh_rec0, dc0, dG0, WT0, tb, te, s2); },
+                          side);
         if (rc) return rc;
       }
     }
@@ -888,13 +1086,20 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
     transpose_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * H, 256), 256, 0, st>>>(w_hh[l], H4, H, H, WT);
     AVVAD_LAUNCHED();
     AVVAD_CUDA(cudaMemsetAsync(dc, 0, (size_t)B * H * 4, st));
+    if (int rcz = zero_pos0(dG)) return rcz;
     auto run_steps = [&](cudaStream_t st) -> int {   // `st`: the caller's stream, or the capture stream
-      for (int t = (int)T - 1; t >= 0; --t) {
+      for (int t = (int)T - 1; t >= t_min; --t) {
         const int has_rec = (t < (int)T - 1) ? kBpttSplit : 0;  // number of partial products to sum
-        lstm_bwd_cell_kernel<<<(unsigned)ceil_div(B * H, 256), 256, 0, st>>>(tv.gates, tv.c, dY, dl_step, head_w32, dh_rec,
-                                                                            dc, len_st, (int)B, (int)T, H, t, has_rec, dG);
+        if (bs)
+          lstm_bwd_cell_state_kernel<<<(unsigned)ceil_div(B * H, 256), 256, 0, st>>>(
+              tv.gates, tv.c, dY, dl_step, head_w32, dh_rec, dc, len_st, (int)B, (int)T, H, t, has_rec, dG,
+              bs->layer(l, B, H));
+        else
+          lstm_bwd_cell_kernel<<<(unsigned)ceil_div(B * H, 256), 256, 0, st>>>(tv.gates, tv.c, dY, dl_step, head_w32,
+                                                                              dh_rec, dc, len_st, (int)B, (int)T, H, t,
+                                                                              has_rec, dG);
         AVVAD_LAUNCHED();
-        if (t > 0) {
+        if (t > t_min) {
           tc::EpiParams ep{};
           ep.C = dh_rec;
           ep.ldc = H;
@@ -907,9 +1112,10 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
       return AVVAD_OK;
     };
     {
-      const std::vector<uintptr_t> key = {(uintptr_t)tv.gates, (uintptr_t)tv.c, (uintptr_t)dY, (uintptr_t)dl_step,
-                                          (uintptr_t)head_w32, (uintptr_t)dh_rec, (uintptr_t)dc, (uintptr_t)len_st,
-                                          (uintptr_t)dG, (uintptr_t)WT, (uintptr_t)B, (uintptr_t)T, (uintptr_t)H};
+      const std::vector<uintptr_t> key = state_key({(uintptr_t)tv.gates, (uintptr_t)tv.c, (uintptr_t)dY,
+                                                    (uintptr_t)dl_step, (uintptr_t)head_w32, (uintptr_t)dh_rec,
+                                                    (uintptr_t)dc, (uintptr_t)len_st, (uintptr_t)dG, (uintptr_t)WT,
+                                                    (uintptr_t)B, (uintptr_t)T, (uintptr_t)H});
       auto warm = [&]() -> int {   // the kernels' one-time attribute setup is not capturable: one real split-K launch
         tc::EpiParams ep{};
         ep.C = dh_rec;
@@ -928,6 +1134,97 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
       dX_out = (dX_out == dYa) ? dYb : dYa;
     }
   }
+  return AVVAD_OK;
+}
+
+// ---- stateful backward (avvad_lstm_backward_state) over a tape of T + 1 positions per row.  The per-call tensors of
+// T steps are laid out once more with a leading position 0 -- zero rows of x and dlogits, lengths + 1 -- so that
+// lstm_backward_impl runs its schedules unchanged over T + 1 positions; dx is read back from positions 1..T.
+__global__ void shift_lengths_bwd_kernel(const int32_t* __restrict__ lengths, int B, int32_t* __restrict__ out) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b < B) out[b] = lengths[b] + 1;
+}
+
+namespace {
+struct StateBwdWs {
+  int32_t* len1;
+  __nv_bfloat16* x1;  // [B][T+1][ld0]
+  float* dl1;         // [B][T+1][y_dim]
+  float* dx1;         // [B][T+1][input_size]
+  float *dh_out, *dc_out, *dh_in, *dc_in;  // [L][B][H]
+  uint8_t* inner;     // lstm_backward_impl's workspace
+  size_t total;
+};
+StateBwdWs carve_state_bwd(int layers, int input_size, int64_t ld0, int H, int y_dim, int64_t B, int64_t T, void* base) {
+  StateBwdWs w{};
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    void* p = base ? (uint8_t*)base + off : nullptr;
+    off += align_up(bytes, 256);
+    return p;
+  };
+  const int64_t T1 = T + 1;
+  const size_t st = (size_t)layers * B * H * sizeof(float);
+  w.len1 = (int32_t*)take((size_t)B * 4);
+  w.x1 = (__nv_bfloat16*)take((size_t)B * T1 * ld0 * 2);
+  w.dl1 = (float*)take((size_t)B * T1 * y_dim * 4);
+  w.dx1 = (float*)take((size_t)B * T1 * input_size * 4);
+  w.dh_out = (float*)take(st);
+  w.dc_out = (float*)take(st);
+  w.dh_in = (float*)take(st);
+  w.dc_in = (float*)take(st);
+  w.inner = (uint8_t*)take(0);
+  w.total = off + lstm_backward_workspace(layers, input_size, ld0, H, y_dim, B, T1);
+  return w;
+}
+}  // namespace
+
+size_t lstm_backward_state_workspace(int layers, int input_size, int64_t ld0, int H, int y_dim, int64_t B, int64_t T) {
+  return carve_state_bwd(layers, input_size, ld0, H, y_dim, B, T, nullptr).total;
+}
+
+int lstm_backward_state_impl(int layers, int input_size, int64_t ld0, int H, int y_dim, __nv_bfloat16* const* w_ih,
+                             __nv_bfloat16* const* w_hh, const float* head_w32, const __nv_bfloat16* head_w16,
+                             const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T, void* tape,
+                             const float* dlogits, const float* dh_out, const float* dc_out, float* dh_in, float* dc_in,
+                             void* workspace, size_t workspace_bytes, float* const* dW_ih, float* const* dW_hh,
+                             float* const* db, float* dW_head, float* db_head, float* dx, cudaStream_t st,
+                             BpttGraphCache* cache) {
+  AVVAD_CHECK_ARG(B > 0 && T > 0, "bad sizes");
+  const StateBwdWs w = carve_state_bwd(layers, input_size, ld0, H, y_dim, B, T, workspace);
+  AVVAD_CHECK_ARG(workspace_bytes >= w.total, "workspace too small");
+  const int64_t T1 = T + 1;
+  shift_lengths_bwd_kernel<<<(unsigned)ceil_div(B, 256), 256, 0, st>>>(lengths, (int)B, w.len1);
+  AVVAD_LAUNCHED();
+  // [B][T][n] -> [B][T+1][n] with a zero row at position 0
+  auto widen = [&](void* dst, const void* src, size_t row_bytes) -> int {
+    AVVAD_CUDA(cudaMemset2DAsync(dst, T1 * row_bytes, 0, row_bytes, (size_t)B, st));
+    AVVAD_CUDA(cudaMemcpy2DAsync((uint8_t*)dst + row_bytes, T1 * row_bytes, src, T * row_bytes, T * row_bytes, (size_t)B,
+                                 cudaMemcpyDeviceToDevice, st));
+    return AVVAD_OK;
+  };
+  int rc = widen(w.x1, x_bf16, (size_t)ld0 * 2);
+  if (!rc) rc = widen(w.dl1, dlogits, (size_t)y_dim * 4);
+  if (rc) return rc;
+  // the state gradients at stable addresses (inputs copied first, so outputs may alias them)
+  const size_t sbytes = (size_t)layers * B * H * sizeof(float);
+  if (dh_out) AVVAD_CUDA(cudaMemcpyAsync(w.dh_out, dh_out, sbytes, cudaMemcpyDeviceToDevice, st));
+  else AVVAD_CUDA(cudaMemsetAsync(w.dh_out, 0, sbytes, st));
+  if (dc_out) AVVAD_CUDA(cudaMemcpyAsync(w.dc_out, dc_out, sbytes, cudaMemcpyDeviceToDevice, st));
+  else AVVAD_CUDA(cudaMemsetAsync(w.dc_out, 0, sbytes, st));
+  const bool want = dh_in || dc_in;
+  const BpttState bs{w.dh_out, w.dc_out, want ? w.dh_in : nullptr, want ? w.dc_in : nullptr};
+  rc = lstm_backward_impl(layers, input_size, ld0, H, y_dim, w_ih, w_hh, head_w32, head_w16, w.x1, w.len1, B, T1, tape,
+                          w.dl1, w.inner, workspace_bytes - (size_t)(w.inner - (uint8_t*)workspace), dW_ih, dW_hh, db,
+                          dW_head, db_head, dx ? w.dx1 : nullptr, st, cache, &bs);
+  if (rc) return rc;
+  if (dx) {
+    const size_t row = (size_t)input_size * 4;
+    AVVAD_CUDA(cudaMemcpy2DAsync(dx, T * row, (uint8_t*)w.dx1 + row, T1 * row, T * row, (size_t)B,
+                                 cudaMemcpyDeviceToDevice, st));
+  }
+  if (dh_in) AVVAD_CUDA(cudaMemcpyAsync(dh_in, w.dh_in, sbytes, cudaMemcpyDeviceToDevice, st));
+  if (dc_in) AVVAD_CUDA(cudaMemcpyAsync(dc_in, w.dc_in, sbytes, cudaMemcpyDeviceToDevice, st));
   return AVVAD_OK;
 }
 }  // namespace avvad

@@ -7,8 +7,8 @@ import torchvision.models as models
 from .compact_bilinear_pooling import CompactBilinearPooling
 from .utils import weights_init_normal
 from ._engine import (E, EngineCache, LstmHeadFunction, McbBnFunction, TrunkFunction, all_parameters, bump_generation,
-                      device_of, full_state_dict, lstm_params, on_input_device, select_state, trunk_bn_modules,
-                      trunk_engine, trunk_params)
+                      device_of, full_state_dict, lstm_params, lstm_with_hx, on_input_device, select_state,
+                      trunk_bn_modules, trunk_engine, trunk_params)
 
 
 class DeepVAD_AV(nn.Module):
@@ -74,8 +74,17 @@ class DeepVAD_AV(nn.Module):
         return eng
 
     @on_input_device
-    def forward(self, audio, video, lengths, return_posteriors=False):
-        """audio (B,T,513), video (B,T,67,67), lengths list / CPU / CUDA tensor -> logits (B,T,y_dim)."""
+    def forward(self, audio, video, lengths, return_posteriors=False, hx=None):
+        """audio (B,T,513), video (B,T,67,67), lengths list / CPU / CUDA tensor -> logits (B,T,y_dim).
+
+        ``hx = (h0, c0)``, each (lstm_layers, B, H) as for nn.LSTM: the LSTM continues from that state and the call
+        returns ``(logits, (h_n, c_n))`` with the state at each row's last valid step; in a training step gradients
+        flow to h0 / c0 and from h_n / c_n.  Feeding h_n / c_n (detached) into the next block of the same utterances
+        trains it in blocks (truncated BPTT).  Blocks of one utterance are separate calls, so the quantities a call
+        computes over all its frames -- train()-mode BatchNorm statistics and, with MCB, the L2 norm of the fused features -- are per block: the caller decides
+        whether that is what it wants."""
+        if hx is not None and return_posteriors:
+            raise ValueError("hx: posteriors are not returned with a state; apply a sigmoid to the logits")
         device = device_of(audio, video)
         eng = self._build(device)
         batch, frames, height, width = video.size()
@@ -135,6 +144,9 @@ class DeepVAD_AV(nn.Module):
                 E.pack_rows_bf16(feat.detach(), xv, self.num_audio_ftrs, False)
                 # the LSTM's input gradient (B,T,1025) reaches the trunk through this concatenation (AV_Net.py:124)
                 proxy = torch.cat([aud.view(batch, frames, -1), feat.view(batch, frames, -1)], dim=2)
+        if hx is not None:
+            return lstm_with_hx(eng["lstm"], x, lengths, proxy, hx, lstm_params(self.lstm_merged, self.vad_merged),
+                                need_grad)
         if need_grad:
             return LstmHeadFunction.apply(eng["lstm"], x, lengths, proxy,
                                           *lstm_params(self.lstm_merged, self.vad_merged))

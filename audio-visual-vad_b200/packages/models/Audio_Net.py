@@ -4,7 +4,7 @@ import torch.nn as nn
 
 from .utils import weights_init_normal
 from ._engine import (E, EngineCache, LstmHeadFunction, all_parameters, device_of, full_state_dict, lstm_params,
-                      on_input_device, select_state)
+                      lstm_with_hx, on_input_device, select_state)
 
 
 class DeepVAD_audio(nn.Module):
@@ -41,14 +41,25 @@ class DeepVAD_audio(nn.Module):
                                           lambda e: e.load(sd, device, "lstm_audio", "vad_audio"))}
 
     @on_input_device
-    def forward(self, x, lengths, return_posteriors=False):
-        """x (B,T,513) standardised log-power, lengths -> logits (B,T,y_dim)."""
+    def forward(self, x, lengths, return_posteriors=False, hx=None):
+        """x (B,T,513) standardised log-power, lengths -> logits (B,T,y_dim).
+
+        ``hx = (h0, c0)``, each (lstm_layers, B, H) as for nn.LSTM: the LSTM continues from that state and the call
+        returns ``(logits, (h_n, c_n))`` with the state at each row's last valid step; in a training step gradients
+        flow to h0 / c0 and from h_n / c_n.  Feeding h_n / c_n (detached) into the next block of the same utterances
+        trains it in blocks (truncated BPTT)."""
+        if hx is not None and return_posteriors:
+            raise ValueError("hx: posteriors are not returned with a state; apply a sigmoid to the logits")
         device = device_of(x)
         eng = self._build(device)
         B, T, F = x.shape
         xb = eng["lstm"].new_input(B, T, device)
         E.pack_rows_bf16(x.detach().to(torch.float32).reshape(B * T, F).contiguous(), xb.view(B * T, -1), 0, False)
-        if torch.is_grad_enabled() and any(p.requires_grad for p in all_parameters(self)):
+        train = torch.is_grad_enabled() and any(p.requires_grad for p in all_parameters(self))
+        if hx is not None:
+            return lstm_with_hx(eng["lstm"], xb, lengths, x if x.requires_grad else None, hx,
+                                lstm_params(self.lstm_audio, self.vad_audio), train)
+        if train:
             # training step: forward keeps a tape, loss.backward() runs BPTT on the device (SURVEY O1)
             return LstmHeadFunction.apply(eng["lstm"], xb, lengths, x if x.requires_grad else None,
                                           *lstm_params(self.lstm_audio, self.vad_audio))

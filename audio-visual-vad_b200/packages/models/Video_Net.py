@@ -5,8 +5,8 @@ import torchvision.models as models
 
 from .utils import weights_init_normal, method1, method3  # noqa: F401  (re-exported like the reference)
 from ._engine import (E, EngineCache, LstmHeadFunction, TrunkFunction, all_parameters, bump_generation, device_of,
-                      full_state_dict, lstm_params, on_input_device, select_state, trunk_bn_modules, trunk_engine,
-                      trunk_params)
+                      full_state_dict, lstm_params, lstm_with_hx, on_input_device, select_state, trunk_bn_modules,
+                      trunk_engine, trunk_params)
 
 
 class DeepVAD_video(nn.Module):
@@ -48,8 +48,17 @@ class DeepVAD_video(nn.Module):
                               lambda e: e.load(sd, device, "lstm_video", "vad_video"))}
 
     @on_input_device
-    def forward(self, x, lengths, return_last=False):
-        """x (B,T,67,67), lengths -> logits (B,T,y_dim), or (B,y_dim) at the last valid step."""
+    def forward(self, x, lengths, return_last=False, hx=None):
+        """x (B,T,67,67), lengths -> logits (B,T,y_dim), or (B,y_dim) at the last valid step.
+
+        ``hx = (h0, c0)``, each (lstm_layers, B, H) as for nn.LSTM: the LSTM continues from that state and the call
+        returns ``(logits, (h_n, c_n))`` with the state at each row's last valid step; in a training step gradients
+        flow to h0 / c0 and from h_n / c_n.  Feeding h_n / c_n (detached) into the next block of the same utterances
+        trains it in blocks (truncated BPTT).  Blocks of one utterance are separate calls, so the quantities a call
+        computes over all its frames -- train()-mode BatchNorm statistics -- are per block: the caller decides
+        whether that is what it wants."""
+        if hx is not None and return_last:
+            raise ValueError("hx and return_last=True cannot be combined: with hx the call returns (logits, (h_n, c_n))")
         device = device_of(x)
         eng = self._build(device)
         batch, frames, height, width = x.size()
@@ -79,6 +88,9 @@ class DeepVAD_video(nn.Module):
                 bump_generation(b.running_mean, b.running_var)
         else:
             eng["trunk"].forward(vid, feat_bf16=xb.view(M, -1), col_off=0, want_f32=False)
+        if hx is not None:
+            return lstm_with_hx(eng["lstm"], xb, lengths, x_src, hx, lstm_params(self.lstm_video, self.vad_video),
+                                need_grad)
         if need_grad:
             return LstmHeadFunction.apply(eng["lstm"], xb, lengths, x_src, *lstm_params(self.lstm_video, self.vad_video))
         logits, _, _, last = eng["lstm"].forward(xb, lengths, want_last=return_last)

@@ -140,6 +140,60 @@ class LstmHeadFunction(torch.autograd.Function):
         return (None, None, None, g["dx"]) + tuple(grads)
 
 
+class LstmHeadStateFunction(torch.autograd.Function):
+    """LstmHeadFunction with nn.LSTM's ``hx``: ``h0`` (f32, rounded to bf16 for the kernel; its gradient is passed
+    straight through the rounding) and ``c0`` (f32), both (layers, B, H), are differentiable inputs, and the final
+    state ``h_n`` / ``c_n`` at each row's last valid step (f32) is a differentiable output next to the logits."""
+
+    @staticmethod
+    def forward(ctx, lstm_engine, x_bf16, lengths, x_src, h0, c0, *params):
+        logits, tape, (h_n, c_n) = E.lstm_train_forward(lstm_engine, x_bf16, lengths, state=(h0, c0))
+        ctx.lstm_engine = lstm_engine
+        ctx.tape = tape
+        ctx.want_dx = x_src is not None and x_src.requires_grad
+        ctx.want_state = h0.requires_grad or c0.requires_grad
+        return logits, h_n.float(), c_n
+
+    @staticmethod
+    def backward(ctx, dlogits, dh_n, dc_n):
+        eng = ctx.lstm_engine
+        g = E.lstm_train_backward(eng, ctx.tape, dlogits, want_dx=ctx.want_dx, d_state=(dh_n, dc_n),
+                                  want_state_grad=ctx.want_state)
+        ctx.tape = None
+        grads = []
+        for l in range(eng.layers):
+            grads += [g["weight_ih"][l], g["weight_hh"][l], g["bias"][l], g["bias"][l]]
+        grads += [g["head_w"], g["head_b"]]
+        return (None, None, None, g["dx"], g.get("dh_in"), g.get("dc_in")) + tuple(grads)
+
+
+def lstm_hx(hx, layers: int, B: int, H: int, device):
+    """Checks nn.LSTM's ``hx = (h0, c0)``, each (num_layers, B, H), and returns it as f32 tensors on ``device``."""
+    if not (isinstance(hx, (tuple, list)) and len(hx) == 2):
+        raise ValueError("hx must be a pair (h0, c0)")
+    h0, c0 = hx
+    shape = (layers, B, H)
+    if tuple(h0.shape) != shape or tuple(c0.shape) != shape:
+        raise ValueError(f"hx: expected h0, c0 of shape {shape}, got {tuple(h0.shape)}, {tuple(c0.shape)}")
+    return h0.to(device=device, dtype=torch.float32), c0.to(device=device, dtype=torch.float32)
+
+
+def lstm_with_hx(lstm_engine, x_bf16, lengths, x_src, hx, params, train: bool):
+    """(logits, (h_n, c_n)) of the LSTM + head continued from ``hx``: the autograd path when ``train``, else the
+    inference recurrence with a state (``Lstm.forward(state=)``).  h_n / c_n are f32 (num_layers, B, H), taken at each
+    row's last valid step as nn.LSTM returns them for packed input (``hx`` itself for rows of length 0)."""
+    B = x_bf16.shape[0]
+    h0, c0 = lstm_hx(hx, lstm_engine.layers, B, lstm_engine.hidden, x_bf16.device)
+    if train:
+        logits, h_n, c_n = LstmHeadStateFunction.apply(lstm_engine, x_bf16, lengths, x_src, h0, c0, *params)
+        return logits, (h_n, c_n)
+    state = E.LstmState(lstm_engine, B, x_bf16.device)
+    state.h.copy_(h0.detach())
+    state.c.copy_(c0.detach())
+    logits, _, _, _ = lstm_engine.forward(x_bf16, lengths, state=state)
+    return logits, (state.h.float(), state.c)
+
+
 class McbBnFunction(torch.autograd.Function):
     """Training-mode MCB fusion.  Fills the bf16 LSTM operand buffer (side effect) and returns a zero-storage fp32
     proxy of its shape through which the LSTM's input gradient reaches the BatchNorm1d affine parameters (the only

@@ -393,6 +393,29 @@ size_t avvad_lstm_backward_workspace_bytes(const avvad_lstm* h, int64_t B, int64
 int avvad_lstm_backward(avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T, void* tape,
                         const float* dlogits, void* workspace, size_t workspace_bytes, float* const* dW_ih,
                         float* const* dW_hh, float* const* db, float* dW_head, float* db_head, float* dx, void* stream);
+/* Training with a carried state (nn.LSTM's hx, truncated BPTT over blocks of a long sequence).  State shapes and the
+ * NULL / aliasing rules are those of avvad_lstm_forward_state: h bf16 and c f32, both [layers][B][H].
+ * The stateful tape holds T + 1 positions per row (tape_bytes >= avvad_lstm_tape_bytes(layers, H, B, T + 1); inspect it
+ * with avvad_lstm_tape_layout(layers, H, B, T + 1, ...)): position 0 holds the initial state -- h_in in hseq, c_in in
+ * c, zero gates -- and positions 1..lengths[b] the call's steps.
+ * workspace: avvad_lstm_train_state_workspace_bytes(h, B, T). */
+size_t avvad_lstm_train_state_workspace_bytes(const avvad_lstm* h, int64_t B, int64_t T);
+int avvad_lstm_forward_train_state(avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T,
+                                   const void* h_in, const float* c_in, void* h_out, float* c_out,
+                                   void* workspace, size_t workspace_bytes, void* tape, size_t tape_bytes,
+                                   float* logits, void* stream);
+/* BPTT over a stateful tape; x_bf16, lengths, B and T as given to avvad_lstm_forward_train_state, dlogits f32
+ * [B][T][y_dim], the gradients as in avvad_lstm_backward.  dh_out / dc_out f32 [layers][B][H] (NULL = zero): the
+ * gradient w.r.t. h_out / c_out, entering each row at its last step lengths[b] - 1.  dh_in / dc_in f32 [layers][B][H]
+ * (NULL = not wanted; the recurrent GEMM that produces them is then skipped): the gradient w.r.t. h_in / c_in.  A row
+ * of length 0 passes dh_out / dc_out through.  The outputs may alias dh_out / dc_out.
+ * workspace: avvad_lstm_backward_state_workspace_bytes(h, B, T). */
+size_t avvad_lstm_backward_state_workspace_bytes(const avvad_lstm* h, int64_t B, int64_t T);
+int avvad_lstm_backward_state(avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T,
+                              void* tape, const float* dlogits, const float* dh_out, const float* dc_out,
+                              float* dh_in, float* dc_in, void* workspace, size_t workspace_bytes,
+                              float* const* dW_ih, float* const* dW_hh, float* const* db,
+                              float* dW_head, float* db_head, float* dx, void* stream);
 /* torch.optim.Adam update (no weight decay, no amsgrad): step >= 1 is the 1-based update count. */
 int avvad_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n, float lr,
                     float beta1, float beta2, float eps, int64_t step, void* stream);
