@@ -18,6 +18,7 @@
 
 #include <vector>
 
+#include "lstm_internal.cuh"
 #include "lstm_persist.cuh"
 #include "lstm_pair.cuh"
 
@@ -96,8 +97,6 @@ __global__ void gather_last_kernel(const __nv_bfloat16* __restrict__ hseq, const
   for (int i = threadIdx.x; i < H / 8; i += blockDim.x) dst[i] = src[i];
 }
 
-// Streaming state (avvad_lstm_forward_state): the persistent recurrences run the call's steps at positions 1..T of a
-// [B][T+1][H] sequence whose position 0 holds h_in, so their masks see len_b + 1
 __global__ void shift_lengths_kernel(const int32_t* __restrict__ lengths, int B, int32_t* __restrict__ out) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b < B) out[b] = lengths[b] + 1;
@@ -133,33 +132,7 @@ __global__ void gather_state_kernel(const __nv_bfloat16* __restrict__ hseq, cons
 
 }  // namespace avvad
 
-namespace avvad {
-struct BpttGraphCache;
-struct BpttState;
-BpttGraphCache* bptt_cache_create();
-void bptt_cache_destroy(BpttGraphCache* c);
-}  // namespace avvad
-
 using namespace avvad;
-
-struct avvad_lstm {
-  int layers, input_size, H, y_dim;
-  int64_t ld0;               // padded layer-0 input width
-  __nv_bfloat16* w_ih[8];    // [4H][ld_l]
-  __nv_bfloat16* w_hh[8];    // [4H][H]
-  float* bias[8];            // [4H] gate-interleaved, b_ih + b_hh
-  float* head_w32;           // [y_dim][H]
-  __nv_bfloat16* head_w16;   // [y_dim][H]
-  float* head_b;             // [y_dim]
-  bool set[8];
-  bool head_set;
-  BpttGraphCache* bptt;      // cached CUDA graphs of the backward recurrence (lstm_train.cu)
-  // layer overlap (lstm_forward_impl): layer 1 follows layer 0 one chunk of time steps behind on a side stream
-  cudaStream_t side = nullptr;
-  int side_device = -1;
-  cudaEvent_t ev_chunk[32] = {};
-  cudaEvent_t ev_done = nullptr;
-};
 
 extern "C" int avvad_lstm_create(avvad_lstm** out, int layers, int input_size, int hidden, int y_dim) {
   AVVAD_CHECK_ARG(out, "null out");
@@ -246,30 +219,6 @@ namespace tc {
 int encode_tiled_bf16(CUtensorMap* m, const void* ptr, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
                       const uint32_t* box);
 }
-}  // namespace avvad
-
-namespace avvad {
-struct TapeView {
-  __nv_bfloat16* gates;
-  float* c;
-  __nv_bfloat16* hseq;
-};
-TapeView tape_layer(void* tape, int l, int H, int64_t B, int64_t T);
-int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim, __nv_bfloat16* const* w_ih,
-                       __nv_bfloat16* const* w_hh, const float* head_w32, const __nv_bfloat16* head_w16,
-                       const void* x_bf16, const int32_t* lengths,
-                       int64_t B, int64_t T, void* tape, const float* dlogits, void* workspace, size_t workspace_bytes,
-                       float* const* dW_ih, float* const* dW_hh, float* const* db, float* dW_head, float* db_head,
-                       float* dx, cudaStream_t st, BpttGraphCache* cache, const BpttState* bs);
-size_t lstm_backward_workspace(int layers, int input_size, int64_t ld0, int H, int y_dim, int64_t B, int64_t T);
-int lstm_backward_state_impl(int layers, int input_size, int64_t ld0, int H, int y_dim, __nv_bfloat16* const* w_ih,
-                             __nv_bfloat16* const* w_hh, const float* head_w32, const __nv_bfloat16* head_w16,
-                             const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T, void* tape,
-                             const float* dlogits, const float* dh_out, const float* dc_out, float* dh_in, float* dc_in,
-                             void* workspace, size_t workspace_bytes, float* const* dW_ih, float* const* dW_hh,
-                             float* const* db, float* dW_head, float* db_head, float* dx, cudaStream_t st,
-                             BpttGraphCache* cache);
-size_t lstm_backward_state_workspace(int layers, int input_size, int64_t ld0, int H, int y_dim, int64_t B, int64_t T);
 }  // namespace avvad
 
 namespace {
@@ -891,7 +840,7 @@ extern "C" int avvad_lstm_forward_train(avvad_lstm* h, const void* x_bf16, const
 
 extern "C" size_t avvad_lstm_backward_workspace_bytes(const avvad_lstm* h, int64_t B, int64_t T) {
   if (!h || B <= 0 || T <= 0) return 0;
-  return lstm_backward_workspace(h->layers, h->input_size, h->ld0, h->H, h->y_dim, B, T);
+  return lstm_backward_workspace(h, B, T);
 }
 
 // dlogits f32 [B][T][1] (e.g. from avvad_bce_loss).  Gradients in PyTorch layout, fp32: dW_ih[l] [4H][I_l],
@@ -903,10 +852,8 @@ extern "C" int avvad_lstm_backward(avvad_lstm* h, const void* x_bf16, const int3
                                    float* db_head, float* dx, void* stream) {
   AVVAD_CHECK_ARG(h && x_bf16 && lengths && tape && dlogits && workspace && dW_ih && dW_hh && db && dW_head && db_head,
                   "null pointer");
-  return lstm_backward_impl(h->layers, h->input_size, h->ld0, h->H, h->y_dim, h->w_ih, h->w_hh, h->head_w32,
-                            h->head_w16, x_bf16,
-                            lengths, B, T, tape, dlogits, workspace, workspace_bytes, dW_ih, dW_hh, db, dW_head, db_head,
-                            dx, (cudaStream_t)stream, h->bptt, nullptr);
+  return lstm_backward_impl(h, x_bf16, lengths, B, T, tape, dlogits, workspace, workspace_bytes, dW_ih, dW_hh, db,
+                            dW_head, db_head, dx, (cudaStream_t)stream, nullptr);
 }
 
 // ---- training with a carried state (truncated BPTT, nn.LSTM's hx).  The forward is avvad_lstm_forward_state's
@@ -932,7 +879,7 @@ extern "C" int avvad_lstm_forward_train_state(avvad_lstm* h, const void* x_bf16,
 
 extern "C" size_t avvad_lstm_backward_state_workspace_bytes(const avvad_lstm* h, int64_t B, int64_t T) {
   if (!h || B <= 0 || T <= 0) return 0;
-  return lstm_backward_state_workspace(h->layers, h->input_size, h->ld0, h->H, h->y_dim, B, T);
+  return lstm_backward_state_workspace(h, B, T);
 }
 
 extern "C" int avvad_lstm_backward_state(avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T,
@@ -942,8 +889,6 @@ extern "C" int avvad_lstm_backward_state(avvad_lstm* h, const void* x_bf16, cons
                                          float* db_head, float* dx, void* stream) {
   AVVAD_CHECK_ARG(h && x_bf16 && lengths && tape && dlogits && workspace && dW_ih && dW_hh && db && dW_head && db_head,
                   "null pointer");
-  return lstm_backward_state_impl(h->layers, h->input_size, h->ld0, h->H, h->y_dim, h->w_ih, h->w_hh, h->head_w32,
-                                  h->head_w16, x_bf16, lengths, B, T, tape, dlogits, dh_out, dc_out, dh_in, dc_in,
-                                  workspace, workspace_bytes, dW_ih, dW_hh, db, dW_head, db_head, dx,
-                                  (cudaStream_t)stream, h->bptt);
+  return lstm_backward_state_impl(h, x_bf16, lengths, B, T, tape, dlogits, dh_out, dc_out, dh_in, dc_in, workspace,
+                                  workspace_bytes, dW_ih, dW_hh, db, dW_head, db_head, dx, (cudaStream_t)stream);
 }

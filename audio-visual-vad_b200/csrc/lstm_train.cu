@@ -12,123 +12,20 @@
 //                             db = column sums of dG
 // Gradients are returned in PyTorch's layout (gate-major rows i,f,g,o), fp32.
 // With a carried state (avvad_lstm_backward_state) the same schedules run over a tape of T + 1 positions whose position 0
-// holds the initial state; see lstm_bwd_cell_state_kernel and lstm_backward_state_impl.
+// holds the initial state; see the kState instantiations of the cell kernels and lstm_backward_state_impl.
 #include <vector>
 
 #include "gemm_tma.cuh"
+#include "lstm_internal.cuh"
 
 namespace avvad {
 
 __device__ __forceinline__ float bf16lo(uint32_t u) { return __uint_as_float(u << 16); }
 __device__ __forceinline__ float bf16hi(uint32_t u) { return __uint_as_float(u & 0xFFFF0000u); }
 
-// one thread per (b, u)
-__global__ void lstm_bwd_cell_kernel(const __nv_bfloat16* __restrict__ gates, const float* __restrict__ cst,
-                                     const float* __restrict__ dY, const float* __restrict__ dl,
-                                     const float* __restrict__ w_head, const float* __restrict__ dh_rec,
-                                     float* __restrict__ dc, const int32_t* __restrict__ lengths, int B, int T, int H,
-                                     int t, int has_rec, __nv_bfloat16* __restrict__ dG) {
-  // dh_rec holds `has_rec` split-K partial products [has_rec][B][H] of the recurrent GEMM of step t+1
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= B * H) return;
-  const int b = idx / H, u = idx - b * H;
-  const int64_t row = (int64_t)b * T + t;
-  uint2* out = reinterpret_cast<uint2*>(dG + row * 4 * H + 4 * u);
-  if (t >= lengths[b]) {  // padded step: no gradient flows (packed-sequence semantics)
-    *out = make_uint2(0u, 0u);
-    dc[idx] = 0.f;
-    return;
-  }
-  const uint2 gp = *reinterpret_cast<const uint2*>(gates + row * 4 * H + 4 * u);
-  const float gi = bf16lo(gp.x), gf = bf16hi(gp.x), gg = bf16lo(gp.y), go = bf16hi(gp.y);
-  const float c = cst[row * H + u];
-  const float cp = t > 0 ? cst[(row - 1) * H + u] : 0.f;
-  float dh = dY ? dY[row * H + u] : dl[row] * w_head[u];
-  for (int sp = 0; sp < has_rec; ++sp) dh += dh_rec[(int64_t)sp * B * H + idx];
-  const float tc = tanhf(c);
-  const float d_o = dh * tc * go * (1.f - go);
-  const float dcc = dh * go * (1.f - tc * tc) + dc[idx];
-  const float d_i = dcc * gg * gi * (1.f - gi);
-  const float d_g = dcc * gi * (1.f - gg * gg);
-  const float d_f = dcc * cp * gf * (1.f - gf);
-  dc[idx] = dcc * gf;
-  uint2 o;
-  o.x = pack_bf16x2(d_i, d_f);
-  o.y = pack_bf16x2(d_g, d_o);
-  *out = o;
-}
-
-// ---- two-layer wavefront (small per-rank batches): layer 1 at step t1 = T-1-s and layer 0 at step t0 = T-s run in the
-// SAME launches, so the dependent chain is T+1 (cell, GEMM) pairs instead of 2T.  One GEMM per iteration does all three
-// products on a block-structured operand:
-//   A [2B][2*4H]:  rows 0..B-1   = [ dG1_t1 | 0 ],   rows B..2B-1 = [ 0 | dG0_t0 ]
-//   W [2H][2*4H]:  rows 0..H-1   = [ W_hh1^T | W_hh0^T ],   rows H..2H-1 = [ W_ih1^T | 0 ]
-//   C [2B][2H]  :  rows 0..B-1   = [ dh_rec1 | dY0_t1 ],    rows B..2B-1 = [ dh_rec0 | 0 ]
-// which the next iteration's cell launch consumes (layer 0 then sits at the step layer 1 just left).
-__global__ void lstm_bwd_cell_wf_kernel(const __nv_bfloat16* __restrict__ gates1, const float* __restrict__ cst1,
-                                        const __nv_bfloat16* __restrict__ gates0, const float* __restrict__ cst0,
-                                        const float* __restrict__ dY1, const float* __restrict__ dl,
-                                        const float* __restrict__ w_head, const float* __restrict__ Cpart, int nsplit,
-                                        float* __restrict__ dc2, const int32_t* __restrict__ lengths, int B, int T, int H,
-                                        int s, __nv_bfloat16* __restrict__ dG1, __nv_bfloat16* __restrict__ dG0,
-                                        __nv_bfloat16* __restrict__ Abuf) {
-  const int layer = 1 - (int)blockIdx.y;   // blockIdx.y 0 -> layer 1, 1 -> layer 0
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= B * H) return;
-  const int b = idx / H, u = idx - b * H;
-  const int t = (layer == 1) ? (T - 1 - s) : (T - s);
-  const int64_t K2 = 8ll * H;              // row length of Abuf (null: the GEMMs read dG1 / dG0 directly)
-  uint2* aout = Abuf ? reinterpret_cast<uint2*>(Abuf + (int64_t)(layer == 1 ? b : B + b) * K2 + (layer == 1 ? 0 : 4 * H) + 4 * u)
-                     : nullptr;
-  if (t < 0 || t > T - 1) {                // this layer is idle in iteration s: contribute nothing to the GEMM
-    if (aout) *aout = make_uint2(0u, 0u);
-    return;
-  }
-  const int64_t row = (int64_t)b * T + t;
-  __nv_bfloat16* dG = layer == 1 ? dG1 : dG0;
-  uint2* gout = reinterpret_cast<uint2*>(dG + row * 4 * H + 4 * u);
-  float* dc = dc2 + (int64_t)layer * B * H;
-  if (t >= lengths[b]) {
-    *gout = make_uint2(0u, 0u);
-    if (aout) *aout = make_uint2(0u, 0u);
-    dc[idx] = 0.f;
-    return;
-  }
-  const __nv_bfloat16* gates = layer == 1 ? gates1 : gates0;
-  const float* cst = layer == 1 ? cst1 : cst0;
-  const uint2 gp = *reinterpret_cast<const uint2*>(gates + row * 4 * H + 4 * u);
-  const float gi = bf16lo(gp.x), gf = bf16hi(gp.x), gg = bf16lo(gp.y), go = bf16hi(gp.y);
-  const float c = cst[row * H + u];
-  const float cp = t > 0 ? cst[(row - 1) * H + u] : 0.f;
-  const int64_t cstride = 2ll * B * 2 * H;  // one split-K partial of C
-  float dh;
-  if (layer == 1) {
-    dh = dY1 ? dY1[row * H + u] : dl[row] * w_head[u];
-    if (s > 0)
-      for (int sp = 0; sp < nsplit; ++sp) dh += Cpart[sp * cstride + (int64_t)b * 2 * H + u];
-  } else {
-    dh = 0.f;
-    for (int sp = 0; sp < nsplit; ++sp) {
-      dh += Cpart[sp * cstride + (int64_t)b * 2 * H + H + u];                      // dY0_t = dG1_t * W_ih1
-      if (t < T - 1) dh += Cpart[sp * cstride + (int64_t)(B + b) * 2 * H + u];      // recurrent term from step t+1
-    }
-  }
-  const float tc = tanhf(c);
-  const float d_o = dh * tc * go * (1.f - go);
-  const float dcc = dh * go * (1.f - tc * tc) + dc[idx];
-  const float d_i = dcc * gg * gi * (1.f - gi);
-  const float d_g = dcc * gi * (1.f - gg * gg);
-  const float d_f = dcc * cp * gf * (1.f - gf);
-  dc[idx] = dcc * gf;
-  uint2 o;
-  o.x = pack_bf16x2(d_i, d_f);
-  o.y = pack_bf16x2(d_g, d_o);
-  *gout = o;
-  if (aout) *aout = o;
-}
 // ---- stateful BPTT (avvad_lstm_backward_state).  The tape has T + 1 positions per row and lengths are shifted by one:
-// position 0 holds the initial state (h_in in hseq, c_in in c) and is frozen -- read, never differentiated.  The
-// stateless kernels above are left exactly as they were (their SASS is unchanged); these are their stateful twins.
+// position 0 holds the initial state (h_in in hseq, c_in in c) and is frozen -- read, never differentiated.  The cell
+// kernels below take it as their kState instantiation:
 //   * position t >= 1 reads cp = c[t-1], so the first step's forget-gate term uses c_in
 //   * at the last valid position len_b (shifted) - 1 the incoming state gradients dh_out / dc_out [B][H] are added
 //   * at position 0 nothing is written to dG but zeros; the state gradients leave as dh_in = the recurrent term of
@@ -140,6 +37,9 @@ struct BwdStateArgs {
   float* dh_in;         // null: no state gradient requested
   float* dc_in;
 };
+// One cell step backward: gate gradients (bf16, gate-interleaved) from dh and the cell-state gradient *dc, which is
+// read in place and replaced by its value for step t-1.  The stateless kernels pass dc in global memory, so that the
+// load stays where the arithmetic needs it.
 __device__ __forceinline__ uint2 lstm_cell_bwd(uint2 gp, float c, float cp, float dh, float* dc) {
   const float gi = bf16lo(gp.x), gf = bf16hi(gp.x), gg = bf16lo(gp.y), go = bf16hi(gp.y);
   const float tc = tanhf(c);
@@ -161,61 +61,78 @@ __device__ __forceinline__ void lstm_state_grad_out(const BwdStateArgs& sa, int 
   if (sa.dc_in) sa.dc_in[idx] = dc + (last ? sa.dc_out[idx] : 0.f);
 }
 
-__global__ void lstm_bwd_cell_state_kernel(const __nv_bfloat16* __restrict__ gates, const float* __restrict__ cst,
-                                           const float* __restrict__ dY, const float* __restrict__ dl,
-                                           const float* __restrict__ w_head, const float* __restrict__ dh_rec,
-                                           float* __restrict__ dc, const int32_t* __restrict__ lengths, int B, int T,
-                                           int H, int t, int has_rec, __nv_bfloat16* __restrict__ dG, BwdStateArgs sa) {
+// one thread per (b, u); `sa` is unused without kState
+template <bool kState>
+__global__ void lstm_bwd_cell_kernel(const __nv_bfloat16* __restrict__ gates, const float* __restrict__ cst,
+                                     const float* __restrict__ dY, const float* __restrict__ dl,
+                                     const float* __restrict__ w_head, const float* __restrict__ dh_rec,
+                                     float* __restrict__ dc, const int32_t* __restrict__ lengths, int B, int T, int H,
+                                     int t, int has_rec, __nv_bfloat16* __restrict__ dG, BwdStateArgs sa) {
+  // dh_rec holds `has_rec` split-K partial products [has_rec][B][H] of the recurrent GEMM of step t+1
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= B * H) return;
   const int b = idx / H, u = idx - b * H;
   const int64_t row = (int64_t)b * T + t;
   uint2* out = reinterpret_cast<uint2*>(dG + row * 4 * H + 4 * u);
   const int len = lengths[b];
-  if (t == 0) {  // frozen initial state
+  if (kState && t == 0) {  // frozen initial state
     float rec = 0.f;
     for (int sp = 0; sp < has_rec; ++sp) rec += dh_rec[(int64_t)sp * B * H + idx];
     lstm_state_grad_out(sa, idx, len == 1, rec, dc[idx]);
     *out = make_uint2(0u, 0u);
     return;
   }
-  if (t >= len) {
+  if (t >= len) {  // padded step: no gradient flows (packed-sequence semantics)
     *out = make_uint2(0u, 0u);
     dc[idx] = 0.f;
     return;
   }
   const uint2 gp = *reinterpret_cast<const uint2*>(gates + row * 4 * H + 4 * u);
   const float c = cst[row * H + u];
-  const float cp = cst[(row - 1) * H + u];
+  const float cp = (kState || t > 0) ? cst[(row - 1) * H + u] : 0.f;
   float dh = dY ? dY[row * H + u] : dl[row] * w_head[u];
   for (int sp = 0; sp < has_rec; ++sp) dh += dh_rec[(int64_t)sp * B * H + idx];
-  float dcv = dc[idx];
-  if (t == len - 1) {
-    dh += sa.dh_out[idx];
-    dcv += sa.dc_out[idx];
+  if constexpr (kState) {
+    float dcv = dc[idx];
+    if (t == len - 1) {
+      dh += sa.dh_out[idx];
+      dcv += sa.dc_out[idx];
+    }
+    *out = lstm_cell_bwd(gp, c, cp, dh, &dcv);
+    dc[idx] = dcv;
+  } else {
+    *out = lstm_cell_bwd(gp, c, cp, dh, dc + idx);
   }
-  *out = lstm_cell_bwd(gp, c, cp, dh, &dcv);
-  dc[idx] = dcv;
 }
 
-// Stateful twin of lstm_bwd_cell_wf_kernel (same schedule over T + 1 positions); sa0 / sa1: layer 0 / layer 1
-__global__ void lstm_bwd_cell_wf_state_kernel(const __nv_bfloat16* __restrict__ gates1, const float* __restrict__ cst1,
-                                              const __nv_bfloat16* __restrict__ gates0, const float* __restrict__ cst0,
-                                              const float* __restrict__ dY1, const float* __restrict__ dl,
-                                              const float* __restrict__ w_head, const float* __restrict__ Cpart,
-                                              int nsplit, float* __restrict__ dc2, const int32_t* __restrict__ lengths,
-                                              int B, int T, int H, int s, __nv_bfloat16* __restrict__ dG1,
-                                              __nv_bfloat16* __restrict__ dG0, __nv_bfloat16* __restrict__ Abuf,
-                                              BwdStateArgs sa1, BwdStateArgs sa0) {
-  const int layer = 1 - (int)blockIdx.y;
+// ---- two-layer wavefront (small per-rank batches): layer 1 at step t1 = T-1-s and layer 0 at step t0 = T-s run in the
+// SAME launches, so the dependent chain is T+1 (cell, GEMM) pairs instead of 2T.  One GEMM per iteration does all three
+// products on a block-structured operand:
+//   A [2B][2*4H]:  rows 0..B-1   = [ dG1_t1 | 0 ],   rows B..2B-1 = [ 0 | dG0_t0 ]
+//   W [2H][2*4H]:  rows 0..H-1   = [ W_hh1^T | W_hh0^T ],   rows H..2H-1 = [ W_ih1^T | 0 ]
+//   C [2B][2H]  :  rows 0..B-1   = [ dh_rec1 | dY0_t1 ],    rows B..2B-1 = [ dh_rec0 | 0 ]
+// which the next iteration's cell launch consumes (layer 0 then sits at the step layer 1 just left).  With kState it
+// runs over T + 1 positions; sa0 / sa1: layer 0 / layer 1.
+template <bool kState>
+__global__ void lstm_bwd_cell_wf_kernel(const __nv_bfloat16* __restrict__ gates1, const float* __restrict__ cst1,
+                                        const __nv_bfloat16* __restrict__ gates0, const float* __restrict__ cst0,
+                                        const float* __restrict__ dY1, const float* __restrict__ dl,
+                                        const float* __restrict__ w_head, const float* __restrict__ Cpart, int nsplit,
+                                        float* __restrict__ dc2, const int32_t* __restrict__ lengths, int B, int T, int H,
+                                        int s, __nv_bfloat16* __restrict__ dG1, __nv_bfloat16* __restrict__ dG0,
+                                        __nv_bfloat16* __restrict__ Abuf, BwdStateArgs sa1, BwdStateArgs sa0) {
+  const int layer = 1 - (int)blockIdx.y;   // blockIdx.y 0 -> layer 1, 1 -> layer 0
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= B * H) return;
   const int b = idx / H, u = idx - b * H;
   const int t = (layer == 1) ? (T - 1 - s) : (T - s);
-  const int64_t K2 = 8ll * H;
+  // Abuf is never null.  Its null tests and the two copies of cstride below keep the instructions of the kernels this
+  // template replaced: without the tests ptxas schedules the stateless instantiation differently, and forward +
+  // backward of 2 x LSTM-1024 at B = 32, T = 317 measured 8.97 -> 9.18 ms (one B200 at 1000 W).
+  const int64_t K2 = 8ll * H;              // row length of Abuf
   uint2* aout = Abuf ? reinterpret_cast<uint2*>(Abuf + (int64_t)(layer == 1 ? b : B + b) * K2 + (layer == 1 ? 0 : 4 * H) + 4 * u)
                      : nullptr;
-  if (t < 0 || t > T - 1) {
+  if (t < 0 || t > T - 1) {                // this layer is idle in iteration s: contribute nothing to the GEMM
     if (aout) *aout = make_uint2(0u, 0u);
     return;
   }
@@ -223,15 +140,15 @@ __global__ void lstm_bwd_cell_wf_state_kernel(const __nv_bfloat16* __restrict__ 
   __nv_bfloat16* dG = layer == 1 ? dG1 : dG0;
   uint2* gout = reinterpret_cast<uint2*>(dG + row * 4 * H + 4 * u);
   float* dc = dc2 + (int64_t)layer * B * H;
-  const int64_t cstride = 2ll * B * 2 * H;
+  const int64_t cstride0 = 2ll * B * 2 * H;  // one split-K partial of C
   const int len = lengths[b];
-  if (t == 0) {  // frozen initial state: the recurrent term of step 1 is dh_in
+  if (kState && t == 0) {  // frozen initial state: the recurrent term of step 1 is dh_in
     float rec = 0.f;
     if (layer == 1) {
       if (s > 0)
-        for (int sp = 0; sp < nsplit; ++sp) rec += Cpart[sp * cstride + (int64_t)b * 2 * H + u];
+        for (int sp = 0; sp < nsplit; ++sp) rec += Cpart[sp * cstride0 + (int64_t)b * 2 * H + u];
     } else if (T > 1) {
-      for (int sp = 0; sp < nsplit; ++sp) rec += Cpart[sp * cstride + (int64_t)(B + b) * 2 * H + u];
+      for (int sp = 0; sp < nsplit; ++sp) rec += Cpart[sp * cstride0 + (int64_t)(B + b) * 2 * H + u];
     }
     lstm_state_grad_out(layer == 1 ? sa1 : sa0, idx, len == 1, rec, dc[idx]);
     *gout = make_uint2(0u, 0u);
@@ -248,7 +165,8 @@ __global__ void lstm_bwd_cell_wf_state_kernel(const __nv_bfloat16* __restrict__ 
   const float* cst = layer == 1 ? cst1 : cst0;
   const uint2 gp = *reinterpret_cast<const uint2*>(gates + row * 4 * H + 4 * u);
   const float c = cst[row * H + u];
-  const float cp = cst[(row - 1) * H + u];
+  const float cp = (kState || t > 0) ? cst[(row - 1) * H + u] : 0.f;
+  const int64_t cstride = 2ll * B * 2 * H;
   float dh;
   if (layer == 1) {
     dh = dY1 ? dY1[row * H + u] : dl[row] * w_head[u];
@@ -257,18 +175,23 @@ __global__ void lstm_bwd_cell_wf_state_kernel(const __nv_bfloat16* __restrict__ 
   } else {
     dh = 0.f;
     for (int sp = 0; sp < nsplit; ++sp) {
-      dh += Cpart[sp * cstride + (int64_t)b * 2 * H + H + u];
-      if (t < T - 1) dh += Cpart[sp * cstride + (int64_t)(B + b) * 2 * H + u];
+      dh += Cpart[sp * cstride + (int64_t)b * 2 * H + H + u];                      // dY0_t = dG1_t * W_ih1
+      if (t < T - 1) dh += Cpart[sp * cstride + (int64_t)(B + b) * 2 * H + u];      // recurrent term from step t+1
     }
   }
-  float dcv = dc[idx];
-  if (t == len - 1) {
-    const BwdStateArgs& sa = layer == 1 ? sa1 : sa0;
-    dh += sa.dh_out[idx];
-    dcv += sa.dc_out[idx];
+  uint2 o;
+  if constexpr (kState) {
+    float dcv = dc[idx];
+    if (t == len - 1) {
+      const BwdStateArgs& sa = layer == 1 ? sa1 : sa0;
+      dh += sa.dh_out[idx];
+      dcv += sa.dc_out[idx];
+    }
+    o = lstm_cell_bwd(gp, c, cp, dh, &dcv);
+    dc[idx] = dcv;
+  } else {
+    o = lstm_cell_bwd(gp, c, cp, dh, dc + idx);
   }
-  const uint2 o = lstm_cell_bwd(gp, c, cp, dh, &dcv);
-  dc[idx] = dcv;
   *gout = o;
   if (aout) *aout = o;
 }
@@ -482,29 +405,25 @@ namespace avvad {
 // captured once into a CUDA graph and replayed while every pointer baked into its kernel parameters is unchanged (the
 // key below); the per-call inputs that PyTorch re-allocates (lengths, dlogits) are first copied into the caller's
 // workspace so that a steady-state training loop always hits the cache.  AVVAD_BPTT_GRAPH=0 disables it.
-constexpr int kBpttSlots = 40;      // graphs: per layer (0, 1), wavefront (2), per (layer, chunk) of the overlapped chains
-constexpr int kBpttMaxChunks = 16;
+constexpr int kBpttChunks = 8;  // chunks of layer 1's chain in the overlapped two-layer schedule (fewer for short T)
+// graphs: per layer (slot l, up to 8 layers), wavefront (2), per (layer, chunk) of the overlapped chains (3 + ...)
+constexpr int kBpttSlots = 3 + 2 * kBpttChunks;
 struct BpttGraphCache {
   cudaGraphExec_t exec[kBpttSlots] = {};
   std::vector<uintptr_t> key[kBpttSlots];
   size_t nodes[kBpttSlots] = {};
   // overlapped two-layer backward: layer 0's chain runs on `side`, one chunk of time steps behind layer 1
   cudaStream_t side = nullptr;
-  cudaEvent_t ev_chunk[kBpttMaxChunks] = {};
+  cudaEvent_t ev_chunk[kBpttChunks] = {};
   cudaEvent_t ev_side_done = nullptr;
   // Capture happens on a private stream: PyTorch's default current stream is the legacy NULL stream, which cannot be
   // captured; the instantiated graph is then launched into the caller's stream (any stream, the NULL stream included).
   cudaStream_t cap_stream = nullptr;
-  cudaStream_t cap_stream2 = nullptr;  // forked branch of the two-GEMM wavefront
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   int cap_device = -1;
   ~BpttGraphCache() {
     for (auto e : exec)
       if (e) cudaGraphExecDestroy(e);
     if (cap_stream) cudaStreamDestroy(cap_stream);
-    if (cap_stream2) cudaStreamDestroy(cap_stream2);
-    if (ev_fork) cudaEventDestroy(ev_fork);
-    if (ev_join) cudaEventDestroy(ev_join);
     if (side) cudaStreamDestroy(side);
     for (auto e : ev_chunk)
       if (e) cudaEventDestroy(e);
@@ -528,41 +447,30 @@ struct BpttState {
   }
 };
 
-// exposed to lstm.cu
-int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim, __nv_bfloat16* const* w_ih,
-                       __nv_bfloat16* const* w_hh, const float* head_w32, const __nv_bfloat16* head_w16,
-                       const void* x_bf16, const int32_t* lengths,
-                       int64_t B, int64_t T, void* tape, const float* dlogits, void* workspace, size_t workspace_bytes,
-                       float* const* dW_ih, float* const* dW_hh, float* const* db, float* dW_head, float* db_head,
-                       float* dx, cudaStream_t st, BpttGraphCache* cache, const BpttState* bs);
-// split-K factor of the per-step recurrent-gradient GEMMs (AVVAD_BPTT_SPLIT = 1..8, buffers are sized for 8)
+// split-K factor of the per-step recurrent-gradient GEMMs: 8 for per-rank batches up to 64 rows (one m-tile: 256 CTAs
+// instead of 128), 4 above (DESIGN.md §3 has the measurements); the partial-product buffers are sized for 8
 constexpr int kBpttSplitMax = 8;
-// Default: 8 for per-rank batches up to 64 rows (one m-tile: 256 CTAs instead of 128, backward 6.0 -> 5.4 ms at B = 32),
-// 4 above (B = 256: 16.7 ms with 4, 17.0 with 8, 19.7 with 2).
-static int bptt_split(int64_t B) {
-  static int v = [] {
-    const char* e = getenv("AVVAD_BPTT_SPLIT");
-    int x = e ? atoi(e) : 0;
-    return x < 0 ? 0 : (x > kBpttSplitMax ? kBpttSplitMax : x);
+static int bptt_split(int64_t B) { return B <= 64 ? 8 : 4; }
+
+// Two layers at per-rank batches 2B <= 128 run as a wavefront (layer 0 one step behind layer 1, both in one 128-row MMA
+// block per GEMM): T + 1 dependent iterations instead of 2T.  Measured (B200, T = 317, backward of 2 x LSTM-1024):
+// 7.9 -> 6.1 ms at B = 32 and 8.8 -> 7.3 ms at B = 64.  AVVAD_BPTT_WAVEFRONT=0 runs the layers one after the other.
+static bool bptt_wavefront(int layers, int64_t B) {
+  static const bool on = [] {
+    const char* e = getenv("AVVAD_BPTT_WAVEFRONT");
+    return !e || atoi(e) != 0;
   }();
-  return v ? v : (B <= 64 ? 8 : 4);
+  return on && layers == 2 && 2 * B <= 128;
 }
 
-// Two layers run as a wavefront (layer 0 one step behind layer 1): T + 1 dependent iterations instead of 2T.
-//   mode 1 (2B <= 128): one block-structured GEMM per iteration (both layers in one 128-row MMA block)
-//   mode 2 (larger batches): two GEMMs per iteration on forked streams of the captured graph
-// AVVAD_BPTT_WAVEFRONT=0 disables both, =1 (default) allows only mode 1, =2 both.  Measured (B200, T = 317, backward of
-// 2 x LSTM-1024): mode 1 7.9 -> 6.1 ms at B = 32 and 8.8 -> 7.3 ms at B = 64; mode 2 with the GEMMs in order 9.9 -> 9.5 ms
-// at B = 96, 11.9 -> 11.8 at B = 128 and 15.5 -> 19.0 ms at B = 256 (the merged cell kernel and the extra N = H columns
-// cost more than the shorter chain saves once a step fills the GPU), forked onto two captured streams 43.7 ms.
-static int bptt_wavefront(int layers, int64_t B) {
-  static int v = [] {
-    const char* e = getenv("AVVAD_BPTT_WAVEFRONT");
-    return e ? atoi(e) : 1;
+// Two layers at larger batches run as chunked chains on two streams (lstm_backward_impl); AVVAD_BPTT_CHUNKS=1 runs
+// them one after the other.
+static bool bptt_chains_enabled() {
+  static const bool on = [] {
+    const char* e = getenv("AVVAD_BPTT_CHUNKS");
+    return !e || atoi(e) > 1;
   }();
-  if (v == 0 || layers != 2) return 0;
-  if (2 * B <= 128) return 1;
-  return v >= 2 ? 2 : 0;
+  return on;
 }
 
 static bool bptt_graph_enabled() {
@@ -573,13 +481,6 @@ static bool bptt_graph_enabled() {
   return v != 0;
 }
 
-size_t lstm_backward_workspace(int layers, int input_size, int64_t ld0, int H, int y_dim, int64_t B, int64_t T);
-
-struct TapeView {
-  __nv_bfloat16* gates;
-  float* c;
-  __nv_bfloat16* hseq;
-};
 TapeView tape_layer(void* tape, int l, int H, int64_t B, int64_t T) {
   const TapeOffsets o = tape_offsets(l, H, B, T);
   uint8_t* p = (uint8_t*)tape;
@@ -592,41 +493,76 @@ TapeView tape_layer(void* tape, int l, int H, int64_t B, int64_t T) {
 
 static int64_t head_pad(int y_dim) { return ((int64_t)y_dim + 63) / 64 * 64; }
 
-size_t lstm_backward_workspace(int layers, int input_size, int64_t ld0, int H, int y_dim, int64_t B, int64_t T) {
-  (void)input_size;
+// The workspace of lstm_backward_impl, each buffer 256-byte aligned; with a null base only `total` is meaningful.
+struct BpttWs {
+  __nv_bfloat16* dG;       // [BT][4H] (layer 1's in the two-layer schedules)
+  __nv_bfloat16* dGT;      // dG^T [4H][BTp]
+  __nv_bfloat16* XT;       // X^T / H_prev^T [maxI][BTp]
+  float *dYa, *dYb;        // dY ping-pong [BT][maxI]
+  float* dh_rec;           // split-K partials of the recurrent term [kBpttSplitMax][B][H] (each 256-byte aligned)
+  float* dc;               // [B][H]
+  float* dWp;              // dW' (interleaved) [4H][maxI]
+  __nv_bfloat16* WT;       // W^T [maxI][4H]
+  float* partial;          // head / bias partial sums
+  int32_t* len_st;         // stable copies of lengths / dlogits (y_dim == 1), see BpttGraphCache
+  float* dl_st;
+  __nv_bfloat16 *dl16, *dlT, *WTh;  // y_dim > 1: dlogits bf16 [BT][yp], its transpose, W_head^T [H][yp]
+  __nv_bfloat16* dG0;               // two layers: layer 0's dG (both layers are live at once)
+  __nv_bfloat16 *Abuf, *Wcat;       // wavefront: A [128][8H], Wcat [2H][8H],
+  float *Cpart, *dc2;               //   C partials [kBpttSplitMax][128][2H], dc of both layers
+  float *dh_rec0, *dc0;             // chunked chains: layer 0's dh_rec partials and dc,
+  __nv_bfloat16 *WT0, *WTi;         //   W_hh0'^T and W_ih1'^T [H][4H]
+  size_t total;
+};
+static BpttWs carve_bptt(const avvad_lstm* h, int64_t B, int64_t T, void* base) {
+  BpttWs w{};
+  size_t off = 0;
+  auto take = [&](size_t bytes) {
+    void* p = base ? (uint8_t*)base + off : nullptr;
+    off += align_up(bytes, 256);
+    return p;
+  };
+  const int H = h->H;
   const int64_t BT = B * T, BTp = (BT + 63) / 64 * 64;
-  const int64_t maxI = ld0 > H ? ld0 : H;
-  size_t s = 0;
-  s += align_up((size_t)BT * 4 * H * 2, 256);          // dG
-  s += align_up((size_t)4 * H * BTp * 2, 256);         // dG^T
-  s += align_up((size_t)maxI * BTp * 2, 256);          // X^T / H_prev^T
-  s += 2 * align_up((size_t)BT * maxI * 4, 256);       // dY ping-pong (f32)
-  s += (kBpttSplitMax + 1) * align_up((size_t)B * H * 4, 256);  // dh_rec split-K partials, dc
-  s += align_up((size_t)4 * H * maxI * 4, 256);        // dW' (interleaved)
-  s += align_up((size_t)maxI * 4 * H * 2, 256);        // W^T (bf16)
-  s += align_up((size_t)1024 * (H + 1) * 4, 256);      // head partials
-  s += align_up((size_t)B * 4, 256) + align_up((size_t)BT * 4, 256);  // stable copies of lengths / dlogits (y_dim == 1)
-  if (bptt_wavefront(layers, B)) {
-    const int64_t rows = 2 * B > 128 ? 2 * B : 128;
-    s += align_up((size_t)BT * 4 * H * 2, 256);                        // second dG (both layers are live at once)
-    s += align_up((size_t)128 * 8 * H * 2, 256);                       // A [2B <= 128][8H] (mode 1)
-    s += align_up((size_t)2 * H * 8 * H * 2, 256);                     // Wcat [2H][8H]
-    s += align_up((size_t)kBpttSplitMax * rows * 2 * H * 4, 256);         // C partials [split][2B][2H]
-    s += align_up((size_t)2 * B * H * 4, 256);                         // dc of both layers
+  const int64_t maxI = h->ld0 > H ? h->ld0 : H;
+  const size_t bh = (size_t)B * H * 4;
+  w.dG = (__nv_bfloat16*)take((size_t)BT * 4 * H * 2);
+  w.dGT = (__nv_bfloat16*)take((size_t)4 * H * BTp * 2);
+  w.XT = (__nv_bfloat16*)take((size_t)maxI * BTp * 2);
+  w.dYa = (float*)take((size_t)BT * maxI * 4);
+  w.dYb = (float*)take((size_t)BT * maxI * 4);
+  w.dh_rec = (float*)take(kBpttSplitMax * align_up(bh, 256));
+  w.dc = (float*)take(bh);
+  w.dWp = (float*)take((size_t)4 * H * maxI * 4);
+  w.WT = (__nv_bfloat16*)take((size_t)maxI * 4 * H * 2);
+  w.partial = (float*)take((size_t)1024 * (H + 1) * 4);
+  w.len_st = (int32_t*)take((size_t)B * 4);
+  w.dl_st = (float*)take((size_t)BT * 4);
+  if (h->y_dim > 1) {
+    const int64_t yp = head_pad(h->y_dim);
+    w.dl16 = (__nv_bfloat16*)take((size_t)BT * yp * 2);
+    w.dlT = (__nv_bfloat16*)take((size_t)yp * BTp * 2);
+    w.WTh = (__nv_bfloat16*)take((size_t)H * yp * 2);
   }
-  if (layers == 2 && !bptt_wavefront(layers, B)) {     // overlapped chains (see lstm_backward_impl)
-    s += align_up((size_t)BT * 4 * H * 2, 256);                        // second dG
-    s += (kBpttSplitMax + 1) * align_up((size_t)B * H * 4, 256);       // layer 0's dh_rec partials, dc
-    s += 2 * align_up((size_t)H * 4 * H * 2, 256);                     // W_hh0'^T, W_ih1'^T
+  if (h->layers == 2) {
+    w.dG0 = (__nv_bfloat16*)take((size_t)BT * 4 * H * 2);
+    if (bptt_wavefront(h->layers, B)) {
+      w.Abuf = (__nv_bfloat16*)take((size_t)128 * 8 * H * 2);
+      w.Wcat = (__nv_bfloat16*)take((size_t)2 * H * 8 * H * 2);
+      w.Cpart = (float*)take((size_t)kBpttSplitMax * 128 * 2 * H * 4);
+      w.dc2 = (float*)take(2 * bh);
+    } else {  // also sized when the chains do not run (AVVAD_BPTT_CHUNKS=1, short T, profiling)
+      w.dh_rec0 = (float*)take(kBpttSplitMax * align_up(bh, 256));
+      w.dc0 = (float*)take(bh);
+      w.WT0 = (__nv_bfloat16*)take((size_t)H * 4 * H * 2);
+      w.WTi = (__nv_bfloat16*)take((size_t)H * 4 * H * 2);
+    }
   }
-  if (y_dim > 1) {
-    const int64_t yp = head_pad(y_dim);
-    s += align_up((size_t)BT * yp * 2, 256);           // dlogits bf16, padded columns
-    s += align_up((size_t)yp * BTp * 2, 256);          // its transpose
-    s += align_up((size_t)H * yp * 2, 256);            // W_head^T bf16 [H][yp]
-  }
-  return s + 1024;
+  w.total = off + 1024;
+  return w;
 }
+
+size_t lstm_backward_workspace(const avvad_lstm* h, int64_t B, int64_t T) { return carve_bptt(h, B, T, nullptr).total; }
 
 // Runs `steps(stream)` -- a long chain of tiny dependent launches -- either directly (cache == nullptr) or as a CUDA graph
 // captured once on the cache's private stream and replayed while `key` (every pointer / size baked into the kernel
@@ -636,15 +572,8 @@ static int bptt_cache_streams(BpttGraphCache* cache) {
   AVVAD_CUDA(cudaGetDevice(&dev));
   if (!cache->cap_stream || cache->cap_device != dev) {
     if (cache->cap_stream) cudaStreamDestroy(cache->cap_stream);
-    if (cache->cap_stream2) cudaStreamDestroy(cache->cap_stream2);
-    if (cache->ev_fork) cudaEventDestroy(cache->ev_fork);
-    if (cache->ev_join) cudaEventDestroy(cache->ev_join);
-    cache->cap_stream = cache->cap_stream2 = nullptr;
-    cache->ev_fork = cache->ev_join = nullptr;
+    cache->cap_stream = nullptr;
     AVVAD_CUDA(cudaStreamCreateWithFlags(&cache->cap_stream, cudaStreamNonBlocking));
-    AVVAD_CUDA(cudaStreamCreateWithFlags(&cache->cap_stream2, cudaStreamNonBlocking));
-    AVVAD_CUDA(cudaEventCreateWithFlags(&cache->ev_fork, cudaEventDisableTiming));
-    AVVAD_CUDA(cudaEventCreateWithFlags(&cache->ev_join, cudaEventDisableTiming));
     if (cache->side) cudaStreamDestroy(cache->side);
     cache->side = nullptr;
     AVVAD_CUDA(cudaStreamCreateWithFlags(&cache->side, cudaStreamNonBlocking));
@@ -707,40 +636,26 @@ static int run_captured(BpttGraphCache* cache, int slot, std::vector<uintptr_t> 
   return AVVAD_OK;
 }
 
-int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim, __nv_bfloat16* const* w_ih,
-                       __nv_bfloat16* const* w_hh, const float* head_w32, const __nv_bfloat16* head_w16,
-                       const void* x_bf16, const int32_t* lengths,
-                       int64_t B, int64_t T, void* tape, const float* dlogits, void* workspace, size_t workspace_bytes,
-                       float* const* dW_ih, float* const* dW_hh, float* const* db, float* dW_head, float* db_head,
-                       float* dx, cudaStream_t st, BpttGraphCache* cache, const BpttState* bs) {
+int lstm_backward_impl(const avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T, void* tape,
+                       const float* dlogits, void* workspace, size_t workspace_bytes, float* const* dW_ih,
+                       float* const* dW_hh, float* const* db, float* dW_head, float* db_head, float* dx, cudaStream_t st,
+                       const BpttState* bs) {
+  const int layers = h->layers, H = h->H, y_dim = h->y_dim;
   AVVAD_CHECK_ARG(y_dim >= 1, "bad y_dim");
-  AVVAD_CHECK_ARG(workspace_bytes >= lstm_backward_workspace(layers, input_size, ld0, H, y_dim, B, T),
-                  "workspace too small");
+  const BpttWs w = carve_bptt(h, B, T, workspace);
+  AVVAD_CHECK_ARG(workspace_bytes >= w.total, "workspace too small");
   const int64_t BT = B * T, BTp = (BT + 63) / 64 * 64;
-  const int64_t maxI = ld0 > H ? ld0 : H;
   const int H4 = 4 * H;
-  uint8_t* p = (uint8_t*)workspace;
-  auto take = [&](size_t bytes) { void* q = p; p += align_up(bytes, 256); return q; };
-  __nv_bfloat16* dG = (__nv_bfloat16*)take((size_t)BT * H4 * 2);
-  __nv_bfloat16* dGT = (__nv_bfloat16*)take((size_t)H4 * BTp * 2);
-  __nv_bfloat16* XT = (__nv_bfloat16*)take((size_t)maxI * BTp * 2);
-  float* dYa = (float*)take((size_t)BT * maxI * 4);
-  float* dYb = (float*)take((size_t)BT * maxI * 4);
-  float* dh_rec = (float*)take((size_t)kBpttSplitMax * align_up((size_t)B * H * 4, 256));
-  float* dc = (float*)take((size_t)B * H * 4);
-  float* dWp = (float*)take((size_t)H4 * maxI * 4);
-  __nv_bfloat16* WT = (__nv_bfloat16*)take((size_t)maxI * H4 * 2);
-  float* partial = (float*)take((size_t)1024 * (H + 1) * 4);
-  int32_t* len_st = (int32_t*)take((size_t)B * 4);
-  float* dl_st = (float*)take((size_t)BT * 4);
+  BpttGraphCache* cache = h->bptt;
   // stable-address copies of the per-call inputs the step kernels read (see BpttGraphCache)
-  AVVAD_CUDA(cudaMemcpyAsync(len_st, lengths, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
-  if (y_dim == 1) AVVAD_CUDA(cudaMemcpyAsync(dl_st, dlogits, (size_t)BT * 4, cudaMemcpyDeviceToDevice, st));
-  const float* dl_step = (y_dim == 1) ? dl_st : dlogits;
-  const bool use_graph = cache && bptt_graph_enabled() && !tc::profiling_on() && !sync_debug();
+  AVVAD_CUDA(cudaMemcpyAsync(w.len_st, lengths, (size_t)B * 4, cudaMemcpyDeviceToDevice, st));
+  if (y_dim == 1) AVVAD_CUDA(cudaMemcpyAsync(w.dl_st, dlogits, (size_t)BT * 4, cudaMemcpyDeviceToDevice, st));
+  const float* dl_step = (y_dim == 1) ? w.dl_st : dlogits;
+  const bool use_graph = bptt_graph_enabled() && !tc::profiling_on() && !sync_debug();
   const int kBpttSplit = bptt_split(B);  // split-K factor of the per-step GEMMs of this call
   // stateful: the last position visited (0 when state gradients leave through the frozen position 0, else 1)
   const int t_min = (bs && !bs->dh_in) ? 1 : 0;
+  const auto state_args = [&](int l) { return bs ? bs->layer(l, B, H) : BwdStateArgs{}; };
   // stateful: position 0 of dG is never differentiated; zero it once so the weight-gradient GEMMs see zero rows even
   // where the recurrence stops at position 1
   auto zero_pos0 = [&](__nv_bfloat16* dGl) -> int {
@@ -762,9 +677,9 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
     int nblocks = (int)std::min<int64_t>(1024, ceil_div(BT, 64));
     int rows_per_block = (int)ceil_div(BT, nblocks);
     nblocks = (int)ceil_div(BT, rows_per_block);
-    head_grad_partial_kernel<<<nblocks, 256, 0, st>>>(dlogits, top.hseq, BT, H, rows_per_block, partial);
+    head_grad_partial_kernel<<<nblocks, 256, 0, st>>>(dlogits, top.hseq, BT, H, rows_per_block, w.partial);
     AVVAD_LAUNCHED();
-    head_grad_final_kernel<<<(unsigned)ceil_div(H + 1, 256), 256, 0, st>>>(partial, nblocks, H, dW_head, db_head);
+    head_grad_final_kernel<<<(unsigned)ceil_div(H + 1, 256), 256, 0, st>>>(w.partial, nblocks, H, dW_head, db_head);
     AVVAD_LAUNCHED();
   } else {
     // ---- head gradients (IBM head, y_dim = 513): three GEMMs on bf16 copies of dlogits
@@ -772,35 +687,32 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
     //   dW_head [y][H]   = dL^T [yp][BT] * h_top [BT][H]
     //   db_head [y]      = column sums of dL (fp32)
     const int64_t yp = head_pad(y_dim);
-    __nv_bfloat16* dl16 = (__nv_bfloat16*)take((size_t)BT * yp * 2);
-    __nv_bfloat16* dlT = (__nv_bfloat16*)take((size_t)yp * BTp * 2);
-    __nv_bfloat16* WTh = (__nv_bfloat16*)take((size_t)H * yp * 2);
     TapeView top = tape_layer(tape, layers - 1, H, B, T);
-    int rc = avvad_pack_rows_bf16(dlogits, y_dim, dl16, yp, 0, BT, y_dim, 1, st);
+    int rc = avvad_pack_rows_bf16(dlogits, y_dim, w.dl16, yp, 0, BT, y_dim, 1, st);
     if (rc) return rc;
-    head_wt_kernel<<<(unsigned)ceil_div((int64_t)H * yp, 256), 256, 0, st>>>(head_w16, y_dim, H, (int)yp, WTh);
+    head_wt_kernel<<<(unsigned)ceil_div((int64_t)H * yp, 256), 256, 0, st>>>(h->head_w16, y_dim, H, (int)yp, w.WTh);
     AVVAD_LAUNCHED();
     {
       tc::EpiParams ep{};
-      ep.C = dYa;
+      ep.C = w.dYa;
       ep.ldc = H;
-      rc = tc::gemm_dispatch(dl16, yp, WTh, yp, BT, H, (int)yp, ep, tc::EPI_F32, 0, st);
+      rc = tc::gemm_dispatch(w.dl16, yp, w.WTh, yp, BT, H, (int)yp, ep, tc::EPI_F32, 0, st);
       if (rc) return rc;
-      dY_head = dYa;
+      dY_head = w.dYa;
     }
     {
       dim3 grid((unsigned)ceil_div(BTp, 32), (unsigned)ceil_div(yp, 32));
-      transpose_bf16_kernel<<<grid, dim3(32, 8), 0, st>>>(dl16, BT, (int)yp, yp, BTp, 0, (int)T, dlT);
+      transpose_bf16_kernel<<<grid, dim3(32, 8), 0, st>>>(w.dl16, BT, (int)yp, yp, BTp, 0, (int)T, w.dlT);
       AVVAD_LAUNCHED();
       dim3 grid2((unsigned)ceil_div(BTp, 32), (unsigned)ceil_div(H, 32));
-      transpose_bf16_kernel<<<grid2, dim3(32, 8), 0, st>>>(top.hseq, BT, H, H, BTp, 0, (int)T, XT);
+      transpose_bf16_kernel<<<grid2, dim3(32, 8), 0, st>>>(top.hseq, BT, H, H, BTp, 0, (int)T, w.XT);
       AVVAD_LAUNCHED();
       tc::EpiParams ep{};
-      ep.C = dWp;
+      ep.C = w.dWp;
       ep.ldc = H;
-      rc = tc::gemm_dispatch(dlT, BTp, XT, BTp, yp, H, (int)BTp, ep, tc::EPI_F32, 0, st);
+      rc = tc::gemm_dispatch(w.dlT, BTp, w.XT, BTp, yp, H, (int)BTp, ep, tc::EPI_F32, 0, st);
       if (rc) return rc;
-      AVVAD_CUDA(cudaMemcpyAsync(dW_head, dWp, (size_t)y_dim * H * sizeof(float), cudaMemcpyDeviceToDevice, st));
+      AVVAD_CUDA(cudaMemcpyAsync(dW_head, w.dWp, (size_t)y_dim * H * sizeof(float), cudaMemcpyDeviceToDevice, st));
     }
     colsum_f32_kernel<<<(unsigned)ceil_div(y_dim, 64), 256, 0, st>>>(dlogits, BT, y_dim, db_head);
     AVVAD_LAUNCHED();
@@ -809,233 +721,159 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
   // ---- parameter gradients of layer l from its complete gate gradients dGl [BT][4H]; optionally dX = dGl * W_ih'
   auto weight_grads = [&](int l, const __nv_bfloat16* dGl, float* dx_dst) -> int {
     TapeView tv = tape_layer(tape, l, H, B, T);
-    const int64_t ld_in = (l == 0) ? ld0 : H;
-    const int I = (l == 0) ? input_size : H;
+    const int64_t ld_in = (l == 0) ? h->ld0 : H;
+    const int I = (l == 0) ? h->input_size : H;
     const __nv_bfloat16* Xin = (l == 0) ? (const __nv_bfloat16*)x_bf16 : tape_layer(tape, l - 1, H, B, T).hseq;
     // db (= db_ih = db_hh)
-    bias_grad_partial_kernel<<<dim3(H4 / 256, kBiasChunks), 256, 0, st>>>(dGl, BT, H4, dWp);  // dWp is free here
+    bias_grad_partial_kernel<<<dim3(H4 / 256, kBiasChunks), 256, 0, st>>>(dGl, BT, H4, w.dWp);  // dWp is free here
     AVVAD_LAUNCHED();
-    bias_grad_final_kernel<<<(unsigned)ceil_div(H4, 256), 256, 0, st>>>(dWp, H, db[l]);
+    bias_grad_final_kernel<<<(unsigned)ceil_div(H4, 256), 256, 0, st>>>(w.dWp, H, db[l]);
     AVVAD_LAUNCHED();
     // dG^T [4H][BTp]
     {
       dim3 grid((unsigned)ceil_div(BTp, 32), (unsigned)ceil_div(H4, 32));
-      transpose_bf16_kernel<<<grid, dim3(32, 8), 0, st>>>(dGl, BT, H4, H4, BTp, 0, (int)T, dGT);
+      transpose_bf16_kernel<<<grid, dim3(32, 8), 0, st>>>(dGl, BT, H4, H4, BTp, 0, (int)T, w.dGT);
       AVVAD_LAUNCHED();
     }
     // dW_ih' = dG^T * X  -> [4H][ld_in]
     {
       dim3 grid((unsigned)ceil_div(BTp, 32), (unsigned)ceil_div(ld_in, 32));
-      transpose_bf16_kernel<<<grid, dim3(32, 8), 0, st>>>(Xin, BT, (int)ld_in, ld_in, BTp, 0, (int)T, XT);
+      transpose_bf16_kernel<<<grid, dim3(32, 8), 0, st>>>(Xin, BT, (int)ld_in, ld_in, BTp, 0, (int)T, w.XT);
       AVVAD_LAUNCHED();
       tc::EpiParams ep{};
-      ep.C = dWp;
+      ep.C = w.dWp;
       ep.ldc = ld_in;
-      int rc = tc::gemm_dispatch(dGT, BTp, XT, BTp, H4, (int)ld_in, (int)BTp, ep, tc::EPI_F32, 0, st);
+      int rc = tc::gemm_dispatch(w.dGT, BTp, w.XT, BTp, H4, (int)ld_in, (int)BTp, ep, tc::EPI_F32, 0, st);
       if (rc) return rc;
-      deinterleave_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * I, 256), 256, 0, st>>>(dWp, H, I, (int)ld_in, dW_ih[l]);
+      deinterleave_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * I, 256), 256, 0, st>>>(w.dWp, H, I, (int)ld_in, dW_ih[l]);
       AVVAD_LAUNCHED();
     }
     // dW_hh' = dG^T * H_prev -> [4H][H]
     {
       dim3 grid((unsigned)ceil_div(BTp, 32), (unsigned)ceil_div(H, 32));
-      transpose_bf16_kernel<<<grid, dim3(32, 8), 0, st>>>(tv.hseq, BT, H, H, BTp, 1, (int)T, XT);
+      transpose_bf16_kernel<<<grid, dim3(32, 8), 0, st>>>(tv.hseq, BT, H, H, BTp, 1, (int)T, w.XT);
       AVVAD_LAUNCHED();
       tc::EpiParams ep{};
-      ep.C = dWp;
+      ep.C = w.dWp;
       ep.ldc = H;
-      int rc = tc::gemm_dispatch(dGT, BTp, XT, BTp, H4, H, (int)BTp, ep, tc::EPI_F32, 0, st);
+      int rc = tc::gemm_dispatch(w.dGT, BTp, w.XT, BTp, H4, H, (int)BTp, ep, tc::EPI_F32, 0, st);
       if (rc) return rc;
-      deinterleave_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * H, 256), 256, 0, st>>>(dWp, H, H, H, dW_hh[l]);
+      deinterleave_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * H, 256), 256, 0, st>>>(w.dWp, H, H, H, dW_hh[l]);
       AVVAD_LAUNCHED();
     }
     if (dx_dst) {
-      transpose_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * ld_in, 256), 256, 0, st>>>(w_ih[l], H4, (int)ld_in,
-                                                                                       (int)ld_in, WT);
+      transpose_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * ld_in, 256), 256, 0, st>>>(h->w_ih[l], H4, (int)ld_in,
+                                                                                       (int)ld_in, w.WT);
       AVVAD_LAUNCHED();
       tc::EpiParams ep{};
       ep.C = dx_dst;
       ep.ldc = (l == 0) ? I : ld_in;
       // l == 0: only the first I (un-padded) columns are written (N guard in the epilogue)
-      int rc = tc::gemm_dispatch(dGl, H4, WT, H4, BT, (l == 0) ? I : (int)ld_in, H4, ep, tc::EPI_F32, 0, st);
+      int rc = tc::gemm_dispatch(dGl, H4, w.WT, H4, BT, (l == 0) ? I : (int)ld_in, H4, ep, tc::EPI_F32, 0, st);
       if (rc) return rc;
     }
     return AVVAD_OK;
   };
 
-  const int wf_mode = bptt_wavefront(layers, B);
-  if (wf_mode) {
+  // ---- the recurrent-gradient GEMM of one step: split-K partials dh [kBpttSplit][B][H] of dG_t [B][4H] (rows T * 4H
+  // apart) times W_l'.  M = B is tiny: K = 4H is split over kBpttSplit CTAs per output tile so that a step fills the GPU.
+  auto step_gemm = [&](float* dh, const __nv_bfloat16* dGt, const __nv_bfloat16* WTl, cudaStream_t s) -> int {
+    tc::EpiParams ep{};
+    ep.C = dh;
+    ep.ldc = H;
+    return tc::launch_tma_gemm(dGt, (int64_t)T * H4, WTl, H4, B, H, H4, ep, tc::EPI_F32, 64, s, kBpttSplit,
+                               (int64_t)B * H);
+  };
+  // one real launch of the step GEMM before any capture: the kernels' one-time attribute setup is not capturable
+  auto warm = [&]() -> int { return step_gemm(w.dh_rec, w.dG, w.WT, st); };
+  // steps te-1 .. tb of layer l, not below t_min: (cell, recurrent GEMM) pairs on stream s
+  auto steps = [&](int l, const TapeView& tv, const float* dYl, float* dh, float* dcl, __nv_bfloat16* dGl,
+                   const __nv_bfloat16* WTl, int tb, int te, cudaStream_t s) -> int {
+    const auto cell = bs ? &lstm_bwd_cell_kernel<true> : &lstm_bwd_cell_kernel<false>;
+    const BwdStateArgs sa = state_args(l);
+    for (int t = te - 1; t >= tb && t >= t_min; --t) {
+      const int has_rec = (t < (int)T - 1) ? kBpttSplit : 0;  // number of partial products to sum
+      cell<<<(unsigned)ceil_div(B * H, 256), 256, 0, s>>>(tv.gates, tv.c, dYl, dl_step, h->head_w32, dh, dcl, w.len_st,
+                                                          (int)B, (int)T, H, t, has_rec, dGl, sa);
+      AVVAD_LAUNCHED();
+      if (t > t_min) {
+        int rc = step_gemm(dh, dGl + (int64_t)t * H4, WTl, s);
+        if (rc) return rc;
+      }
+    }
+    return AVVAD_OK;
+  };
+
+  if (bptt_wavefront(layers, B)) {
     // ---- both layers as one wavefront: T + 1 dependent iterations instead of 2T (see lstm_bwd_cell_wf_kernel)
-    const int64_t rows = 2 * B > 128 ? 2 * B : 128;
-    __nv_bfloat16* dG0 = (__nv_bfloat16*)take((size_t)BT * H4 * 2);
-    __nv_bfloat16* Abuf = (__nv_bfloat16*)take((size_t)128 * 8 * H * 2);
-    __nv_bfloat16* Wcat = (__nv_bfloat16*)take((size_t)2 * H * 8 * H * 2);
-    float* Cpart = (float*)take((size_t)kBpttSplitMax * rows * 2 * H * 4);
-    float* dc2 = (float*)take((size_t)2 * B * H * 4);
     TapeView t1 = tape_layer(tape, 1, H, B, T), t0 = tape_layer(tape, 0, H, B, T);
-    lstm_wf_pack_w_kernel<<<(unsigned)ceil_div((int64_t)2 * H * 8 * H, 256), 256, 0, st>>>(w_hh[1], w_ih[1], w_hh[0], H,
-                                                                                          Wcat);
+    lstm_wf_pack_w_kernel<<<(unsigned)ceil_div((int64_t)2 * H * 8 * H, 256), 256, 0, st>>>(h->w_hh[1], h->w_ih[1],
+                                                                                          h->w_hh[0], H, w.Wcat);
     AVVAD_LAUNCHED();
-    AVVAD_CUDA(cudaMemsetAsync(dc2, 0, (size_t)2 * B * H * 4, st));
-    if (int rcz = zero_pos0(dG)) return rcz;
-    if (int rcz = zero_pos0(dG0)) return rcz;
-    if (wf_mode == 1) AVVAD_CUDA(cudaMemsetAsync(Abuf, 0, (size_t)128 * 8 * H * 2, st));  // rows 2B..127 stay zero
-    const int64_t cstride = 2 * B * 2 * H;
-    // mode 1: C [2B][2H] = A [2B][8H] * Wcat^T
-    auto wf_gemm = [&](cudaStream_t s2) -> int {
+    AVVAD_CUDA(cudaMemsetAsync(w.dc2, 0, (size_t)2 * B * H * 4, st));
+    if (int rcz = zero_pos0(w.dG)) return rcz;
+    if (int rcz = zero_pos0(w.dG0)) return rcz;
+    AVVAD_CUDA(cudaMemsetAsync(w.Abuf, 0, (size_t)128 * 8 * H * 2, st));  // rows 2B..127 stay zero
+    // C [2B][2H] = A [2B][8H] * Wcat^T
+    auto wf_gemm = [&](cudaStream_t s) -> int {
       tc::EpiParams ep{};
-      ep.C = Cpart;
+      ep.C = w.Cpart;
       ep.ldc = 2 * H;
-      return tc::launch_tma_gemm(Abuf, 8 * H, Wcat, 8 * H, 2 * B, 2 * H, 8 * H, ep, tc::EPI_F32, 64, s2, kBpttSplit,
-                                 cstride);
+      return tc::launch_tma_gemm(w.Abuf, 8 * H, w.Wcat, 8 * H, 2 * B, 2 * H, 8 * H, ep, tc::EPI_F32, 64, s, kBpttSplit,
+                                 2 * B * 2 * H);
     };
-    // mode 2: rows 0..B-1 = dG1_t [B][4H] * [W_hh1^T | W_ih1^T] (N = 2H); rows B..2B-1 = dG0_t * W_hh0^T (N = H); both
-    // read the first / second 4H columns of Wcat's rows
-    auto gemm_l1 = [&](int t, cudaStream_t s2) -> int {
-      tc::EpiParams ep{};
-      ep.C = Cpart;
-      ep.ldc = 2 * H;
-      return tc::launch_tma_gemm(dG + (int64_t)t * H4, (int64_t)T * H4, Wcat, 8 * H, B, 2 * H, H4, ep, tc::EPI_F32, 64, s2,
-                                 kBpttSplit, cstride);
-    };
-    auto gemm_l0 = [&](int t, cudaStream_t s2) -> int {
-      tc::EpiParams ep{};
-      ep.C = Cpart + B * 2 * H;
-      ep.ldc = 2 * H;
-      return tc::launch_tma_gemm(dG0 + (int64_t)t * H4, (int64_t)T * H4, Wcat + H4, 8 * H, B, H, H4, ep, tc::EPI_F32, 64, s2,
-                                 kBpttSplit, cstride);
-    };
+    const auto cell = bs ? &lstm_bwd_cell_wf_kernel<true> : &lstm_bwd_cell_wf_kernel<false>;
+    const BwdStateArgs sa1 = state_args(1), sa0 = state_args(0);
     auto run_wf = [&](cudaStream_t s1) -> int {
-      // Forking the layer-0 GEMM onto a second captured stream was measured 3-4x SLOWER than issuing both GEMMs in order
-      // (B = 256: 43.7 ms against 15.5 ms for the layer-by-layer loop): AVVAD_BPTT_FORK=1 keeps the experiment reachable.
-      static int fork_pref = [] {
-        const char* e = getenv("AVVAD_BPTT_FORK");
-        return e ? atoi(e) : 0;
-      }();
-      cudaStream_t s2 = (use_graph && wf_mode == 2 && fork_pref) ? cache->cap_stream2 : nullptr;
+      // stateful: layer 0 reaches position 1 in iteration T - 1 and the frozen position 0 in iteration T
       for (int s = 0; s <= (int)T; ++s) {
-        if (bs)  // layer 0 reaches position 1 in iteration T - 1 and the frozen position 0 in iteration T
-          lstm_bwd_cell_wf_state_kernel<<<dim3((unsigned)ceil_div(B * H, 256), 2), 256, 0, s1>>>(
-              t1.gates, t1.c, t0.gates, t0.c, dY_head, dl_step, head_w32, Cpart, kBpttSplit, dc2, len_st, (int)B, (int)T,
-              H, s, dG, dG0, wf_mode == 1 ? Abuf : nullptr, bs->layer(1, B, H), bs->layer(0, B, H));
-        else
-          lstm_bwd_cell_wf_kernel<<<dim3((unsigned)ceil_div(B * H, 256), 2), 256, 0, s1>>>(
-              t1.gates, t1.c, t0.gates, t0.c, dY_head, dl_step, head_w32, Cpart, kBpttSplit, dc2, len_st, (int)B, (int)T,
-              H, s, dG, dG0, wf_mode == 1 ? Abuf : nullptr);
+        cell<<<dim3((unsigned)ceil_div(B * H, 256), 2), 256, 0, s1>>>(
+            t1.gates, t1.c, t0.gates, t0.c, dY_head, dl_step, h->head_w32, w.Cpart, kBpttSplit, w.dc2, w.len_st, (int)B,
+            (int)T, H, s, w.dG, w.dG0, w.Abuf, sa1, sa0);
         AVVAD_LAUNCHED();
         if (s >= (int)T - t_min) break;
-        if (wf_mode == 1) {
-          int rc = wf_gemm(s1);
-          if (rc) return rc;
-          continue;
-        }
-        const int tl1 = (int)T - 1 - s, tl0 = (int)T - s;   // the steps the layers just finished
-        const bool need0 = s >= 1 && tl0 > 0;               // layer 0's recurrent term for step tl0 - 1
-        if (need0 && s2) {
-          AVVAD_CUDA(cudaEventRecord(cache->ev_fork, s1));
-          AVVAD_CUDA(cudaStreamWaitEvent(s2, cache->ev_fork, 0));
-          int rc = gemm_l0(tl0, s2);
-          if (rc) return rc;
-          AVVAD_CUDA(cudaEventRecord(cache->ev_join, s2));
-        }
-        int rc = gemm_l1(tl1, s1);
+        int rc = wf_gemm(s1);
         if (rc) return rc;
-        if (need0) {
-          if (s2) AVVAD_CUDA(cudaStreamWaitEvent(s1, cache->ev_join, 0));
-          else {
-            rc = gemm_l0(tl0, s1);
-            if (rc) return rc;
-          }
-        }
       }
       return AVVAD_OK;
     };
-    std::vector<uintptr_t> key = {(uintptr_t)t1.gates, (uintptr_t)t1.c, (uintptr_t)t0.gates, (uintptr_t)t0.c,
-                                        (uintptr_t)dY_head, (uintptr_t)dl_step, (uintptr_t)head_w32, (uintptr_t)Cpart,
-                                        (uintptr_t)dc2, (uintptr_t)len_st, (uintptr_t)dG, (uintptr_t)dG0,
-                                        (uintptr_t)Abuf, (uintptr_t)Wcat, (uintptr_t)B, (uintptr_t)T, (uintptr_t)H,
-                                        (uintptr_t)wf_mode};
-    key = state_key(key);
-    auto warm = [&]() -> int {
-      if (wf_mode == 1) return wf_gemm(st);
-      int rc = gemm_l1(0, st);
-      return rc ? rc : gemm_l0(0, st);
-    };
-    int rc = run_captured(use_graph ? cache : nullptr, 2, key, warm, run_wf, st);
+    const std::vector<uintptr_t> key = state_key(
+        {(uintptr_t)t1.gates, (uintptr_t)t1.c, (uintptr_t)t0.gates, (uintptr_t)t0.c, (uintptr_t)dY_head,
+         (uintptr_t)dl_step, (uintptr_t)h->head_w32, (uintptr_t)w.Cpart, (uintptr_t)w.dc2, (uintptr_t)w.len_st,
+         (uintptr_t)w.dG, (uintptr_t)w.dG0, (uintptr_t)w.Abuf, (uintptr_t)w.Wcat, (uintptr_t)B, (uintptr_t)T,
+         (uintptr_t)H});
+    int rc = run_captured(use_graph ? cache : nullptr, 2, key, [&]() { return wf_gemm(st); }, run_wf, st);
     if (rc) return rc;
-    rc = weight_grads(1, dG, nullptr);
+    rc = weight_grads(1, w.dG, nullptr);
     if (rc) return rc;
-    return weight_grads(0, dG0, dx);
+    return weight_grads(0, w.dG0, dx);
   }
 
   // ---- two layers, larger batches: the recurrences of both layers as chunked chains on two streams.  Layer 1 runs its
   // steps in chunks (t descending); after each chunk the input gradient of that chunk (dY0 = dG1 * W_ih1, one time-major
   // GEMM) and then layer 0's steps of the same chunk run on a side stream while layer 1 continues: every step is a
-  // latency-bound (cell kernel, split-K GEMM) pair, so the two chains overlap.  AVVAD_BPTT_CHUNKS=1 disables it.
-  static int chunks_pref = [] {
-    const char* e = getenv("AVVAD_BPTT_CHUNKS");
-    int v = e ? atoi(e) : 8;
-    return v < 1 ? 1 : (v > kBpttMaxChunks ? kBpttMaxChunks : v);
-  }();
-  int n_chunks = chunks_pref;
+  // latency-bound (cell kernel, split-K GEMM) pair, so the two chains overlap.
+  int n_chunks = bptt_chains_enabled() ? kBpttChunks : 1;
   while (n_chunks > 1 && T / n_chunks < 16) --n_chunks;
-  if (layers == 2 && n_chunks > 1 && cache && !tc::profiling_on() && !sync_debug()) {
+  if (layers == 2 && n_chunks > 1 && !tc::profiling_on() && !sync_debug()) {
     int rcs = bptt_cache_streams(cache);
     if (rcs) return rcs;
-    __nv_bfloat16* dG0 = (__nv_bfloat16*)take((size_t)BT * H4 * 2);
-    float* dh_rec0 = (float*)take((size_t)kBpttSplitMax * align_up((size_t)B * H * 4, 256));
-    float* dc0 = (float*)take((size_t)B * H * 4);
-    __nv_bfloat16* WT0 = (__nv_bfloat16*)take((size_t)H * H4 * 2);
-    __nv_bfloat16* WTi = (__nv_bfloat16*)take((size_t)H * H4 * 2);
-    float* dY0 = dY_head ? dYb : dYa;  // [BT][H] fp32: gradient w.r.t. layer 0's output, written chunk by chunk
+    float* dY0 = dY_head ? w.dYb : w.dYa;  // [BT][H] fp32: gradient w.r.t. layer 0's output, written chunk by chunk
     TapeView tv1 = tape_layer(tape, 1, H, B, T), tv0 = tape_layer(tape, 0, H, B, T);
-    transpose_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * H, 256), 256, 0, st>>>(w_hh[1], H4, H, H, WT);
+    transpose_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * H, 256), 256, 0, st>>>(h->w_hh[1], H4, H, H, w.WT);
     AVVAD_LAUNCHED();
-    transpose_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * H, 256), 256, 0, st>>>(w_hh[0], H4, H, H, WT0);
+    transpose_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * H, 256), 256, 0, st>>>(h->w_hh[0], H4, H, H, w.WT0);
     AVVAD_LAUNCHED();
-    transpose_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * H, 256), 256, 0, st>>>(w_ih[1], H4, H, H, WTi);
+    transpose_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * H, 256), 256, 0, st>>>(h->w_ih[1], H4, H, H, w.WTi);
     AVVAD_LAUNCHED();
-    AVVAD_CUDA(cudaMemsetAsync(dc, 0, (size_t)B * H * 4, st));
-    AVVAD_CUDA(cudaMemsetAsync(dc0, 0, (size_t)B * H * 4, st));
-    if (int rcz = zero_pos0(dG)) return rcz;
-    if (int rcz = zero_pos0(dG0)) return rcz;
-    // steps te-1 .. tb of layer l: (cell, recurrent split-K GEMM) pairs
-    auto steps_of = [&](int l, const TapeView& tv, const float* dYl, float* dh, float* dcl, __nv_bfloat16* dGl,
-                        const __nv_bfloat16* WTl, int tb, int te, cudaStream_t s2) -> int {
-      for (int t = te - 1; t >= tb && t >= t_min; --t) {
-        const int has_rec = (t < (int)T - 1) ? kBpttSplit : 0;
-        if (bs)
-          lstm_bwd_cell_state_kernel<<<(unsigned)ceil_div(B * H, 256), 256, 0, s2>>>(
-              tv.gates, tv.c, dYl, dl_step, head_w32, dh, dcl, len_st, (int)B, (int)T, H, t, has_rec, dGl,
-              bs->layer(l, B, H));
-        else
-          lstm_bwd_cell_kernel<<<(unsigned)ceil_div(B * H, 256), 256, 0, s2>>>(tv.gates, tv.c, dYl, dl_step, head_w32, dh,
-                                                                              dcl, len_st, (int)B, (int)T, H, t, has_rec,
-                                                                              dGl);
-        AVVAD_LAUNCHED();
-        if (t > t_min) {
-          tc::EpiParams ep{};
-          ep.C = dh;
-          ep.ldc = H;
-          int rc = tc::launch_tma_gemm(dGl + (int64_t)t * H4, (int64_t)T * H4, WTl, H4, B, H, H4, ep, tc::EPI_F32, 64, s2,
-                                       kBpttSplit, (int64_t)B * H);
-          if (rc) return rc;
-        }
-      }
-      return AVVAD_OK;
-    };
-    auto warm_of = [&](float* dh, const __nv_bfloat16* dGl, const __nv_bfloat16* WTl, cudaStream_t s2) -> int {
-      tc::EpiParams ep{};
-      ep.C = dh;
-      ep.ldc = H;
-      return tc::launch_tma_gemm(dGl, (int64_t)T * H4, WTl, H4, B, H, H4, ep, tc::EPI_F32, 64, s2, kBpttSplit,
-                                 (int64_t)B * H);
-    };
+    AVVAD_CUDA(cudaMemsetAsync(w.dc, 0, (size_t)B * H * 4, st));
+    AVVAD_CUDA(cudaMemsetAsync(w.dc0, 0, (size_t)B * H * 4, st));
+    if (int rcz = zero_pos0(w.dG)) return rcz;
+    if (int rcz = zero_pos0(w.dG0)) return rcz;
     cudaStream_t side = cache->side;
-    // one real launch of the step GEMM before any capture (kernel attributes are set on first use, which cannot be
-    // captured); it must not run between chunks: dh_rec carries the recurrent term from one chunk to the next
+    // the warm-up runs here, not between chunks: dh_rec carries the recurrent term from one chunk to the next
     {
-      int rcw = warm_of(dh_rec, dG, WT, st);
+      int rcw = warm();
       if (rcw) return rcw;
     }
     auto no_warm = []() -> int { return 0; };
@@ -1043,95 +881,64 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
       const int tb = (int)(T * c / n_chunks), te = (int)(T * (c + 1) / n_chunks);
       {  // layer 1, chunk c, on the caller's stream
         const std::vector<uintptr_t> key = state_key({(uintptr_t)tv1.gates, (uintptr_t)tv1.c, (uintptr_t)dY_head,
-                                                      (uintptr_t)dl_step, (uintptr_t)head_w32, (uintptr_t)dh_rec,
-                                                      (uintptr_t)dc, (uintptr_t)len_st, (uintptr_t)dG, (uintptr_t)WT,
-                                                      (uintptr_t)B, (uintptr_t)T, (uintptr_t)H, (uintptr_t)tb,
-                                                      (uintptr_t)te, (uintptr_t)kBpttSplit});
+                                                      (uintptr_t)dl_step, (uintptr_t)h->head_w32, (uintptr_t)w.dh_rec,
+                                                      (uintptr_t)w.dc, (uintptr_t)w.len_st, (uintptr_t)w.dG,
+                                                      (uintptr_t)w.WT, (uintptr_t)B, (uintptr_t)T, (uintptr_t)H,
+                                                      (uintptr_t)tb, (uintptr_t)te, (uintptr_t)kBpttSplit});
         int rc = run_captured(use_graph ? cache : nullptr, 3 + c, key, no_warm,
-                              [&](cudaStream_t s2) { return steps_of(1, tv1, dY_head, dh_rec, dc, dG, WT, tb, te, s2); },
+                              [&](cudaStream_t s2) { return steps(1, tv1, dY_head, w.dh_rec, w.dc, w.dG, w.WT, tb, te, s2); },
                               st);
         if (rc) return rc;
       }
       AVVAD_CUDA(cudaEventRecord(cache->ev_chunk[c], st));
       AVVAD_CUDA(cudaStreamWaitEvent(side, cache->ev_chunk[c], 0));
       // dY0 of the chunk: rows (b, t in [tb, te)) of dG1 times W_ih1
-      int rc = tc::launch_tma_gemm_tm(dG + (int64_t)tb * H4, H4, WTi, H4, B, te - tb, T, H, H4, dY0 + (int64_t)tb * H, H, side);
+      int rc = tc::launch_tma_gemm_tm(w.dG + (int64_t)tb * H4, H4, w.WTi, H4, B, te - tb, T, H, H4, dY0 + (int64_t)tb * H,
+                                      H, side);
       if (rc) return rc;
       {  // layer 0, chunk c, on the side stream
         const std::vector<uintptr_t> key = state_key({(uintptr_t)tv0.gates, (uintptr_t)tv0.c, (uintptr_t)dY0,
-                                                      (uintptr_t)dl_step, (uintptr_t)head_w32, (uintptr_t)dh_rec0,
-                                                      (uintptr_t)dc0, (uintptr_t)len_st, (uintptr_t)dG0, (uintptr_t)WT0,
-                                                      (uintptr_t)B, (uintptr_t)T, (uintptr_t)H, (uintptr_t)tb,
-                                                      (uintptr_t)te, (uintptr_t)kBpttSplit});
-        rc = run_captured(use_graph ? cache : nullptr, 3 + kBpttMaxChunks + c, key, no_warm,
-                          [&](cudaStream_t s2) { return steps_of(0, tv0, dY0, dh_rec0, dc0, dG0, WT0, tb, te, s2); },
+                                                      (uintptr_t)dl_step, (uintptr_t)h->head_w32, (uintptr_t)w.dh_rec0,
+                                                      (uintptr_t)w.dc0, (uintptr_t)w.len_st, (uintptr_t)w.dG0,
+                                                      (uintptr_t)w.WT0, (uintptr_t)B, (uintptr_t)T, (uintptr_t)H,
+                                                      (uintptr_t)tb, (uintptr_t)te, (uintptr_t)kBpttSplit});
+        rc = run_captured(use_graph ? cache : nullptr, 3 + kBpttChunks + c, key, no_warm,
+                          [&](cudaStream_t s2) { return steps(0, tv0, dY0, w.dh_rec0, w.dc0, w.dG0, w.WT0, tb, te, s2); },
                           side);
         if (rc) return rc;
       }
     }
     AVVAD_CUDA(cudaEventRecord(cache->ev_side_done, side));
     // layer 1's parameter gradients (large GEMMs over K = B*T) while layer 0's last chunks still run on the side stream
-    int rc = weight_grads(1, dG, nullptr);
+    int rc = weight_grads(1, w.dG, nullptr);
     if (rc) return rc;
     AVVAD_CUDA(cudaStreamWaitEvent(st, cache->ev_side_done, 0));
-    return weight_grads(0, dG0, dx);
+    return weight_grads(0, w.dG0, dx);
   }
 
   const float* dY = dY_head;  // null (y_dim == 1): the top layer takes dl * w_head on the fly
-  float* dX_out = dY_head ? dYb : dYa;
+  float* dX_out = dY_head ? w.dYb : w.dYa;
   for (int l = layers - 1; l >= 0; --l) {
     TapeView tv = tape_layer(tape, l, H, B, T);
 
     // W_hh'^T [H][4H] for the recurrent gradient GEMM
-    transpose_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * H, 256), 256, 0, st>>>(w_hh[l], H4, H, H, WT);
+    transpose_w_kernel<<<(unsigned)ceil_div((int64_t)H4 * H, 256), 256, 0, st>>>(h->w_hh[l], H4, H, H, w.WT);
     AVVAD_LAUNCHED();
-    AVVAD_CUDA(cudaMemsetAsync(dc, 0, (size_t)B * H * 4, st));
-    if (int rcz = zero_pos0(dG)) return rcz;
-    auto run_steps = [&](cudaStream_t st) -> int {   // `st`: the caller's stream, or the capture stream
-      for (int t = (int)T - 1; t >= t_min; --t) {
-        const int has_rec = (t < (int)T - 1) ? kBpttSplit : 0;  // number of partial products to sum
-        if (bs)
-          lstm_bwd_cell_state_kernel<<<(unsigned)ceil_div(B * H, 256), 256, 0, st>>>(
-              tv.gates, tv.c, dY, dl_step, head_w32, dh_rec, dc, len_st, (int)B, (int)T, H, t, has_rec, dG,
-              bs->layer(l, B, H));
-        else
-          lstm_bwd_cell_kernel<<<(unsigned)ceil_div(B * H, 256), 256, 0, st>>>(tv.gates, tv.c, dY, dl_step, head_w32,
-                                                                              dh_rec, dc, len_st, (int)B, (int)T, H, t,
-                                                                              has_rec, dG);
-        AVVAD_LAUNCHED();
-        if (t > t_min) {
-          tc::EpiParams ep{};
-          ep.C = dh_rec;
-          ep.ldc = H;
-          // M = B is tiny: split K = 4H over kBpttSplit CTAs per output tile so the step fills the GPU
-          int rc = tc::launch_tma_gemm(dG + (int64_t)t * H4, (int64_t)T * H4, WT, H4, B, H, H4, ep, tc::EPI_F32, 64, st,
-                                       kBpttSplit, (int64_t)B * H);
-          if (rc) return rc;
-        }
-      }
-      return AVVAD_OK;
-    };
-    {
-      const std::vector<uintptr_t> key = state_key({(uintptr_t)tv.gates, (uintptr_t)tv.c, (uintptr_t)dY,
-                                                    (uintptr_t)dl_step, (uintptr_t)head_w32, (uintptr_t)dh_rec,
-                                                    (uintptr_t)dc, (uintptr_t)len_st, (uintptr_t)dG, (uintptr_t)WT,
-                                                    (uintptr_t)B, (uintptr_t)T, (uintptr_t)H});
-      auto warm = [&]() -> int {   // the kernels' one-time attribute setup is not capturable: one real split-K launch
-        tc::EpiParams ep{};
-        ep.C = dh_rec;
-        ep.ldc = H;
-        return tc::launch_tma_gemm(dG, (int64_t)T * H4, WT, H4, B, H, H4, ep, tc::EPI_F32, 64, st, kBpttSplit,
-                                   (int64_t)B * H);
-      };
-      int rc = run_captured(use_graph ? cache : nullptr, l, key, warm, run_steps, st);
-      if (rc) return rc;
-    }
+    AVVAD_CUDA(cudaMemsetAsync(w.dc, 0, (size_t)B * H * 4, st));
+    if (int rcz = zero_pos0(w.dG)) return rcz;
+    const std::vector<uintptr_t> key = state_key({(uintptr_t)tv.gates, (uintptr_t)tv.c, (uintptr_t)dY,
+                                                  (uintptr_t)dl_step, (uintptr_t)h->head_w32, (uintptr_t)w.dh_rec,
+                                                  (uintptr_t)w.dc, (uintptr_t)w.len_st, (uintptr_t)w.dG, (uintptr_t)w.WT,
+                                                  (uintptr_t)B, (uintptr_t)T, (uintptr_t)H});
+    int rc = run_captured(use_graph ? cache : nullptr, l, key, warm,
+                          [&](cudaStream_t s) { return steps(l, tv, dY, w.dh_rec, w.dc, w.dG, w.WT, 0, (int)T, s); }, st);
+    if (rc) return rc;
     float* dst = (l == 0) ? dx : dX_out;
-    int rc = weight_grads(l, dG, (l > 0 || dx) ? dst : nullptr);
+    rc = weight_grads(l, w.dG, (l > 0 || dx) ? dst : nullptr);
     if (rc) return rc;
     if (l > 0 || dx) {
       dY = dst;
-      dX_out = (dX_out == dYa) ? dYb : dYa;
+      dX_out = (dX_out == w.dYa) ? w.dYb : w.dYa;
     }
   }
   return AVVAD_OK;
@@ -1140,11 +947,6 @@ int lstm_backward_impl(int layers, int input_size, int64_t ld0, int H, int y_dim
 // ---- stateful backward (avvad_lstm_backward_state) over a tape of T + 1 positions per row.  The per-call tensors of
 // T steps are laid out once more with a leading position 0 -- zero rows of x and dlogits, lengths + 1 -- so that
 // lstm_backward_impl runs its schedules unchanged over T + 1 positions; dx is read back from positions 1..T.
-__global__ void shift_lengths_bwd_kernel(const int32_t* __restrict__ lengths, int B, int32_t* __restrict__ out) {
-  const int b = blockIdx.x * blockDim.x + threadIdx.x;
-  if (b < B) out[b] = lengths[b] + 1;
-}
-
 namespace {
 struct StateBwdWs {
   int32_t* len1;
@@ -1155,7 +957,7 @@ struct StateBwdWs {
   uint8_t* inner;     // lstm_backward_impl's workspace
   size_t total;
 };
-StateBwdWs carve_state_bwd(int layers, int input_size, int64_t ld0, int H, int y_dim, int64_t B, int64_t T, void* base) {
+StateBwdWs carve_state_bwd(const avvad_lstm* h, int64_t B, int64_t T, void* base) {
   StateBwdWs w{};
   size_t off = 0;
   auto take = [&](size_t bytes) {
@@ -1164,37 +966,35 @@ StateBwdWs carve_state_bwd(int layers, int input_size, int64_t ld0, int H, int y
     return p;
   };
   const int64_t T1 = T + 1;
-  const size_t st = (size_t)layers * B * H * sizeof(float);
+  const size_t st = (size_t)h->layers * B * h->H * sizeof(float);
   w.len1 = (int32_t*)take((size_t)B * 4);
-  w.x1 = (__nv_bfloat16*)take((size_t)B * T1 * ld0 * 2);
-  w.dl1 = (float*)take((size_t)B * T1 * y_dim * 4);
-  w.dx1 = (float*)take((size_t)B * T1 * input_size * 4);
+  w.x1 = (__nv_bfloat16*)take((size_t)B * T1 * h->ld0 * 2);
+  w.dl1 = (float*)take((size_t)B * T1 * h->y_dim * 4);
+  w.dx1 = (float*)take((size_t)B * T1 * h->input_size * 4);
   w.dh_out = (float*)take(st);
   w.dc_out = (float*)take(st);
   w.dh_in = (float*)take(st);
   w.dc_in = (float*)take(st);
   w.inner = (uint8_t*)take(0);
-  w.total = off + lstm_backward_workspace(layers, input_size, ld0, H, y_dim, B, T1);
+  w.total = off + lstm_backward_workspace(h, B, T1);
   return w;
 }
 }  // namespace
 
-size_t lstm_backward_state_workspace(int layers, int input_size, int64_t ld0, int H, int y_dim, int64_t B, int64_t T) {
-  return carve_state_bwd(layers, input_size, ld0, H, y_dim, B, T, nullptr).total;
+size_t lstm_backward_state_workspace(const avvad_lstm* h, int64_t B, int64_t T) {
+  return carve_state_bwd(h, B, T, nullptr).total;
 }
 
-int lstm_backward_state_impl(int layers, int input_size, int64_t ld0, int H, int y_dim, __nv_bfloat16* const* w_ih,
-                             __nv_bfloat16* const* w_hh, const float* head_w32, const __nv_bfloat16* head_w16,
-                             const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T, void* tape,
-                             const float* dlogits, const float* dh_out, const float* dc_out, float* dh_in, float* dc_in,
-                             void* workspace, size_t workspace_bytes, float* const* dW_ih, float* const* dW_hh,
-                             float* const* db, float* dW_head, float* db_head, float* dx, cudaStream_t st,
-                             BpttGraphCache* cache) {
+int lstm_backward_state_impl(const avvad_lstm* h, const void* x_bf16, const int32_t* lengths, int64_t B, int64_t T,
+                             void* tape, const float* dlogits, const float* dh_out, const float* dc_out, float* dh_in,
+                             float* dc_in, void* workspace, size_t workspace_bytes, float* const* dW_ih,
+                             float* const* dW_hh, float* const* db, float* dW_head, float* db_head, float* dx,
+                             cudaStream_t st) {
   AVVAD_CHECK_ARG(B > 0 && T > 0, "bad sizes");
-  const StateBwdWs w = carve_state_bwd(layers, input_size, ld0, H, y_dim, B, T, workspace);
+  const StateBwdWs w = carve_state_bwd(h, B, T, workspace);
   AVVAD_CHECK_ARG(workspace_bytes >= w.total, "workspace too small");
   const int64_t T1 = T + 1;
-  shift_lengths_bwd_kernel<<<(unsigned)ceil_div(B, 256), 256, 0, st>>>(lengths, (int)B, w.len1);
+  shift_lengths_kernel<<<(unsigned)ceil_div(B, 256), 256, 0, st>>>(lengths, (int)B, w.len1);
   AVVAD_LAUNCHED();
   // [B][T][n] -> [B][T+1][n] with a zero row at position 0
   auto widen = [&](void* dst, const void* src, size_t row_bytes) -> int {
@@ -1203,23 +1003,23 @@ int lstm_backward_state_impl(int layers, int input_size, int64_t ld0, int H, int
                                  cudaMemcpyDeviceToDevice, st));
     return AVVAD_OK;
   };
-  int rc = widen(w.x1, x_bf16, (size_t)ld0 * 2);
-  if (!rc) rc = widen(w.dl1, dlogits, (size_t)y_dim * 4);
+  int rc = widen(w.x1, x_bf16, (size_t)h->ld0 * 2);
+  if (!rc) rc = widen(w.dl1, dlogits, (size_t)h->y_dim * 4);
   if (rc) return rc;
   // the state gradients at stable addresses (inputs copied first, so outputs may alias them)
-  const size_t sbytes = (size_t)layers * B * H * sizeof(float);
+  const size_t sbytes = (size_t)h->layers * B * h->H * sizeof(float);
   if (dh_out) AVVAD_CUDA(cudaMemcpyAsync(w.dh_out, dh_out, sbytes, cudaMemcpyDeviceToDevice, st));
   else AVVAD_CUDA(cudaMemsetAsync(w.dh_out, 0, sbytes, st));
   if (dc_out) AVVAD_CUDA(cudaMemcpyAsync(w.dc_out, dc_out, sbytes, cudaMemcpyDeviceToDevice, st));
   else AVVAD_CUDA(cudaMemsetAsync(w.dc_out, 0, sbytes, st));
   const bool want = dh_in || dc_in;
   const BpttState bs{w.dh_out, w.dc_out, want ? w.dh_in : nullptr, want ? w.dc_in : nullptr};
-  rc = lstm_backward_impl(layers, input_size, ld0, H, y_dim, w_ih, w_hh, head_w32, head_w16, w.x1, w.len1, B, T1, tape,
-                          w.dl1, w.inner, workspace_bytes - (size_t)(w.inner - (uint8_t*)workspace), dW_ih, dW_hh, db,
-                          dW_head, db_head, dx ? w.dx1 : nullptr, st, cache, &bs);
+  rc = lstm_backward_impl(h, w.x1, w.len1, B, T1, tape, w.dl1, w.inner,
+                          workspace_bytes - (size_t)(w.inner - (uint8_t*)workspace), dW_ih, dW_hh, db, dW_head, db_head,
+                          dx ? w.dx1 : nullptr, st, &bs);
   if (rc) return rc;
   if (dx) {
-    const size_t row = (size_t)input_size * 4;
+    const size_t row = (size_t)h->input_size * 4;
     AVVAD_CUDA(cudaMemcpy2DAsync(dx, T * row, (uint8_t*)w.dx1 + row, T1 * row, T * row, (size_t)B,
                                  cudaMemcpyDeviceToDevice, st));
   }

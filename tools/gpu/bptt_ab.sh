@@ -7,6 +7,5 @@ run() { echo "== $*" >> $O; timeout 300 env "$@" >> $O 2>&1; echo "rc=$?" >> $O;
 for B in ${BS:-96 128 256}; do
 run AVVAD_BPTT_CHUNKS=1 python tools/micro/bptt_ab.py $B 317 --save /tmp/g$B.pt
 run AVVAD_BPTT_CHUNKS=8 python tools/micro/bptt_ab.py $B 317 --cmp /tmp/g$B.pt
-run AVVAD_BPTT_CHUNKS=4 python tools/micro/bptt_ab.py $B 317 --cmp /tmp/g$B.pt
 done
 grep -v "^rc=0" $O
