@@ -61,18 +61,32 @@ def upsampled_length(n_src: int, num=FPS_NUM, den=FPS_DEN) -> int:
 
 def frontend_logpower(wave: torch.Tensor, n_samples, n_frames, t_max: int, mean: Optional[torch.Tensor],
                       std: Optional[torch.Tensor], eps=1e-8, normalise=True, out: Optional[torch.Tensor] = None,
-                      peaks: Optional[torch.Tensor] = None):
+                      peaks: Optional[torch.Tensor] = None, out_bf16: Optional[torch.Tensor] = None,
+                      ld: Optional[int] = None, col_off=0):
     """(B,N) fp32 waveforms -> (B,t_max,513) standardised log-power features (SURVEY A1-A4).
 
     ``peaks`` (f32 (B,)): with ``normalise``, divide by these per-utterance peaks instead of max|x| over the samples
-    given -- a stream sees only part of the utterance."""
+    given -- a stream sees only part of the utterance.
+
+    ``out_bf16`` (bf16, B * t_max rows of ``ld`` elements, default ld = its last dimension): write the features
+    rounded to bf16 there instead, at columns ``col_off .. col_off + 512``, and zero the columns after them -- an LSTM
+    layer-0 operand in one kernel, bit-identical to ``pack_rows_bf16(features, out_bf16, col_off, zero_tail=True)``.
+    Returns ``out_bf16`` then."""
     L.require_cuda(wave)
     assert wave.dim() == 2 and wave.dtype == torch.float32
     wave = wave.contiguous()
     B = wave.shape[0]
     dev = wave.device
     ns, nf = _i32(n_samples, dev), _i32(n_frames, dev)
-    if out is None:
+    if out_bf16 is not None:
+        if out is not None:
+            raise ValueError("frontend_logpower: give out or out_bf16, not both")
+        ld = int(out_bf16.shape[-1]) if ld is None else int(ld)
+        if (out_bf16.dtype != torch.bfloat16 or not out_bf16.is_contiguous() or out_bf16.device != dev
+                or out_bf16.numel() < B * t_max * ld):
+            raise ValueError(f"frontend_logpower: out_bf16 must be a contiguous bf16 tensor of B * t_max = {B * t_max} "
+                             f"rows of ld = {ld} on {dev}")
+    elif out is None:
         out = torch.empty(B, t_max, 513, dtype=torch.float32, device=dev)
     mode = 0
     if normalise:
@@ -85,6 +99,11 @@ def frontend_logpower(wave: torch.Tensor, n_samples, n_frames, t_max: int, mean:
         peak = torch.empty(B, dtype=torch.float32, device=dev)
     m = _f32(mean.reshape(-1), dev) if mean is not None else None
     s = _f32(std.reshape(-1), dev) if std is not None else None
+    if out_bf16 is not None:
+        L.check(L.lib().avvad_frontend_logpower_bf16(L.ptr(wave), wave.stride(0), L.ptr(ns), L.ptr(nf), B, t_max, mode,
+                                                     L.ptr(m), L.ptr(s), eps, L.ptr(out_bf16), ld, int(col_off),
+                                                     L.ptr(peak), L.stream_ptr()))
+        return out_bf16
     L.check(L.lib().avvad_frontend_logpower(L.ptr(wave), wave.stride(0), L.ptr(ns), L.ptr(nf), B, t_max,
                                             mode, L.ptr(m), L.ptr(s), eps, L.ptr(out), L.ptr(peak),
                                             L.stream_ptr()))

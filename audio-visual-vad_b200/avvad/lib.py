@@ -32,7 +32,9 @@ PROTOTYPES = {
     "avvad_stft_num_frames": (C.c_int64, [C.c_int64, C.c_double, C.c_double, C.c_double, C.c_int]),
     "avvad_frontend_logpower": (C.c_int, [VP, C.c_int64, VP, VP, C.c_int32, C.c_int32, C.c_int, VP, VP, C.c_float,
                                           VP, VP, VP]),
-    "avvad_stft": (C.c_int, [VP, C.c_int64, VP, VP, C.c_int32, C.c_int32, VP, VP]),
+    "avvad_frontend_logpower_bf16": (C.c_int, [VP, C.c_int64, VP, VP, C.c_int32, C.c_int32, C.c_int, VP, VP,
+                                               C.c_float, VP, C.c_int64, C.c_int64, VP, VP]),
+    "avvad_stft":(C.c_int, [VP, C.c_int64, VP, VP, C.c_int32, C.c_int32, VP, VP]),
     "avvad_upsampled_length": (C.c_int64, [C.c_int64, C.c_int32, C.c_int32]),
     "avvad_upsample_gather": (C.c_int, [VP, C.c_int, VP, VP, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                         C.c_int32, C.c_float, C.c_float, C.c_float, C.c_int, VP, VP]),

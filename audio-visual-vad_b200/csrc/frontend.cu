@@ -165,11 +165,32 @@ struct FeSmem {
   float stdv[520];
 };
 
+// Output modes of frontend_reg_kernel.  FeOutF32: standardised fp32 rows (B, t_max, 513).  FeOutBf16: the same values
+// rounded to bf16 (__float2bfloat16_rn), written straight into an LSTM layer-0 operand of leading dimension `ld` from
+// column `col_off` on, with the columns [col_off + 513, ld) of every row zeroed (== the fp32 rows through
+// pack_rows_bf16(zero_tail = 1), without the fp32 round trip through HBM).
+struct FeOutF32 {
+  float* __restrict__ p;
+  __device__ float* row(int64_t f) const { return p + f * 513; }
+  __device__ static void put(float* o, int k, float v) { o[k] = v; }
+  __device__ void tail(float*, int) const {}
+};
+struct FeOutBf16 {
+  __nv_bfloat16* __restrict__ p;
+  int64_t ld, col_off;
+  __device__ __nv_bfloat16* row(int64_t f) const { return p + f * ld + col_off; }
+  __device__ static void put(__nv_bfloat16* o, int k, float v) { o[k] = __float2bfloat16_rn(v); }
+  __device__ void tail(__nv_bfloat16* o, int t) const {
+    for (int64_t k = 513 + t; k < ld - col_off; k += kRfThreads) o[k] = __float2bfloat16_rn(0.f);
+  }
+};
+
+template <class Out>
 __global__ void __launch_bounds__(kFeGroups * kRfThreads, 3)
 frontend_reg_kernel(const float* __restrict__ wave, int64_t wave_stride, const int32_t* __restrict__ n_samples,
                     const int32_t* __restrict__ n_frames, int B, int t_max, const float* __restrict__ peak,
                     const float* __restrict__ mean, const float* __restrict__ stdv, float eps,
-                    const float2* __restrict__ tw_g, float* __restrict__ out) {
+                    const float2* __restrict__ tw_g, Out out) {
   extern __shared__ __align__(16) uint8_t fe_smem_raw[];
   FeSmem& sm = *reinterpret_cast<FeSmem*>(fe_smem_raw);
   const int tid = threadIdx.x;
@@ -193,10 +214,12 @@ frontend_reg_kernel(const float* __restrict__ wave, int64_t wave_stride, const i
   const int64_t frames = (int64_t)B * t_max;
   for (int64_t f = (int64_t)blockIdx.x * kFeGroups + g; f < frames; f += (int64_t)gridDim.x * kFeGroups) {
     const int b = (int)(f / t_max), fr = (int)(f - (int64_t)b * t_max);
-    float* o = out + f * 513;
+    auto* o = out.row(f);
+    out.tail(o, t);
     if (fr >= min(n_frames[b], t_max)) {
       // collate padding: zeros are padded BEFORE standardisation -> (0 - mean) / (std + eps)
-      for (int k = t; k < 513; k += kRfThreads) o[k] = has_stats ? (0.f - sm.mean[k]) / (sm.stdv[k] + eps) : 0.f;
+      for (int k = t; k < 513; k += kRfThreads)
+        Out::put(o, k, has_stats ? (0.f - sm.mean[k]) / (sm.stdv[k] + eps) : 0.f);
       continue;
     }
     const int n = n_samples[b];
@@ -217,7 +240,7 @@ frontend_reg_kernel(const float* __restrict__ wave, int64_t wave_stride, const i
       const int k = t + 64 * m;
       if (k <= 512) {
         const float la = logf(v[m].x * v[m].x + v[m].y * v[m].y + eps);
-        o[k] = has_stats ? (la - sm.mean[k]) / (sm.stdv[k] + eps) : la;
+        Out::put(o, k, has_stats ? (la - sm.mean[k]) / (sm.stdv[k] + eps) : la);
       }
     }
   }
@@ -243,12 +266,36 @@ extern "C" int64_t avvad_stft_num_frames(int64_t n_samples, double fs, double wl
   return 1 + (n - nfft) / hop;
 }
 
+template <class Out>
+static int launch_frontend_reg(const float* wave, int64_t wave_stride, const int32_t* n_samples,
+                               const int32_t* n_frames, int32_t B, int32_t t_max, const float* peak,
+                               const float* mean, const float* stdv, float eps, const float2* tw, Out out,
+                               cudaStream_t st) {
+  static PerDeviceOnce attr_once;
+  int sms = 0, dev = 0;
+  AVVAD_CUDA(cudaGetDevice(&dev));
+  AVVAD_CUDA(attr_once.run([] {
+    return cudaFuncSetAttribute(frontend_reg_kernel<Out>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)sizeof(FeSmem));
+  }));
+  AVVAD_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  const int64_t want = ceil_div((int64_t)B * t_max, (int64_t)kFeGroups);
+  const unsigned ctas = (unsigned)std::min<int64_t>(want, (int64_t)sms * 3);
+  frontend_reg_kernel<Out><<<ctas, kFeGroups * kRfThreads, sizeof(FeSmem), st>>>(
+      wave, wave_stride, n_samples, n_frames, B, t_max, peak, mean, stdv, eps, tw, out);
+  return AVVAD_OK;
+}
+
+// out_bf16 != NULL (mode 0 only): bf16 operand rows (FeOutBf16) on the register-FFT kernel, whatever AVVAD_FE_REG says.
 static int launch_frontend(int mode, const float* wave, int64_t wave_stride, const int32_t* n_samples,
                            const int32_t* n_frames, int32_t B, int32_t t_max, int normalise,
                            const float* mean, const float* stdv, float eps, float* out,
-                           float* peak_scratch, cudaStream_t st) {
-  AVVAD_CHECK_ARG(wave && n_samples && n_frames && out, "null pointer");
+                           float* peak_scratch, cudaStream_t st, void* out_bf16 = nullptr, int64_t ld = 0,
+                           int64_t col_off = 0) {
+  AVVAD_CHECK_ARG(wave && n_samples && n_frames && (out || out_bf16), "null pointer");
   AVVAD_CHECK_ARG(B > 0 && t_max > 0 && wave_stride > 0, "B, t_max, wave_stride must be positive");
+  AVVAD_CHECK_ARG(!out_bf16 || (col_off >= 0 && ld % 8 == 0 && ld >= col_off + 513),
+                  "bf16 output: ld must be a multiple of 8 and at least col_off + 513, col_off >= 0");
   AVVAD_CHECK_ARG((mean == nullptr) == (stdv == nullptr), "mean and std must both be given or both NULL");
   AVVAD_CHECK_ARG(normalise >= 0 && normalise <= 2, "normalise must be 0, 1 or 2");
   AVVAD_CHECK_ARG(!normalise || peak_scratch, "peak_scratch required when normalise != 0");
@@ -273,18 +320,15 @@ static int launch_frontend(int mode, const float* wave, int64_t wave_stride, con
     const char* e = getenv("AVVAD_FE_REG");
     reg_mode = (e && e[0] == '0') ? 0 : 1;
   }
-  if (mode == 0 && reg_mode) {
-    static PerDeviceOnce attr_once;
-    int sms = 0, dev = 0;
-    AVVAD_CUDA(cudaGetDevice(&dev));
-    AVVAD_CUDA(attr_once.run([] {
-      return cudaFuncSetAttribute(frontend_reg_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FeSmem));
-    }));
-    AVVAD_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    const int64_t want = ceil_div((int64_t)B * t_max, (int64_t)kFeGroups);
-    const unsigned ctas = (unsigned)std::min<int64_t>(want, (int64_t)sms * 3);
-    frontend_reg_kernel<<<ctas, kFeGroups * kRfThreads, sizeof(FeSmem), st>>>(
-        wave, wave_stride, n_samples, n_frames, B, t_max, normalise ? peak_scratch : nullptr, mean, stdv, eps, tw, out);
+  const float* peak = normalise ? peak_scratch : nullptr;
+  if (mode == 0 && out_bf16) {
+    const int rc = launch_frontend_reg(wave, wave_stride, n_samples, n_frames, B, t_max, peak, mean, stdv, eps, tw,
+                                       FeOutBf16{(__nv_bfloat16*)out_bf16, ld, col_off}, st);
+    if (rc) return rc;
+  } else if (mode == 0 && reg_mode) {
+    const int rc = launch_frontend_reg(wave, wave_stride, n_samples, n_frames, B, t_max, peak, mean, stdv, eps, tw,
+                                       FeOutF32{out}, st);
+    if (rc) return rc;
   } else if (mode == 0)
     frontend_kernel<0><<<grid, kFftThreads, 0, st>>>(wave, wave_stride, n_samples, n_frames, t_max,
                                                      normalise ? peak_scratch : nullptr, mean, stdv, eps, tw, out);
@@ -292,7 +336,8 @@ static int launch_frontend(int mode, const float* wave, int64_t wave_stride, con
     frontend_kernel<1><<<grid, kFftThreads, 0, st>>>(wave, wave_stride, n_samples, n_frames, t_max, nullptr,
                                                      nullptr, nullptr, 0.f, tw, out);
   AVVAD_LAUNCHED();
-  tc::prof_end(st, ptok, 4, (double)B * t_max * (1024.0 + (mode == 0 ? 2052.0 : 4104.0)));
+  const double out_bytes = out_bf16 ? 2.0 * (double)(ld - col_off) : (mode == 0 ? 2052.0 : 4104.0);
+  tc::prof_end(st, ptok, 4, (double)B * t_max * (1024.0 + out_bytes));
   return AVVAD_OK;
 }
 
@@ -302,6 +347,15 @@ extern "C" int avvad_frontend_logpower(const float* wave, int64_t wave_stride, c
                                        float* peak_scratch, void* stream) {
   return launch_frontend(0, wave, wave_stride, n_samples, n_frames, B, t_max, normalise, mean, stdv, eps, out,
                          peak_scratch, (cudaStream_t)stream);
+}
+
+extern "C" int avvad_frontend_logpower_bf16(const float* wave, int64_t wave_stride, const int32_t* n_samples,
+                                            const int32_t* n_frames, int32_t B, int32_t t_max, int normalise,
+                                            const float* mean, const float* stdv, float eps, void* out_bf16,
+                                            int64_t ld, int64_t col_off, float* peak_scratch, void* stream) {
+  AVVAD_CHECK_ARG(out_bf16, "null pointer");
+  return launch_frontend(0, wave, wave_stride, n_samples, n_frames, B, t_max, normalise, mean, stdv, eps, nullptr,
+                         peak_scratch, (cudaStream_t)stream, out_bf16, ld, col_off);
 }
 
 extern "C" int avvad_stft(const float* wave, int64_t wave_stride, const int32_t* n_samples,

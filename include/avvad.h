@@ -78,6 +78,19 @@ int avvad_frontend_logpower(const float* wave, int64_t wave_stride, const int32_
                             const float* mean, const float* std, float eps, float* out,
                             float* peak_scratch, void* stream);
 
+/* avvad_frontend_logpower written straight into a bf16 LSTM layer-0 operand (the audio-only model has nothing between
+ * the front end and the recurrence):
+ * out_bf16 : bf16 [B][t_max][ld] device.  Row (b, t) gets __float2bfloat16_rn of the value avvad_frontend_logpower
+ *            writes to out[b][t][k] at column col_off + k (k < 513), and zeros in columns [col_off + 513, ld); columns
+ *            below col_off are not touched.  == avvad_frontend_logpower + avvad_pack_rows_bf16(zero_tail = 1), bit
+ *            for bit.
+ * ld       : multiple of 8, >= col_off + 513.  Every other argument as avvad_frontend_logpower.  Always runs the
+ *            register-FFT kernel (AVVAD_FE_REG only selects the kernel of the f32 output). */
+int avvad_frontend_logpower_bf16(const float* wave, int64_t wave_stride, const int32_t* n_samples,
+                                 const int32_t* n_frames, int32_t B, int32_t t_max, int normalise,
+                                 const float* mean, const float* std, float eps, void* out_bf16, int64_t ld,
+                                 int64_t col_off, float* peak_scratch, void* stream);
+
 /* Raw STFT, (B, 513, t_max, 2) real view like the legacy torch.stft the reference calls
  * (stft.py:145-151).  No normalisation / log. */
 int avvad_stft(const float* wave, int64_t wave_stride, const int32_t* n_samples,
