@@ -904,6 +904,9 @@ class WaveNetEncoder:
         for i in range(self.n_dil):
             keep.append(put(1, i, f"en_dilation_layer_stack.{i}"))
             keep.append(put(2, i, f"en_dense_layer_stack.{i}"))
+        # weight shapes and bias presence in the backward's gradient order (WAVENET_LAYER_NAMES)
+        self.grad_layout = [(tuple(sd[n + ".weight"].shape), (n + ".bias") in sd)
+                            for n in wavenet_layer_names(self.n_dil)]
         torch.cuda.current_stream().synchronize()
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
@@ -915,3 +918,47 @@ class WaveNetEncoder:
         out = torch.empty(B, self.bottleneck, self.pool, dtype=torch.float32, device=x.device)
         L.check(L.lib().avvad_wavenet_encode(self.h, L.ptr(x), B, N, L.ptr(ws), ws.numel(), L.ptr(out), L.stream_ptr()))
         return out
+
+    def forward_train(self, x: torch.Tensor):
+        """(out, tape): ``forward``'s output, bit for bit, and the tape ``backward`` reads (its own buffer per call, so
+        several forwards may precede their backwards)."""
+        L.require_cuda(x)
+        x = x.detach().to(torch.float32).contiguous()
+        B, _, N = x.shape
+        ws = self.ws.get(L.lib().avvad_wavenet_workspace_bytes(self.h, B, N), x.device)
+        tape = torch.empty(max(int(L.lib().avvad_wavenet_tape_bytes(self.h, B, N)), 1), dtype=torch.uint8,
+                           device=x.device)
+        out = torch.empty(B, self.bottleneck, self.pool, dtype=torch.float32, device=x.device)
+        L.check(L.lib().avvad_wavenet_encode_train(self.h, L.ptr(x), B, N, L.ptr(ws), ws.numel(), L.ptr(tape),
+                                                   tape.numel(), L.ptr(out), L.stream_ptr()))
+        return out, (x, tape)
+
+    def backward(self, tape, dout: torch.Tensor, want_dx: bool = False):
+        """Gradients from a ``forward_train`` tape and d loss / d out (any strides).  Returns (dx or None, grads), grads
+        in ``wavenet_params`` order: weight (and bias, when the module has them) of en_causal_layer, then per layer
+        en_dilation_layer_stack.i / en_dense_layer_stack.i, then bottleneck_layer, in PyTorch's layout."""
+        x, tp = tape
+        B, _, N = x.shape
+        dout = dout.detach().to(device=x.device, dtype=torch.float32).contiguous()
+        dws = [torch.empty(shape, dtype=torch.float32, device=x.device) for shape, _ in self.grad_layout]
+        dbs = [torch.empty(shape[0], dtype=torch.float32, device=x.device) if has_b else None
+               for shape, has_b in self.grad_layout]
+        dx = torch.empty_like(x) if want_dx else None
+        n = len(dws)
+        pw = (C.c_void_p * n)(*[t.data_ptr() for t in dws])
+        pb = (C.c_void_p * n)(*[t.data_ptr() if t is not None else None for t in dbs])
+        ws = self.ws.get(L.lib().avvad_wavenet_backward_workspace_bytes(self.h, B, N), x.device)
+        L.check(L.lib().avvad_wavenet_backward(self.h, L.ptr(x), B, N, L.ptr(tp), tp.numel(), L.ptr(dout), L.ptr(dx),
+                                               pw, pb, L.ptr(ws), ws.numel(), L.stream_ptr()))
+        grads = []
+        for w, b in zip(dws, dbs):
+            grads += [w] if b is None else [w, b]
+        return dx, grads
+
+
+def wavenet_layer_names(n_dilations: int):
+    """Conv1d layers of the WaveNet encoder in the C ABI's gradient order."""
+    names = ["en_causal_layer"]
+    for i in range(n_dilations):
+        names += [f"en_dilation_layer_stack.{i}", f"en_dense_layer_stack.{i}"]
+    return names + ["bottleneck_layer"]

@@ -111,6 +111,11 @@ PROTOTYPES = {
     "avvad_wavenet_encoded_length": (C.c_int64, [VP, C.c_int64]),
     "avvad_wavenet_workspace_bytes": (C.c_size_t, [VP, C.c_int64, C.c_int64]),
     "avvad_wavenet_encode": (C.c_int, [VP, VP, C.c_int64, C.c_int64, VP, C.c_size_t, VP, VP]),
+    "avvad_wavenet_tape_bytes": (C.c_size_t, [VP, C.c_int64, C.c_int64]),
+    "avvad_wavenet_encode_train": (C.c_int, [VP, VP, C.c_int64, C.c_int64, VP, C.c_size_t, VP, C.c_size_t, VP, VP]),
+    "avvad_wavenet_backward_workspace_bytes": (C.c_size_t, [VP, C.c_int64, C.c_int64]),
+    "avvad_wavenet_backward": (C.c_int, [VP, VP, C.c_int64, C.c_int64, VP, C.c_size_t, VP, VP, VP, VP, VP, C.c_size_t,
+                                         VP]),
     "avvad_mcb_forward_train": (C.c_int, [VP, VP, VP, C.c_int64, VP, C.c_size_t, VP, VP, C.c_float, VP, VP, VP, C.c_int64,
                                           VP, VP]),
     "avvad_mcb_backward_bn": (C.c_int, [VP, VP, VP, C.c_int64, C.c_int64, VP, VP, VP]),

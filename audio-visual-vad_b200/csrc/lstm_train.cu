@@ -15,6 +15,7 @@
 // holds the initial state; see the kState instantiations of the cell kernels and lstm_backward_state_impl.
 #include <vector>
 
+#include "bwd_common.cuh"
 #include "gemm_tma.cuh"
 #include "lstm_internal.cuh"
 
@@ -210,31 +211,6 @@ __global__ void lstm_wf_pack_w_kernel(const __nv_bfloat16* __restrict__ whh1, co
   out[idx] = v;
 }
 
-// bf16 [R][ld] (first C columns) -> [C][Rp] with zero fill for r >= R; `shift` > 0 reads row r - shift*? (see below)
-// mode 0: plain transpose.  mode 1: H_prev transpose: out[c][b*T + t] = in[b*T + t - 1][c] for t > 0, else 0.
-__global__ void transpose_bf16_kernel(const __nv_bfloat16* __restrict__ in, int64_t R, int C, int64_t ld, int64_t Rp,
-                                      int mode, int T, __nv_bfloat16* __restrict__ out) {
-  __shared__ __nv_bfloat16 tile[32][33];
-  const int64_t r0 = (int64_t)blockIdx.x * 32;
-  const int c0 = blockIdx.y * 32;
-  for (int i = threadIdx.y; i < 32; i += 8) {
-    const int64_t r = r0 + i;
-    const int c = c0 + threadIdx.x;
-    __nv_bfloat16 v = __float2bfloat16_rn(0.f);
-    if (r < R && c < C) {
-      if (mode == 0) v = in[r * ld + c];
-      else if ((r % T) != 0) v = in[(r - 1) * ld + c];
-    }
-    tile[i][threadIdx.x] = v;
-  }
-  __syncthreads();
-  for (int i = threadIdx.y; i < 32; i += 8) {
-    const int c = c0 + i;
-    const int64_t r = r0 + threadIdx.x;
-    if (c < C && r < Rp) out[(int64_t)c * Rp + r] = tile[threadIdx.x][i];
-  }
-}
-
 // W' (gate-interleaved rows 4u+g) bf16 [4H][ld] -> W'^T bf16 [cols][4H]
 __global__ void transpose_w_kernel(const __nv_bfloat16* __restrict__ w, int rows, int cols, int ld,
                                    __nv_bfloat16* __restrict__ out) {
@@ -295,21 +271,6 @@ __global__ void head_wt_kernel(const __nv_bfloat16* __restrict__ w, int y, int H
   const int u = (int)(idx / yp), k = (int)(idx - (int64_t)u * yp);
   out[idx] = (k < y) ? w[(int64_t)k * H + u] : __float2bfloat16_rn(0.f);
 }
-// out[c] = sum_r x[r][c]  (fp32, 64 columns per block, fixed-order reduction over four row lanes)
-__global__ void __launch_bounds__(256) colsum_f32_kernel(const float* __restrict__ x, int64_t R, int Ccols,
-                                                         float* __restrict__ out) {
-  __shared__ float sm[4][64];
-  const int col = blockIdx.x * 64 + (threadIdx.x & 63);
-  const int part = threadIdx.x >> 6;
-  float acc = 0.f;
-  if (col < Ccols)
-    for (int64_t r = part; r < R; r += 4) acc += x[r * Ccols + col];
-  sm[part][threadIdx.x & 63] = acc;
-  __syncthreads();
-  if (threadIdx.x < 64 && col < Ccols)
-    out[col] = sm[0][threadIdx.x] + sm[1][threadIdx.x] + sm[2][threadIdx.x] + sm[3][threadIdx.x];
-}
-
 // y_dim == 1 head: dW[u] = sum_r dl[r] * h[r][u]; db = sum_r dl[r].  Two-stage deterministic reduction.
 __global__ void __launch_bounds__(256) head_grad_partial_kernel(const float* __restrict__ dl,
                                                                 const __nv_bfloat16* __restrict__ h, int64_t R, int H,

@@ -22,6 +22,7 @@
 //   max-pool / average-pool        : index-exact (first maximum in scan order, as PyTorch's kernels pick)
 // Gradient activations travel in bf16 (fp32 accumulation inside every kernel), parameters' gradients come back fp32 in
 // PyTorch's layout.
+#include "bwd_common.cuh"
 
 namespace avvad {
 namespace bwd {
@@ -414,15 +415,6 @@ __global__ void __launch_bounds__(256) im2col_t_kernel(const __nv_bfloat16* __re
     }
     *reinterpret_cast<uint4*>(col + ((int64_t)tap * Cin + c0 + c) * Pp + p0 + pc * 8) = make_uint4(w[0], w[1], w[2], w[3]);
   }
-}
-// acc[j] (+)= sum_s part[s][j]
-__global__ void sum_partials_kernel(const float* __restrict__ part, int nparts, int64_t elems, int accumulate,
-                                    float* __restrict__ acc) {
-  const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (j >= elems) return;
-  float t = accumulate ? acc[j] : 0.f;
-  for (int s = 0; s < nparts; ++s) t += part[(int64_t)s * elems + j];
-  acc[j] = t;
 }
 // [O][tap][I] fp32 -> PyTorch layout [O][I][k][k]
 __global__ void wgrad_layout_kernel(const float* __restrict__ acc, int O, int I, int k, float* __restrict__ dw) {

@@ -223,22 +223,76 @@ extern "C" size_t avvad_wavenet_workspace_bytes(const avvad_wavenet* h, int64_t 
   return align_up(rows * h->k * maxC * 2, 256) + align_up(rows * maxC * 2, 256) + 3 * align_up(rows * maxC * 4, 256) + 1024;
 }
 
+// Training tape: S_i = the input of dilated layer i (i = 0..n; S_n feeds the bottleneck) as bf16 [B][L_i][Rp], back to
+// back; act_i = relu(dilated_i + bias) as bf16 [B][L_{i+1}][Dp], back to back; the bottleneck output relu(...) as f32
+// [B][L_n][bp] (the tensor the pool reads).  bf16(relu(S_i)) is exactly the operand the forward fed to dilated layer i
+// (ReLU commutes with round-to-nearest), and bf16 keeps fp32's exponent range, so the ReLU masks survive the rounding.
+struct WnTape {
+  std::vector<int64_t> L;   // L[i] = rows per item of S_i
+  std::vector<__nv_bfloat16*> S, act;
+  float* out = nullptr;
+  size_t bytes = 0;
+};
+static WnTape wn_tape(const avvad_wavenet* h, int64_t B, int64_t N, void* base) {
+  WnTape t;
+  const int n = (int)h->dil.size();
+  t.L.resize(n + 1);
+  t.L[0] = N - (h->k - 1);
+  for (int i = 0; i < n; ++i) t.L[i + 1] = t.L[i] - (int64_t)(h->k - 1) * h->dil[i];
+  uint8_t* p = (uint8_t*)base;
+  size_t off = 0;
+  for (int i = 0; i <= n; ++i) {
+    t.S.push_back(p ? (__nv_bfloat16*)(p + off) : nullptr);
+    off += (size_t)B * t.L[i] * h->Rp * 2;
+  }
+  off = align_up(off, 256);
+  for (int i = 0; i < n; ++i) {
+    t.act.push_back(p ? (__nv_bfloat16*)(p + off) : nullptr);
+    off += (size_t)B * t.L[i + 1] * h->Dp * 2;
+  }
+  off = align_up(off, 256);
+  t.out = p ? (float*)(p + off) : nullptr;
+  t.bytes = off + align_up((size_t)B * t.L[n] * h->bp * 4, 256);
+  return t;
+}
+
+extern "C" size_t avvad_wavenet_tape_bytes(const avvad_wavenet* h, int64_t B, int64_t N) {
+  if (!h || B <= 0 || wn_out_len(h, N) < 1) return 0;
+  return wn_tape(h, B, N, nullptr).bytes;
+}
+
 static int wn_gemm(const __nv_bfloat16* A, int K, const WnLayer& l, int N, void* C, int ldc, bool c_bf16, bool relu,
                    int64_t M, cudaStream_t st) {
   return avvad_gemm_bf16(A, K, l.w, K, l.b, C, ldc, c_bf16 ? 1 : 0, relu ? 1 : 0, M, N, K, st);
 }
 
-// x: f32 (B, q, N) channel-major like the reference input; out: f32 (B, bottleneck, pool)
-extern "C" int avvad_wavenet_encode(avvad_wavenet* h, const float* x, int64_t B, int64_t N, void* workspace,
-                                    size_t workspace_bytes, float* out, void* stream) {
-  AVVAD_CHECK_ARG(h && x && workspace && out && B > 0, "bad argument");
-  const int64_t Lfinal = wn_out_len(h, N);
-  AVVAD_CHECK_ARG(Lfinal >= 1, "input shorter than the receptive field");
+static int wn_check(const avvad_wavenet* h, int64_t N) {
+  AVVAD_CHECK_ARG(wn_out_len(h, N) >= 1, "input shorter than the receptive field");
   if (!h->causal.set || !h->bottleneck.set) { set_error("wavenet: layers not loaded"); return AVVAD_ERR_STATE; }
   for (size_t i = 0; i < h->dil.size(); ++i)
     if (!h->dilated[i].set || !h->dense[i].set) { set_error("wavenet: layers not loaded"); return AVVAD_ERR_STATE; }
-  if (workspace_bytes < avvad_wavenet_workspace_bytes(h, B, N)) { set_error("wavenet: workspace too small"); return AVVAD_ERR_WORKSPACE; }
-  cudaStream_t st = (cudaStream_t)stream;
+  return AVVAD_OK;
+}
+
+template <bool kTape>
+static int wn_launch_fused(const tc::WnFusedGeom& g, const CUtensorMap& wmap, int k, int64_t B, cudaStream_t st) {
+  const size_t smem = tc::wavenet_fused_smem_bytes(k);
+  static PerDeviceOnce once;
+  const cudaError_t ae = once.run([] {
+    return cudaFuncSetAttribute(tc::wavenet_fused_kernel<kTape>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)tc::wavenet_fused_smem_bytes(tc::kWnMaxK));
+  });
+  if (ae != cudaSuccess) { set_error(std::string("cudaFuncSetAttribute(wavenet): ") + cudaGetErrorString(ae)); return AVVAD_ERR_CUDA; }
+  tc::wavenet_fused_kernel<kTape><<<(unsigned)(B * g.tiles_per_item), tc::kWnThreads, smem, st>>>(wmap, g);
+  AVVAD_LAUNCHED();
+  return AVVAD_OK;
+}
+
+// The forward of both entry points; with a tape (training) it also stores what the backward reads.  The values
+// computed are the same either way.
+static int wn_encode(avvad_wavenet* h, const float* x, int64_t B, int64_t N, void* workspace, const WnTape* tape,
+                     float* out, cudaStream_t st) {
+  const int64_t Lfinal = wn_out_len(h, N);
   if (wn_fused_supported(h)) {
     // ---- fused path: one kernel for the whole stack, history in shared memory (wavenet_fused.cuh) ----
     const int n = (int)h->dil.size(), k = h->k;
@@ -288,20 +342,18 @@ extern "C" int avvad_wavenet_encode(avvad_wavenet* h, const float* x, int64_t B,
     g.tiles_per_item = (int)ceil_div(Lfinal, g.lt);
     g.x = x;
     g.bias = h->bstack;
-    float* act = reinterpret_cast<float*>(workspace);   // [B][L_final][64] fp32 (fits: the workspace holds 3 fp32 streams)
+    // [B][L_final][64] fp32 (fits: the workspace holds 3 fp32 streams); the tape's copy when training
+    float* act = tape ? tape->out : reinterpret_cast<float*>(workspace);
     g.out = act;
+    if (tape) {
+      g.tape_s = tape->S[0];
+      g.tape_act = n > 0 ? tape->act[0] : nullptr;
+    }
     CUtensorMap wmap;
     int rc = tc::encode_weight_map(&wmap, h->wstack, 64, (uint64_t)n_tiles * 64, 64);
     if (rc) return rc;
-    const size_t smem = tc::wavenet_fused_smem_bytes(k);
-    static PerDeviceOnce once;
-    const cudaError_t ae = once.run([] {
-      return cudaFuncSetAttribute(tc::wavenet_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)tc::wavenet_fused_smem_bytes(tc::kWnMaxK));
-    });
-    if (ae != cudaSuccess) { set_error(std::string("cudaFuncSetAttribute(wavenet): ") + cudaGetErrorString(ae)); return AVVAD_ERR_CUDA; }
-    tc::wavenet_fused_kernel<<<(unsigned)(B * g.tiles_per_item), tc::kWnThreads, smem, st>>>(wmap, g);
-    AVVAD_LAUNCHED();
+    rc = tape ? wn_launch_fused<true>(g, wmap, k, B, st) : wn_launch_fused<false>(g, wmap, k, B, st);
+    if (rc) return rc;
     const int np = (int)(B * h->bott * h->pool);
     wn_pool_kernel<<<(unsigned)ceil_div(np, 128), 128, 0, st>>>(act, (int)B, (int)Lfinal, 64, h->bott, h->pool, out);
     AVVAD_LAUNCHED();
@@ -324,6 +376,10 @@ extern "C" int avvad_wavenet_encode(avvad_wavenet* h, const float* x, int64_t B,
     AVVAD_LAUNCHED();
     int rc = wn_gemm(A, h->k * h->qp, h->causal, h->Rp, s0, h->Rp, false, false, B * L0, st);
     if (rc) return rc;
+    if (tape) {
+      rc = avvad_pack_rows_bf16(s0, h->Rp, tape->S[0], h->Rp, 0, B * L0, h->Rp, 0, st);
+      if (rc) return rc;
+    }
   }
   float* cur = s0;
   float* nxt = s1;
@@ -334,13 +390,18 @@ extern "C" int avvad_wavenet_encode(avvad_wavenet* h, const float* x, int64_t B,
     const int64_t tot = (int64_t)B * Lo * h->k * h->Rp;
     wn_gather_kernel<<<(unsigned)ceil_div(tot, 256), 256, 0, st>>>(cur, (int)B, (int)L, h->Rp, h->k, d, (int)Lo, 1, A);
     AVVAD_LAUNCHED();
-    int rc = wn_gemm(A, h->k * h->Rp, h->dilated[i], h->Dp, act, h->Dp, true, true, B * Lo, st);  // conv + ReLU
+    __nv_bfloat16* act_i = tape ? tape->act[i] : act;
+    int rc = wn_gemm(A, h->k * h->Rp, h->dilated[i], h->Dp, act_i, h->Dp, true, true, B * Lo, st);  // conv + ReLU
     if (rc) return rc;
-    rc = wn_gemm(act, h->Dp, h->dense[i], h->Rp, tmp, h->Rp, false, false, B * Lo, st);
+    rc = wn_gemm(act_i, h->Dp, h->dense[i], h->Rp, tmp, h->Rp, false, false, B * Lo, st);
     if (rc) return rc;
     const int64_t tot2 = (int64_t)B * Lo * h->Rp;
     wn_add_slice_kernel<<<(unsigned)ceil_div(tot2, 256), 256, 0, st>>>(tmp, cur, (int)B, (int)L, (int)Lo, h->Rp, nxt);
     AVVAD_LAUNCHED();
+    if (tape) {
+      rc = avvad_pack_rows_bf16(nxt, h->Rp, tape->S[i + 1], h->Rp, 0, B * Lo, h->Rp, 0, st);
+      if (rc) return rc;
+    }
     float* t = cur; cur = nxt; nxt = t;
     L = Lo;
   }
@@ -348,11 +409,36 @@ extern "C" int avvad_wavenet_encode(avvad_wavenet* h, const float* x, int64_t B,
     const int64_t tot = (int64_t)B * L * h->Rp;
     wn_gather_kernel<<<(unsigned)ceil_div(tot, 256), 256, 0, st>>>(cur, (int)B, (int)L, h->Rp, 1, 1, (int)L, 0, A);
     AVVAD_LAUNCHED();
-    int rc = wn_gemm(A, h->Rp, h->bottleneck, h->bp, tmp, h->bp, false, true, B * L, st);
+    float* z = tape ? tape->out : tmp;
+    int rc = wn_gemm(A, h->Rp, h->bottleneck, h->bp, z, h->bp, false, true, B * L, st);
     if (rc) return rc;
     const int n = (int)(B * h->bott * h->pool);
-    wn_pool_kernel<<<(unsigned)ceil_div(n, 128), 128, 0, st>>>(tmp, (int)B, (int)L, h->bp, h->bott, h->pool, out);
+    wn_pool_kernel<<<(unsigned)ceil_div(n, 128), 128, 0, st>>>(z, (int)B, (int)L, h->bp, h->bott, h->pool, out);
     AVVAD_LAUNCHED();
   }
   return AVVAD_OK;
 }
+
+// x: f32 (B, q, N) channel-major like the reference input; out: f32 (B, bottleneck, pool)
+extern "C" int avvad_wavenet_encode(avvad_wavenet* h, const float* x, int64_t B, int64_t N, void* workspace,
+                                    size_t workspace_bytes, float* out, void* stream) {
+  AVVAD_CHECK_ARG(h && x && workspace && out && B > 0, "bad argument");
+  const int rc = wn_check(h, N);
+  if (rc) return rc;
+  if (workspace_bytes < avvad_wavenet_workspace_bytes(h, B, N)) { set_error("wavenet: workspace too small"); return AVVAD_ERR_WORKSPACE; }
+  return wn_encode(h, x, B, N, workspace, nullptr, out, (cudaStream_t)stream);
+}
+
+extern "C" int avvad_wavenet_encode_train(avvad_wavenet* h, const float* x, int64_t B, int64_t N, void* workspace,
+                                          size_t workspace_bytes, void* tape, size_t tape_bytes, float* out,
+                                          void* stream) {
+  AVVAD_CHECK_ARG(h && x && workspace && tape && out && B > 0, "bad argument");
+  const int rc = wn_check(h, N);
+  if (rc) return rc;
+  if (workspace_bytes < avvad_wavenet_workspace_bytes(h, B, N)) { set_error("wavenet: workspace too small"); return AVVAD_ERR_WORKSPACE; }
+  const WnTape t = wn_tape(h, B, N, tape);
+  if (tape_bytes < t.bytes) { set_error("wavenet: tape too small"); return AVVAD_ERR_WORKSPACE; }
+  return wn_encode(h, x, B, N, workspace, &t, out, (cudaStream_t)stream);
+}
+
+#include "wavenet_bwd.cuh"

@@ -44,12 +44,20 @@ struct WnFusedGeom {
   const float* x;
   const float* bias;         // [1 + 2*n_layers + 1][64]: causal, (dilated_i, dense_i)..., bottleneck
   float* out;                // [B][L_final][64] fp32: relu(bottleneck), time-major
+  // training forward (kTape): S_i for i = 0..n_layers, [B][L_i][64] each, back to back; act_i for i < n_layers,
+  // [B][L_{i+1}][64] each, back to back (see avvad_wavenet_tape_bytes)
+  __nv_bfloat16* tape_s;
+  __nv_bfloat16* tape_act;
 };
 
 __device__ __forceinline__ uint32_t wn_sw128_off(int row, int chunk16) {
   return (uint32_t)row * 128u + (uint32_t)((chunk16 ^ (row & 7)) << 4);
 }
 
+// kTape: also store the tile's OWNED rows of every layer input S_i (bf16, before the ReLU) and of every act_i =
+// relu(dilated_i + bias) (bf16: the dense GEMM's operand) -- rows [o0, o0 + lt) of a non-last tile, [o0, L_i) of the
+// last tile of an item, so every row is written exactly once.  The arithmetic is the same in both instantiations.
+template <bool kTape>
 __global__ void __launch_bounds__(kWnThreads)
 wavenet_fused_kernel(const __grid_constant__ CUtensorMap wmap, const WnFusedGeom g) {
   extern __shared__ uint8_t smem_raw[];
@@ -127,6 +135,10 @@ wavenet_fused_kernel(const __grid_constant__ CUtensorMap wmap, const WnFusedGeom
   const int erow = q4 * 32 + lane;
 
   int rows_in = rows0 + (g.k - 1);  // rows of the CURRENT layer's input (for the causal layer: rows_x)
+  const bool last_tile = tile == g.tiles_per_item - 1;
+  int L_in = g.L_final + g.sum_shift;   // kTape: global length of the current layer's input (S_0 for slot 1)
+  __nv_bfloat16* tape_s = g.tape_s;     // kTape: S_{slot-1} of this item
+  __nv_bfloat16* tape_a = g.tape_act;   // kTape: act_{slot-1} of this item
   for (int slot = 0; slot <= g.n_layers + 1; ++slot) {
     const bool causal = slot == 0, bott = slot == g.n_layers + 1;
     const int d = (causal || bott) ? 1 : g.dil[slot - 1];
@@ -156,6 +168,11 @@ wavenet_fused_kernel(const __grid_constant__ CUtensorMap wmap, const WnFusedGeom
           o.z = pack_relu_bf16x2(b.x, b.y); o.w = pack_relu_bf16x2(b.z, b.w);
         }
         *reinterpret_cast<uint4*>(A + wn_sw128_off(r, ch)) = o;
+        if constexpr (kTape) {
+          if (r < (last_tile ? rows_in : g.lt))
+            *reinterpret_cast<uint4*>(tape_s + ((int64_t)item * L_in + o0 + r) * 64 + ch * 8) =
+                make_uint4(pack_bf16x2(a.x, a.y), pack_bf16x2(a.z, a.w), pack_bf16x2(b.x, b.y), pack_bf16x2(b.z, b.w));
+        }
       }
     }
     fence_proxy_async();
@@ -221,6 +238,13 @@ wavenet_fused_kernel(const __grid_constant__ CUtensorMap wmap, const WnFusedGeom
         for (int cq = 0; cq < 4; ++cq)
           *reinterpret_cast<uint4*>(A2 + wn_sw128_off(erow, half * 4 + cq)) =
               make_uint4(pk[4 * cq], pk[4 * cq + 1], pk[4 * cq + 2], pk[4 * cq + 3]);
+        if constexpr (kTape) {
+          if (r < (last_tile ? rows_out : g.lt)) {
+            uint4* dst = reinterpret_cast<uint4*>(tape_a + ((int64_t)item * (L_in - shift) + o0 + r) * 64 + half * 32);
+#pragma unroll
+            for (int cq = 0; cq < 4; ++cq) dst[cq] = make_uint4(pk[4 * cq], pk[4 * cq + 1], pk[4 * cq + 2], pk[4 * cq + 3]);
+          }
+        }
       }
       tc_fence_before();
       fence_proxy_async();
@@ -265,6 +289,13 @@ wavenet_fused_kernel(const __grid_constant__ CUtensorMap wmap, const WnFusedGeom
       __syncthreads();
     }
     rows_in = rows_out;
+    if constexpr (kTape) {
+      if (!causal) {
+        tape_s += (int64_t)g.B * L_in * 64;
+        tape_a += (int64_t)g.B * (L_in - shift) * 64;
+        L_in -= shift;
+      }
+    }
   }
   tc_fence_before();
   __syncthreads();

@@ -236,6 +236,38 @@ class TrunkFunction(torch.autograd.Function):
         return (None, None, None) + tuple(grads)
 
 
+class WaveNetFunction(torch.autograd.Function):
+    """Differentiable WaveNet encoder on libavvad: forward keeps a tape (its output is the inference output, bit for
+    bit), backward runs the device backward (csrc/wavenet_bwd.cuh) and returns the gradients of the Conv1d parameters
+    in the order `wavenet_params` lists them, and of the input when it requires grad.  The input and the tape go
+    through save_for_backward: an in-place change of x before the backward, or a second backward without
+    retain_graph=True, raises autograd's own error."""
+
+    @staticmethod
+    def forward(ctx, wavenet_engine, x, *params):
+        out, (xt, tape) = wavenet_engine.forward_train(x)
+        ctx.wavenet_engine = wavenet_engine
+        ctx.save_for_backward(x, xt, tape)
+        ctx.want_dx = x.requires_grad
+        return out
+
+    @staticmethod
+    def backward(ctx, dout):
+        _, xt, tape = ctx.saved_tensors
+        dx, grads = ctx.wavenet_engine.backward((xt, tape), dout, want_dx=ctx.want_dx)
+        return (None, dx) + tuple(grads)
+
+
+def wavenet_params(module: torch.nn.Module):
+    """Weight (and bias, when present) of every Conv1d of a wavenet_autoencoder in the C ABI's gradient order.  Read
+    through the attributes, so inside an nn.DataParallel replica these are the broadcast copies."""
+    ps = []
+    for name in E.wavenet_layer_names(len(module.dilations)):
+        conv = module.get_submodule(name)
+        ps += [conv.weight] + ([conv.bias] if conv.bias is not None else [])
+    return ps
+
+
 def trunk_params(features: torch.nn.Module):
     """(conv.weight, bn.weight, bn.bias) of the 20 conv layers in libavvad's layer order."""
     ps = []

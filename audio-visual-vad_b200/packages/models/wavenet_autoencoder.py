@@ -1,9 +1,11 @@
 """WaveNet-style encoder with the reference's constructor and parameters
 (packages/models/wavenet_autoencoder.py:7-108); `_encode` / `forward` run on libavvad (csrc/wavenet.cu)."""
+import warnings
+
 import torch
 import torch.nn as nn
 
-from ._engine import E, EngineCache, device_of, full_state_dict, on_input_device
+from ._engine import E, EngineCache, WaveNetFunction, device_of, full_state_dict, on_input_device, wavenet_params
 
 
 class wavenet_autoencoder(nn.Module):
@@ -50,7 +52,22 @@ class wavenet_autoencoder(nn.Module):
 
     def _encode(self, sample):
         device = device_of(sample)
-        return self._build(device).forward(sample)
+        eng = self._build(device)
+        if torch.is_grad_enabled():
+            params = wavenet_params(self)
+            want_params = any(p.requires_grad for p in params)
+            # Differentiable when x requires grad, or when a parameter does in train() mode.  In eval() the parameters'
+            # requires_grad alone keeps the inference output (no grad_fn, so `.numpy()` works on it as it always
+            # has); the values are the same either way, the encoder has no mode-dependent layer.
+            if sample.requires_grad or (want_params and self.training):
+                # the forward keeps a tape (its output is the inference output, bit for bit) and loss.backward() runs
+                # the device backward (csrc/wavenet_bwd.cuh)
+                return WaveNetFunction.apply(eng, sample, *params)
+            if want_params:
+                warnings.warn("wavenet_autoencoder in eval() returns an output without a graph to its parameters; "
+                              "call train() to train them (the values are identical in both modes) or run under "
+                              "torch.no_grad()", stacklevel=3)
+        return eng.forward(sample)
 
     @on_input_device
     def forward(self, wave_sample):

@@ -463,6 +463,21 @@ size_t avvad_wavenet_workspace_bytes(const avvad_wavenet* h, int64_t B, int64_t 
 /* x f32 (B, quantization_channel, N) -> out f32 (B, bottleneck_width, pool_size) */
 int avvad_wavenet_encode(avvad_wavenet* h, const float* x, int64_t B, int64_t N, void* workspace,
                          size_t workspace_bytes, float* out, void* stream);
+/* Training.  The forward with a tape computes exactly what avvad_wavenet_encode computes and also keeps, in the caller's
+ * tape buffer (avvad_wavenet_tape_bytes), every layer input S_i (bf16), every dense-layer operand relu(dilated_i + bias)
+ * (bf16) and the bottleneck output (f32).  Same workspace as avvad_wavenet_encode. */
+size_t avvad_wavenet_tape_bytes(const avvad_wavenet* h, int64_t B, int64_t N);
+int avvad_wavenet_encode_train(avvad_wavenet* h, const float* x, int64_t B, int64_t N, void* workspace,
+                               size_t workspace_bytes, void* tape, size_t tape_bytes, float* out, void* stream);
+size_t avvad_wavenet_backward_workspace_bytes(const avvad_wavenet* h, int64_t B, int64_t N);
+/* Gradients of a loss given dout = d loss / d out, f32 (B, bottleneck_width, pool_size) contiguous, from the tape of
+ * avvad_wavenet_encode_train on the same x, B, N and weights.  dw[i] (f32 [O][I][k], torch Conv1d layout) and db[i]
+ * (f32 [O]) for i = 0 en_causal_layer, 1 + 2j en_dilation_layer_stack[j], 2 + 2j en_dense_layer_stack[j],
+ * 1 + 2n bottleneck_layer; every dw[i] is required, db may be NULL or hold NULL entries (use_bias=False: nothing is
+ * written).  dx: f32 (B, quantization_channel, N) or NULL.  Deterministic: identical calls give identical bits. */
+int avvad_wavenet_backward(avvad_wavenet* h, const float* x, int64_t B, int64_t N, const void* tape, size_t tape_bytes,
+                           const float* dout, float* dx, float* const* dw, float* const* db, void* workspace,
+                           size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }
